@@ -122,6 +122,34 @@ def build_workload(chains_per_pair):
     return pack, out
 
 
+DUMP_CHAINS = 256          # chains per model in a --dump-outputs sample
+DUMP_BYTES = 64 << 20      # bound on everything --dump-outputs writes
+
+
+def dump_outputs(out_dir, samples, states, row_major):
+    """Write what the last timed step returned as float64 .npy files, so two builds run with the same arguments can be
+    compared file by file.  samples: {model: the rows run() returned}, states: {model: [n, state_size] chain state}.
+    Per model: `model<m>_samples` [chains, rows, d+1] for a fixed seeded sample of DUMP_CHAINS chains (every row while
+    they fit an equal share of DUMP_BYTES, else evenly spaced rows), `model<m>_state` of the same chains, and the
+    indices `model<m>_chains` and `model<m>_rows` the sample was taken at."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    rng = np.random.default_rng(0)
+    budget = DUMP_BYTES // len(samples) - (1 << 20)    # 1 MB per model left for the state and the index files
+    for model in sorted(samples):
+        by_chain = samples[model].transpose(0, 1) if row_major else samples[model]    # [n, rows, d+1]
+        n, rows, width = by_chain.shape
+        chains = np.sort(rng.choice(n, size=min(DUMP_CHAINS, n), replace=False))
+        keep = min(rows, budget // (len(chains) * width * 8))
+        picked = np.unique(np.linspace(0, rows - 1, keep).round().astype(np.int64))
+        ci = torch.as_tensor(chains, device=by_chain.device)
+        out = {"samples": by_chain.index_select(0, ci).index_select(1, torch.as_tensor(picked, device=by_chain.device)),
+               "state": states[model].index_select(0, ci), "chains": chains, "rows": picked}
+        for name, a in out.items():
+            a = a.cpu().numpy() if torch.is_tensor(a) else a
+            np.save(os.path.join(out_dir, "model%d_%s.npy" % (model, name)), np.ascontiguousarray(a, dtype=np.float64))
+
+
 # ----------------------------------------------------------------------------------------------
 # clocks sampler (nvidia-smi during the timed region)
 # ----------------------------------------------------------------------------------------------
@@ -322,7 +350,12 @@ def main():
     ap.add_argument("--occupancy-hint", type=int, default=0, help="developer knob: min CTAs/SM variant")
     ap.add_argument("--cta-order", type=int, default=0, help="developer knob: 0 chain blocks by decreasing cost, 1 index order")
     ap.add_argument("--serial-models", action="store_true", help="run the two models back to back on one stream")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write a fixed sample of the rows and chain state the last timed step "
+                         "produced (rank 0) as DIR/<name>.npy, float64, at most 64 MB in all")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference_arm(args)
     args.warmup = max(args.warmup, 3)
@@ -378,6 +411,7 @@ def main():
 
     main_stream = torch.cuda.current_stream(dev)
     stream_events = None
+    returned = {}     # the rows each model's latest run() returned
 
     def step(first=True, last=True):
         """one step = one launch per model; the two models' launches go to two streams.  Inside a run of steps the
@@ -386,7 +420,7 @@ def main():
         for them."""
         if args.serial_models:
             for model in (2, 1):
-                samplers[model].run(K, samples=buffers[model], row_major=row_major)
+                returned[model] = samplers[model].run(K, samples=buffers[model], row_major=row_major)
             return
         if first:
             ev = torch.cuda.Event()
@@ -399,7 +433,7 @@ def main():
                 if stream_events is not None:   # per-launch duration on the launching stream
                     a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
                     a.record(st)
-                samplers[model].run(K, samples=buffers[model], row_major=row_major)
+                returned[model] = samplers[model].run(K, samples=buffers[model], row_major=row_major)
                 if stream_events is not None:
                     b.record(st)
                     stream_events[model].append((a, b))
@@ -447,6 +481,8 @@ def main():
     ms = max_over_ranks(ms)
     total_iters = float(n_chains) * K * args.steps * world
     value = total_iters / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:     # before the launches below overwrite the buffers and advance the chains
+        dump_outputs(args.dump_outputs, returned, {m: samplers[m].state for m in (1, 2)}, row_major)
 
     # ---- per-kernel launch durations (each model's kernel alone on the device), for the roofline ----
     kern_ms = {}

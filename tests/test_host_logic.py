@@ -346,10 +346,7 @@ def test_dataset_cost_orders_datasets_by_work():
     assert np.all(pack.dataset_cost(1) < c)
 
 
-def test_bench_flop_counts_match_the_survey_cost_table():
-    """bench.py's algorithmic-work figures (the roofline's numerator) against SURVEY.md section 8d's worked values:
-    model 2 on Amiodarone/hERG (d = 3, 4 doses, one of them censored) = 954 flops per chain-iteration, model 1 ~ 790,
-    hierarchical Ne = 3, N = 12 ~ 6.1 kflops; a prior-only (t = 0) chain is charged no likelihood."""
+def _import_bench():
     import importlib.util
     import sys
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -365,6 +362,14 @@ def test_bench_flop_counts_match_the_survey_cost_table():
         os.dup2(fd1, 1)
         os.close(fd1)
         sys.stdout = stdout
+    return bench
+
+
+def test_bench_flop_counts_match_the_survey_cost_table():
+    """bench.py's algorithmic-work figures (the roofline's numerator) against SURVEY.md section 8d's worked values:
+    model 2 on Amiodarone/hERG (d = 3, 4 doses, one of them censored) = 954 flops per chain-iteration, model 1 ~ 790,
+    hierarchical Ne = 3, N = 12 ~ 6.1 kflops; a prior-only (t = 0) chain is charged no likelihood."""
+    bench = _import_bench()
     from pyhillfit_b200.packing import SinglePack
     t = Table("crumb_data")
     pack = SinglePack([t.concat("Amiodarone", "hERG")])
@@ -374,6 +379,39 @@ def test_bench_flop_counts_match_the_survey_cost_table():
     assert bench.flops_per_iteration(2, g, prior_only=True) == 954 - (40 + 58 + 4 * 53 + 3 * 5 + 133 + 6)
     assert 5900 <= bench.hier_flops_per_iteration(3, 12) <= 6300
     assert bench.pack_flops(2, pack)[0] == 954
+
+
+@pytest.mark.parametrize("row_major", [True, False])
+def test_bench_dump_outputs_is_a_fixed_bounded_sample(tmp_path, monkeypatch, row_major):
+    """bench.py --dump-outputs: float64 files holding exactly the returned rows and chain state at the recorded chain
+    and row indices, the same indices on every call, all rows while they fit and evenly spaced rows (first and last
+    kept) within the size bound when they do not."""
+    import torch
+    bench = _import_bench()
+    monkeypatch.setattr(bench, "DUMP_BYTES", 4 << 20)          # 1 MB of rows per model: 128 rows of 256 chains x 4
+    g = torch.Generator().manual_seed(1)
+    shapes = {1: (100, 300, 3), 2: (1000, 300, 4)}                # [rows, n, d+1]: model 1 fits, model 2 does not
+    samples = {m: torch.randn(s, dtype=torch.float64, generator=g) for m, s in shapes.items()}
+    if not row_major:
+        samples = {m: s.transpose(0, 1).contiguous() for m, s in samples.items()}
+    states = {m: torch.randn((300, 12 + 5 * (m - 1)), dtype=torch.float64, generator=g) for m in (1, 2)}
+    for out in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / out), samples, states, row_major)
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == sorted("model%d_%s.npy" % (m, k) for m in (1, 2) for k in ("samples", "state", "chains", "rows"))
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= bench.DUMP_BYTES
+    for f in files:
+        a, b = np.load(tmp_path / "a" / f), np.load(tmp_path / "b" / f)
+        assert a.dtype == np.float64 and np.array_equal(a, b), f
+    for m in (1, 2):
+        load = lambda k: np.load(tmp_path / "a" / ("model%d_%s.npy" % (m, k)))
+        chains, rows = load("chains").astype(np.int64), load("rows").astype(np.int64)
+        by_chain = (samples[m].transpose(0, 1) if row_major else samples[m]).numpy()
+        assert len(chains) == 256 and len(np.unique(chains)) == 256
+        assert rows[0] == 0 and rows[-1] == shapes[m][0] - 1
+        assert len(rows) == (100 if m == 1 else 128)
+        assert np.array_equal(load("samples"), by_chain[chains][:, rows])
+        assert np.array_equal(load("state"), states[m].numpy()[chains])
 
 
 def test_assemble_bfs_bands_and_files(tmp_path, monkeypatch, capsys):
