@@ -301,6 +301,31 @@ int phf_best_fit_batch(int model, int64_t n_datasets, const int64_t *offsets, co
                        const double *responses, double pic50_lower, double *theta, double *ss, void *stream);
 
 /* ------------------------------------------------------------------------------------------------
+ * Convergence diagnostics (the reference has none).  Split R-hat and multi-chain effective sample size (BDA3
+ * 11.4-11.5 with Geyer's initial positive and initial monotone sequences) of every column of every group of chains,
+ * as defined by pyhillfit_b200/ess.py:chain_diagnostics.
+ *   samples        DEVICE, [n_chains][n_rows_total][n_cols] (chain-major: what the samplers write by default); rows
+ *                  [row_begin, n_rows_total) are used, split into two half-chains of n = (n_rows_total - row_begin) / 2
+ *                  rows (the middle row is dropped when the count is odd)
+ *   group_offsets  HOST, [n_groups + 1]: group g is chains group_offsets[g] .. group_offsets[g+1]-1; strictly increasing
+ *                  from 0 to n_chains
+ *   max_lag        0: no cap; otherwise Geyer pairs reach at most lag max_lag
+ *   out            DEVICE, [n_groups][n_cols][5]: pooled mean, sd = sqrt(var+), R-hat, ESS, lags (2K, the lags the
+ *                  sum used; negative when the pairs ran out -- max_lag or n -- before one was non-positive).  A column
+ *                  with W = 0 gives R-hat 1, ESS = m n, lags 0 when all half-chain means agree, else R-hat +inf, ESS 0.
+ * Arguments are checked before any CUDA call: non-positive counts, fewer than 8 rows after row_begin, NULL pointers and
+ * bad offsets give PHF_EINVAL.  The lags are taken in blocks of 32 until every column of every group has stopped; after
+ * each block the call reads the active groups back, so it SYNCHRONISES `stream` (once per block; one or two blocks for
+ * well-mixed thinned single-level chains, up to n / 32 when a group's chains disagree), and launches the next block on
+ * their chains only.  It takes a stream-ordered temporary of about n_chains * n_cols * (2 n / (8 q) + 34) doubles,
+ * q = max(1, 64 / min(16, n_cols)) (for 4 columns about 1/128 of the rows used).  Deterministic: fixed-order sums over
+ * partitions that depend on the shapes alone, the same bits on every call.
+ * ---------------------------------------------------------------------------------------------- */
+int phf_chain_diagnostics(int64_t n_chains, int64_t n_rows_total, int64_t row_begin, int32_t n_cols,
+                          const double *samples, int32_t n_groups, const int64_t *group_offsets, int64_t max_lag,
+                          double *out, void *stream);
+
+/* ------------------------------------------------------------------------------------------------
  * Utilities
  * ---------------------------------------------------------------------------------------------- */
 int phf_version(void);

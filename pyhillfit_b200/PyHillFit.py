@@ -31,6 +31,9 @@ def build_parser():
     parser.add_argument("--segment", type=int, default=50000, help="iterations per kernel launch [new]")
     parser.add_argument("--selection", type=str, default=None,
                         help="'d1,d2:c1,c2' 1-based drug and channel numbers instead of the interactive menu [new]")
+    parser.add_argument("--diagnostics", action='store_true', default=False,
+                        help="split R-hat and multi-chain ESS of each pair's chains, computed on the GPU, written "
+                             "beside the chain file as ..._diagnostics.txt [new]")
     requiredNamed = parser.add_argument_group('required arguments')
     requiredNamed.add_argument("--data-file", type=str, help="csv file from which to read in data, in same format as provided crumb_data.csv", required=True)
     requiredNamed.add_argument("-m", "--model", type=int, help="For non-hierarchical (put anything for hierarchical):1. fix Hill=1; 2. vary Hill", required=True)
@@ -122,6 +125,7 @@ def run_single_level(dr, args, pairs):
     torch.cuda.synchronize()
     assert at == kept
     print("\n{} chains x {} iterations in {:.2f} s on the GPU\n".format(s.n, args.iterations, time.time() - start))
+    diag = run_diagnostics(args, chain, len(jobs), R, 0)
     t_phase = time.time()
     host = chain.cpu().numpy()                              # burn-in already removed (PyHillFit.py:861-864)
     print("chains to the host: {:.2f} s".format(time.time() - t_phase))
@@ -130,9 +134,27 @@ def run_single_level(dr, args, pairs):
         for r in range(R):
             f = job["chain_file"] if r == 0 else chainio.extra_chain_name(job["chain_file"], r)
             chainio.save_single_level_chain(f, host[j * R + r], job["drug"], job["channel"])
+        if diag is not None:
+            names = ["pIC50", "sigma"] if args.model == 1 else ["pIC50", "Hill", "sigma"]
+            chainio.save_diagnostics(job["chain_file"], diag[j], names + ["log-target"], R, 0, kept)
         print("\n\n{} + {} complete!\n\n".format(job["drug"], job["channel"]))
     print("chain files: {:.2f} s".format(time.time() - t_phase))
     return jobs
+
+
+def run_diagnostics(args, chain, n_targets, R, row_begin):
+    """--diagnostics: split R-hat / multi-chain ESS of each target's R chains from rows [row_begin, ...) of the device
+    tensor `chain` [n_targets * R, rows, d+1] (before it is copied to the host); None without the flag."""
+    if not args.diagnostics:
+        return None
+    from . import ess
+    if chain.shape[1] - row_begin < 8:
+        print("--diagnostics: fewer than 8 rows per chain, no diagnostics written")
+        return None
+    t_phase = time.time()
+    diag = ess.chain_diagnostics_gpu(chain, np.arange(n_targets + 1) * R, row_begin=row_begin)
+    print("{} ({:.2f} s)".format(ess.diagnostics_summary(diag), time.time() - t_phase))
+    return diag
 
 
 def hierarchical_start(experiments, locs, best_fits=None):
@@ -222,12 +244,17 @@ def run_hierarchical(dr, args, pairs):
             done += k
         torch.cuda.synchronize()
         print("{} hierarchical chains (Ne={}) x {} iterations in {:.2f} s".format(s.n, ne, args.iterations, time.time() - start))
+        diag = run_diagnostics(args, chain, len(grp), R, burn)
         host = chain.cpu().numpy()
         rng = np.random.RandomState(args.seed)
         for j, job in enumerate(grp):
             for r in range(R):
                 f = job["chain_file"] if r == 0 else chainio.extra_chain_name(job["chain_file"], r)
                 chainio.save_hierarchical_chain(f, host[j * R + r])     # whole chain, burn-in kept (PyHillFit.py:514-515)
+            if diag is not None:
+                names = ["alpha", "beta", "mu", "s"] + [p + "_{}".format(e + 1) for e in range(ne) for p in ("pIC50", "Hill")]
+                chainio.save_diagnostics(job["chain_file"], diag[j], names + ["sigma", "log-target"], R, burn,
+                                         saved_iterations)
             samples_file = dr.alpha_mu_downsampling(job["drug"], job["channel"])
             print("saving (alpha,mu) samples to", samples_file)
             chainio.save_alpha_mu_samples(samples_file, host[j * R], burn, args.num_APs, job["drug"], job["channel"], rng)

@@ -28,6 +28,9 @@ def build_parser():
     parser.add_argument("--num-chains", type=int, default=1, help="replicate chains per temperature [new]")
     parser.add_argument("--seed", type=int, default=1, help="Philox seed (the reference seeds numpy with 1) [new]")
     parser.add_argument("--segment", type=int, default=50000, help="iterations per kernel launch [new]")
+    parser.add_argument("--diagnostics", action='store_true', default=False,
+                        help="split R-hat and multi-chain ESS of each temperature's chains, computed on the GPU, "
+                             "written beside the chain file as ..._diagnostics.txt [new]")
     requiredNamed = parser.add_argument_group('required arguments')
     requiredNamed.add_argument("--data-file", type=str, required=True)
     requiredNamed.add_argument("-m", "--model", type=int, required=True)
@@ -38,7 +41,8 @@ def build_parser():
 
 def do_mcmc_all_temperatures(dr, args, concs, responses, temperatures):
     """python/PyHillTemp.py:57-125 for every temperature (x replicates) at once -> [T, R, rows, d+1] host array
-    of post-burn rows, plus the in-kernel mean temperature-1 log-likelihoods [T, R]."""
+    of post-burn rows, the in-kernel mean temperature-1 log-likelihoods [T, R] and, with --diagnostics, the
+    [T, d+1, 5] diagnostics of each temperature's R chains (else None)."""
     import torch
     from .packing import SinglePack
     from .sampler import SingleLevelSampler
@@ -70,8 +74,10 @@ def do_mcmc_all_temperatures(dr, args, concs, responses, temperatures):
         done += k
     torch.cuda.synchronize()
     assert at == kept
+    from .PyHillFit import run_diagnostics
+    diag = run_diagnostics(args, chain, T, R, 0)
     host = chain.cpu().numpy().reshape(T, R, kept, d + 1)
-    return host, s.loglik_t1_mean().reshape(T, R)
+    return host, s.loglik_t1_mean().reshape(T, R), diag
 
 
 def main(argv=None):
@@ -92,7 +98,7 @@ def main(argv=None):
     temperatures = (np.arange(dr.n + 1.) / dr.n) ** dr.c
     print("\nDoing temperatures: {}\n".format(temperatures))
     start = time.time()
-    chains, ll1 = do_mcmc_all_temperatures(dr, args, concs, responses, temperatures)
+    chains, ll1, diag = do_mcmc_all_temperatures(dr, args, concs, responses, temperatures)
     print("\nMCMC time: {} s\n".format(int(time.time() - start)))
     for i, temperature in enumerate(temperatures):
         cdrug, cchannel, chain_file, images_dir = dr.nonhierarchical_chain_file_and_figs_dir(args.model, drug, channel, temperature)
@@ -100,6 +106,9 @@ def main(argv=None):
         for r in range(args.num_chains):
             f = chain_file if r == 0 else chainio.extra_chain_name(chain_file, r)
             chainio.save_tempered_chain(f, chains[i, r])
+        if diag is not None:
+            names = ["pIC50", "sigma"] if args.model == 1 else ["pIC50", "Hill", "sigma"]
+            chainio.save_diagnostics(chain_file, diag[i], names + ["log-target"], args.num_chains, 0, chains.shape[2])
     return 0
 
 

@@ -52,7 +52,7 @@ EXPORTS = ["phf_log_target_batch", "phf_am_single_init", "phf_am_single_run", "p
            "phf_release_workspaces", "phf_best_fit_batch",
            "phf_write_rows_text_host",
            "phf_hier_predictive_cdfs", "phf_format_e18", "phf_format_e18_mismatches", "phf_version", "phf_last_error",
-           "phf_fp64_peak_probe", "phf_launch_count"]
+           "phf_fp64_peak_probe", "phf_launch_count", "phf_chain_diagnostics"]
 
 _lib = None
 _p = C.c_void_p
@@ -96,6 +96,7 @@ def load():
     L.phf_write_rows_text_host.argtypes = [C.c_char_p, C.c_char_p, _p, C.c_int64, C.c_int32, C.c_int64, C.c_int32,
                                            C.c_int32]
     L.phf_best_fit_batch.argtypes = [C.c_int, C.c_int64, _p, _p, _p, C.c_double, _p, _p, _p]
+    L.phf_chain_diagnostics.argtypes = [C.c_int64, C.c_int64, C.c_int64, C.c_int32, _p, C.c_int32, _p, C.c_int64, _p, _p]
     L.phf_format_e18.argtypes = [C.c_double, C.c_char_p]
     L.phf_format_e18_mismatches.argtypes = [_p, C.c_int64]
     L.phf_format_e18_mismatches.restype = C.c_int64

@@ -66,3 +66,24 @@ def extra_chain_name(chain_file, k):
     """File for replicate chain k > 0 of the same target (the reference runs one chain; chain 0 keeps its name)."""
     root, ext = os.path.splitext(chain_file)
     return "{}_rep{}{}".format(root, k, ext)
+
+
+def diagnostics_name(chain_file):
+    """File of the convergence diagnostics of the chains of one target (--diagnostics), beside its chain file."""
+    root, ext = os.path.splitext(chain_file)
+    return "{}_diagnostics{}".format(root, ext)
+
+
+def save_diagnostics(chain_file, diag, names, n_chains, row_begin, row_end):
+    """One line per column of `diag` ([n_cols, 5] of ess.chain_diagnostics): name, mean, sd, R-hat, ESS, lags."""
+    f = diagnostics_name(chain_file)
+    chains = os.path.basename(chain_file)
+    if n_chains > 1:
+        chains += " and its replicates _rep1 .. _rep{}".format(n_chains - 1)
+    with open(f, "w") as out:
+        out.write("# split R-hat and multi-chain ESS of {} chains: {}\n".format(n_chains, chains))
+        out.write("# rows {} .. {} of each chain file's data rows\n".format(row_begin, row_end - 1))
+        out.write("# column mean sd rhat ess lags (negative lags: the sum ran out of lags, not into a non-positive pair)\n")
+        for name, (mean, sd, rhat, ess, lags) in zip(names, diag):
+            out.write("{} {:.18e} {:.18e} {:.18e} {:.18e} {:d}\n".format(name, mean, sd, rhat, ess, int(lags)))
+    return f
