@@ -30,6 +30,17 @@ int check_launch(const char *kernel_name)
     return PHF_OK;
 }
 
+int check_run_config(const phf_am_config &cfg, bool samples_given)
+{
+    if (cfg.thinning == 0) return set_error(PHF_EINVAL, "cfg.thinning must be >= 1");
+    if (cfg.sample_layout != PHF_SAMPLES_CHAIN_MAJOR && cfg.sample_layout != PHF_SAMPLES_ROW_MAJOR)
+        return set_error(PHF_EINVAL, "cfg.sample_layout must be PHF_SAMPLES_CHAIN_MAJOR or PHF_SAMPLES_ROW_MAJOR");
+    if ((uint64_t)cfg.t0 + cfg.n_iters > 0xFFFFFFFFull) return set_error(PHF_EINVAL, "iteration counter overflow");
+    if (samples_given && rows_written(cfg) > cfg.rows_capacity)
+        return set_error(PHF_EINVAL, "cfg.rows_capacity is smaller than the rows this call produces");
+    return PHF_OK;
+}
+
 void count_launch() { g_launches.fetch_add(1, std::memory_order_relaxed); }
 
 int sm_count()

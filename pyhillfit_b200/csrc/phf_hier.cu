@@ -4,14 +4,13 @@
 //   lane i evaluates data point i (Hill curve, truncated-normal normaliser);
 //   lanes 4..dim-2 evaluate the per-experiment logistic / log-logistic terms;
 //   sums are fp64 xor-shuffle reductions inside the group.
-#include "phf_common.cuh"
-#include "phf_math.cuh"
+#include "phf_hier.cuh"
 
 namespace phf {
 
 // Per-lane constants of the Gamma hyper-priors on theta[[0,1,2,3,-1]] (PyHillFit.py:187, 301, 363-364).
 struct LanePrior {
-    double loc, shape_m1, inv_scale;  // zero on lanes that carry no hyper-prior
+    double loc, shape_m1, scale;      // zero on lanes that carry no hyper-prior
     double lower;                     // support: theta_j < lower (or <= for strict) is outside
     bool strict;                      // true: theta_j <= lower is outside (PyHillFit.py:176,182)
     bool has_gamma;
@@ -20,7 +19,7 @@ struct LanePrior {
 PHF_DI LanePrior lane_prior(int gl, int dim, const phf_hier_priors &pr)
 {
     LanePrior lp;
-    lp.loc = 0.0; lp.shape_m1 = 0.0; lp.inv_scale = 0.0; lp.lower = -CUDART_INF; lp.strict = false;
+    lp.loc = 0.0; lp.shape_m1 = 0.0; lp.scale = 0.0; lp.lower = -CUDART_INF; lp.strict = false;
     lp.has_gamma = false;
     int slot = -1;
     if (gl < 4) slot = gl;
@@ -33,7 +32,7 @@ PHF_DI LanePrior lane_prior(int gl, int dim, const phf_hier_priors &pr)
                          : slot == 3 ? pr.shapes[3] : pr.shapes[4];
         const double scl = slot == 0 ? pr.scales[0] : slot == 1 ? pr.scales[1] : slot == 2 ? pr.scales[2]
                          : slot == 3 ? pr.scales[3] : pr.scales[4];
-        lp.loc = loc; lp.shape_m1 = shp - 1.0; lp.inv_scale = 1.0 / scl; lp.lower = loc; lp.strict = true;
+        lp.loc = loc; lp.shape_m1 = shp - 1.0; lp.scale = scl; lp.lower = loc; lp.strict = true;
         lp.has_gamma = true;
     } else if (gl < dim - 1) {
         // gl = 4+2e: pIC50_e >= pic50_lower; gl = 5+2e: Hill_e >= 0 (PyHillFit.py:182)
@@ -78,12 +77,11 @@ PHF_DI double hier_log_target(const double *T, double th_j, int gl, int dim, con
     // ---- one vector log for every entry, one for the Gamma hyper-priors ----
     // (log_pos needs a positive argument: entries that may legitimately be <= 0 -- mu, pIC50_e -- never use theirs;
     //  Hill_e == 0 is in support and the reference's log(0) = -inf is reproduced)
-    const double lth = th_j > 0.0 ? fm::log_pos(T, th_j) : -CUDART_INF;
-    const double xm = th_j - lp.loc;
+    const double lth = hier_safe_log(T, th_j);
     double term = 0.0;
     {
-        const double lg = fm::log_pos(T, xm > 0.0 ? xm : 1.0);
-        if (lp.has_gamma) term = fma(lp.shape_m1, lg, -xm * lp.inv_scale);  // dr.log_gamma_prior (doseresponse.py:308)
+        const double g = hier_gamma_prior(T, th_j - lp.loc, lp.shape_m1, lp.scale);
+        if (lp.has_gamma) term = g;
     }
     const double alpha_l = __shfl_sync(mask, lth, 0, G);
     const double beta = __shfl_sync(mask, th_j, 1, G);
@@ -98,18 +96,15 @@ PHF_DI double hier_log_target(const double *T, double th_j, int gl, int dim, con
     {
         const bool is_pic50 = (gl & 1) == 0;
         const double zz = (th_j - mu) * fm::rcp(s);                          // PyHillFit.py:145
-        const double arg = is_pic50 ? -zz : beta * (lth - alpha_l);          // (x/alpha)**beta, PyHillFit.py:135
-        // log(1 + e^arg): = arg to the last bit beyond 36; the reference's exp overflows to inf beyond ln(DBL_MAX)
-        // and the term becomes -inf (PyHillFit.py:135,146 -- an artefact that is part of its behaviour)
-        double l = fm::log_pos(T, 1.0 + fm::exp_clamped(T, arg));
-        l = arg > 36.0 ? arg : l;
-        l = arg > 709.782712893384 ? CUDART_INF : l;
-        const double t_pic = -zz - s_l - 2.0 * l;                            // PyHillFit.py:146
-        const double t_hill = beta_l - beta * alpha_l + (beta - 1.0) * lth - 2.0 * l;  // PyHillFit.py:135
+        // one softplus per lane, of the argument of the term the lane holds
+        const double l = hier_softplus(T, is_pic50 ? hier_pic50_arg(zz) : hier_hill_arg(beta, alpha_l, lth));
+        const auto softplus = [l](double) { return l; };
+        const double t_pic = hier_pic50_term(zz, s_l, softplus);
+        const double t_hill = hier_hill_term(beta, beta_l, alpha_l, lth, softplus);
         if (gl >= 4 && gl < dim - 1) term = is_pic50 ? t_pic : t_hill;
     }
 
-    // ---- data likelihood, truncated-normal noise (PyHillFit.py:113-125): one point per lane per round ----
+    // ---- data likelihood: one point per lane per round ----
     const double inv_s = fm::rcp(sigma);
     const double inv2s2 = 0.5 * inv_s * inv_s;
     const double inv_s_rt2 = inv_s * kSqrtHalf;
@@ -123,19 +118,8 @@ PHF_DI double hier_log_target(const double *T, double th_j, int gl, int dim, con
         const double hill_e = __shfl_sync(mask, th_j, 5 + 2 * e, G);
         double lic_hi, lic_lo;
         ln_ic50(pic50_e, lic_hi, lic_lo);
-        const double x = hill_ratio_pow(T, P.lnc_hi, P.lnc_lo, lic_hi, lic_lo, hill_e);
-        const double p = hill_response(x);
-        const double r = P.y - p;
-        // st.norm.cdf(100,p,sigma) - st.norm.cdf(0,p,sigma) = 1 - (erfc(ta) + erfc(tb))/2 with ta = (100-p)/(sigma
-        // sqrt2) >= 0, tb = p/(sigma sqrt2) >= 0 (p is in [0,100]); erfc(t) = erfcx(t) e^{-t^2}.  The two
-        // evaluations are independent straight-line code, so they interleave.
-        const double ta = (100.0 - p) * inv_s_rt2, tb = p * inv_s_rt2;
-        const double qa = fm::erfcx_nonneg(T, ta) * fm::exp_clamped(T, -ta * ta);
-        const double qb = fm::erfcx_nonneg(T, tb) * fm::exp_clamped(T, -tb * tb);
-        const double dphi = 1.0 - 0.5 * (qa + qb);
-        const double ldphi = dphi > 0.0 ? fm::log_pos(T, dphi) : -CUDART_INF;
-        const double contrib = -(fma(r * r, inv2s2, ldphi) + sigma_l);
-        if (has) term += contrib;
+        const double nll = hier_point_nll(T, P.lnc_hi, P.lnc_lo, P.y, lic_hi, lic_lo, hill_e, inv2s2, inv_s_rt2, sigma_l);
+        if (has) term -= nll;
     }
     const double total = group_sum<G>(term, mask);
     return bad ? -CUDART_INF : total;
@@ -316,22 +300,13 @@ __global__ void __launch_bounds__(128, hier_min_ctas(DIM)) am_hier_kernel(phf_am
     double zz0 = 0.0, zz1 = 0.0, lu = 0.0;
 
     uint32_t t = cfg.t0;
-    uint32_t until_save = cfg.thinning - (t % cfg.thinning);
-    uint32_t row = t / cfg.thinning;
-    const uint32_t row_base = first_row_written(cfg);
-    // chain-major: rows of a chain DIM+1 doubles apart; row-major: n chains apart (phf_am_config.sample_layout)
-    const bool row_major = cfg.sample_layout == PHF_SAMPLES_ROW_MAJOR;
-    double *out = samples ? samples + (row_major ? (size_t)c : (size_t)c * cfg.rows_capacity) * (DIM + 1) : nullptr;
-    const size_t row_stride = row_major ? (size_t)n * (DIM + 1) : (size_t)(DIM + 1);
+    RowCursor rows(cfg, c, n, DIM, samples);
     double gam_lane = 0.0;
 
     for (uint32_t it = 0; it < cfg.n_iters; ++it) {
         ++t;
         if ((it & 31u) == 0u) {
-            const uint32_t tl = t + lane;
-            gam_lane = tl > cfg.adapt_when  // PyHillFit.py:496-497
-                           ? fm::exp_clamped(T, -0.6 * fm::log_pos(T, (double)(tl - cfg.adapt_when) + 1.0))
-                           : 0.0;
+            gam_lane = adapt_gamma(T, t + lane, cfg.adapt_when);
         }
         const double gam = __shfl_sync(0xffffffffu, gam_lane, it & 31u);
 
@@ -393,15 +368,11 @@ __global__ void __launch_bounds__(128, hier_min_ctas(DIM)) am_hier_kernel(phf_am
         }
 
         // ---- thinned write-out (PyHillFit.py:502-503): lanes write one row, coalesced ----
-        if (--until_save == 0u) {
-            until_save = cfg.thinning;
-            ++row;
-            if (out && active && row >= row_base) {
-                double *o = out + (size_t)(row - row_base) * row_stride;
+        if (rows.due(cfg.thinning))
+            if (double *o = rows.dest(active)) {
                 if (row_ok) o[gl] = th_j;
                 if (gl == DIM) o[DIM] = lt;
             }
-        }
     }
 
     if (active) {
@@ -436,8 +407,6 @@ static int launch_am_hier(const phf_am_config &cfg, int64_t n, double *state, co
     return check_launch("am_hier_kernel");
 }
 
-// phf_hier_thread.cu: one thread per chain, n_expts <= kHierThreadMaxExpts
-constexpr int kHierThreadMaxExpts = 6;
 // cfg.lanes_per_chain == 0: which of the three forms runs a launch of n chains.  Measured on B200 (scripts/hier_probe.py,
 // profiles/r02_hier_forms_by_size.txt; ms per 1000 iterations, lane / thread / quad kernel):
 //   Ne = 3:  2 464 chains 3.8 / 10.1 / 4.8;  4 928: 6.9 / 10.2 / 5.7;  9 856: 11.1 / 10.3 / 6.5;  19 712: 19.5 / 12.6 / 11.9;
@@ -453,23 +422,6 @@ constexpr int kHierThreadMaxExpts = 6;
 constexpr int kHierQuadMinChainsPerSm = 32;
 constexpr int kHierThreadAutoMaxExpts = 3;
 constexpr int kHierThreadMinChainsPerSm = 160;
-int am_hier_thread_launch(const phf_am_config &cfg, int32_t n_expts, int64_t n, double *state, const int32_t *dataset_id,
-                          const phf_hier_dataset *datasets, const phf_hier_point *points, const phf_hier_priors &pr,
-                          double *samples, cudaStream_t s);
-
-// phf_hier_quad.cu: four lanes per chain, n_expts <= kHierQuadMaxExpts
-constexpr int kHierQuadMaxExpts = 5;
-int am_hier_quad_launch(const phf_am_config &cfg, int32_t n_expts, int64_t n, double *state, const int32_t *dataset_id,
-                        const phf_hier_dataset *datasets, const phf_hier_point *points, const phf_hier_priors &pr,
-                        double *samples, cudaStream_t s);
-
-// phf_hier_big.cu
-int hier_big_target_launch(int64_t n, const double *theta, int32_t theta_stride, const double *cov0,
-                           const int32_t *dataset_id, const phf_hier_dataset *datasets, const phf_hier_point *points,
-                           const phf_hier_priors &pr, double *out, double *state, cudaStream_t s);
-int am_hier_big_launch(const phf_am_config &cfg, int32_t n_expts, int64_t n, double *state, const int32_t *dataset_id,
-                       const phf_hier_dataset *datasets, const phf_hier_point *points, const phf_hier_priors &pr,
-                       double *samples, cudaStream_t s);
 
 }  // namespace phf
 
@@ -541,14 +493,9 @@ extern "C" int phf_am_hier_run(const phf_am_config *cfg, int32_t n_expts, int64_
 {
     if (!cfg || !priors) return set_error(PHF_EINVAL, "phf_am_hier_run: cfg/priors is NULL");
     if (n_expts < 1 || n_expts > PHF_HIER_BIG_MAX_EXPTS) return set_error(PHF_ENOTSUP, "n_expts outside 1..128");
-    if (cfg->thinning == 0) return set_error(PHF_EINVAL, "cfg.thinning must be >= 1");
-    if (cfg->sample_layout != PHF_SAMPLES_CHAIN_MAJOR && cfg->sample_layout != PHF_SAMPLES_ROW_MAJOR)
-        return set_error(PHF_EINVAL, "cfg.sample_layout must be PHF_SAMPLES_CHAIN_MAJOR or PHF_SAMPLES_ROW_MAJOR");
+    if (int rc = check_run_config(*cfg, samples != nullptr)) return rc;
     if (n_chains < 0 || (n_chains > 0 && (!state || !dataset_id || !datasets || !points)))
         return set_error(PHF_EINVAL, "phf_am_hier_run: null pointer");
-    if ((uint64_t)cfg->t0 + cfg->n_iters > 0xFFFFFFFFull) return set_error(PHF_EINVAL, "iteration counter overflow");
-    if (samples && rows_written(*cfg) > cfg->rows_capacity)
-        return set_error(PHF_EINVAL, "cfg.rows_capacity is smaller than the rows this call produces");
     if (n_chains == 0 || cfg->n_iters == 0) return PHF_OK;
     cudaStream_t s = (cudaStream_t)stream;
     if (n_expts > PHF_HIER_MAX_EXPTS)

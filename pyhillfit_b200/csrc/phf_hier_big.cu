@@ -5,8 +5,7 @@
 // factor in a column-major scratch triangle, so that for a fixed column the rows handled by consecutive lanes are
 // contiguous.  Same algorithm, same Philox stream and same pivot floor as the small kernels and the oracle
 // (python/PyHillFit.py:113-154, 173-193, 481-511).
-#include "phf_common.cuh"
-#include "phf_math.cuh"
+#include "phf_hier.cuh"
 
 namespace phf {
 
@@ -18,16 +17,6 @@ PHF_DI double warp_sum(double v)
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
     return v;
 }
-
-// log(1 + e^arg) with the reference's overflow artefact (see phf_hier.cu)
-PHF_DI double softplus_ref(const double *T, double arg)
-{
-    double l = fm::log_pos(T, 1.0 + fm::exp_clamped(T, arg));
-    l = arg > 36.0 ? arg : l;
-    return arg > 709.782712893384 ? CUDART_INF : l;
-}
-
-PHF_DI double safe_log(const double *T, double x) { return x > 0.0 ? fm::log_pos(T, x) : -CUDART_INF; }
 
 // log_target_distribution (PyHillFit.py:173-193) of the theta in shared memory `th`; all 32 lanes call it, the
 // result is uniform across the warp.
@@ -48,12 +37,12 @@ PHF_DI double hier_big_log_target(const double *T, const double *th, int dim, in
     bad = __any_sync(0xffffffffu, bad) != 0;
 
     const double alpha = th[0], beta = th[1], mu = th[2], s = th[3], sigma = th[dim - 1];
-    const double alpha_l = safe_log(T, alpha), beta_l = safe_log(T, beta), s_l = safe_log(T, s);
-    const double sigma_l = safe_log(T, sigma);
+    const double alpha_l = hier_safe_log(T, alpha), beta_l = hier_safe_log(T, beta), s_l = hier_safe_log(T, s);
+    const double sigma_l = hier_safe_log(T, sigma);
     const double inv_sc = fm::rcp(s);
 
     double term = 0.0;
-    // ---- Gamma hyper-priors on (alpha, beta, mu, s, sigma): dr.log_gamma_prior (doseresponse.py:308) ----
+    // ---- Gamma hyper-priors on (alpha, beta, mu, s, sigma) ----
     if (lane < 5) {
         const int j = lane < 4 ? lane : dim - 1;
         const double loc = lane == 0 ? pr.locs[0] : lane == 1 ? pr.locs[1] : lane == 2 ? pr.locs[2]
@@ -62,19 +51,17 @@ PHF_DI double hier_big_log_target(const double *T, const double *th, int dim, in
                          : lane == 3 ? pr.shapes[3] : pr.shapes[4];
         const double scl = lane == 0 ? pr.scales[0] : lane == 1 ? pr.scales[1] : lane == 2 ? pr.scales[2]
                          : lane == 3 ? pr.scales[3] : pr.scales[4];
-        const double xm = th[j] - loc;
-        const double inv_scl = 1.0 / scl;
-        term = fma(shp - 1.0, fm::log_pos(T, xm > 0.0 ? xm : 1.0), -xm * inv_scl);
+        term = hier_gamma_prior(T, th[j] - loc, shp - 1.0, scl);
     }
-    // ---- per-experiment logistic / log-logistic terms (PyHillFit.py:134-154) ----
+    // ---- per-experiment terms ----
+    const auto softplus = [T](double a) { return hier_softplus(T, a); };
     for (int e = lane; e < n_expts; e += 32) {
         const double pic50_e = th[4 + 2 * e], hill_e = th[5 + 2 * e];
         const double zz = (pic50_e - mu) * inv_sc;
-        term += -zz - s_l - 2.0 * softplus_ref(T, -zz);
-        const double lh = safe_log(T, hill_e);
-        term += beta_l - beta * alpha_l + (beta - 1.0) * lh - 2.0 * softplus_ref(T, beta * (lh - alpha_l));
+        term += hier_pic50_term(zz, s_l, softplus);
+        term += hier_hill_term(beta, beta_l, alpha_l, hier_safe_log(T, hill_e), softplus);
     }
-    // ---- data likelihood, truncated-normal noise (PyHillFit.py:113-125) ----
+    // ---- data likelihood ----
     const double inv_s = fm::rcp(sigma);
     const double inv2s2 = 0.5 * inv_s * inv_s;
     const double inv_s_rt2 = inv_s * kSqrtHalf;
@@ -83,14 +70,7 @@ PHF_DI double hier_big_log_target(const double *T, const double *th, int dim, in
         const int e = (int)(__double_as_longlong(v.w) & 0xffffffffll);
         double lic_hi, lic_lo;
         ln_ic50(th[4 + 2 * e], lic_hi, lic_lo);
-        const double x = hill_ratio_pow(T, v.x, v.y, lic_hi, lic_lo, th[5 + 2 * e]);
-        const double p = hill_response(x);
-        const double r = v.z - p;
-        const double ta = (100.0 - p) * inv_s_rt2, tb = p * inv_s_rt2;
-        const double qa = fm::erfcx_nonneg(T, ta) * fm::exp_clamped(T, -ta * ta);
-        const double qb = fm::erfcx_nonneg(T, tb) * fm::exp_clamped(T, -tb * tb);
-        const double dphi = 1.0 - 0.5 * (qa + qb);
-        term -= fma(r * r, inv2s2, safe_log(T, dphi)) + sigma_l;
+        term -= hier_point_nll(T, v.x, v.y, v.z, lic_hi, lic_lo, th[5 + 2 * e], inv2s2, inv_s_rt2, sigma_l);
     }
     const double total = warp_sum(term);
     return bad ? -CUDART_INF : total;
@@ -180,20 +160,12 @@ __global__ void __launch_bounds__(32) am_hier_big_kernel(phf_am_config cfg, int3
     __syncwarp();
 
     uint32_t t = cfg.t0;
-    uint32_t until_save = cfg.thinning - (t % cfg.thinning);
-    uint32_t row = t / cfg.thinning;
-    const uint32_t row_base = first_row_written(cfg);
-    const bool row_major = cfg.sample_layout == PHF_SAMPLES_ROW_MAJOR;  // phf_am_config.sample_layout
-    double *out = samples ? samples + (row_major ? (size_t)c : (size_t)c * cfg.rows_capacity) * (dim + 1) : nullptr;
-    const size_t row_stride = row_major ? (size_t)n * (dim + 1) : (size_t)(dim + 1);
+    RowCursor rows(cfg, c, n, dim, samples);
     const int n_pairs = (dim + 1) / 2;
 
     for (uint32_t it = 0; it < cfg.n_iters; ++it) {
         ++t;
-        // gamma_s = 1/(s+1)**0.6 (PyHillFit.py:496-497)
-        const double gam = t > cfg.adapt_when
-                               ? fm::exp_clamped(T, -0.6 * fm::log_pos(T, (double)(t - cfg.adapt_when) + 1.0))
-                               : 0.0;
+        const double gam = adapt_gamma(T, t, cfg.adapt_when);
 
         // ---- draws (stream contract: oracle/hill_oracle.py): pair q -> z[2q], z[2q+1]; u from call 0 ----
         double u;
@@ -273,15 +245,11 @@ __global__ void __launch_bounds__(32) am_hier_big_kernel(phf_am_config cfg, int3
         }
 
         // ---- thinned write-out (PyHillFit.py:502-503) ----
-        if (--until_save == 0u) {
-            until_save = cfg.thinning;
-            ++row;
-            if (out && row >= row_base) {
-                double *o = out + (size_t)(row - row_base) * row_stride;
+        if (rows.due(cfg.thinning))
+            if (double *o = rows.dest(true)) {  // (every chain of the launch is active: blocks past n return early)
                 for (int j = lane; j < dim; j += 32) o[j] = th[j];
                 if (lane == 0) o[dim] = lt;
             }
-        }
     }
 
     for (int j = lane; j < dim; j += 32) {
@@ -295,7 +263,7 @@ __global__ void __launch_bounds__(32) am_hier_big_kernel(phf_am_config cfg, int3
     }
 }
 
-// ---- host-side launchers used by the C ABI entry points in phf_hier.cu ----
+// ---- host-side launchers (phf_hier.cuh) ----
 int hier_big_target_launch(int64_t n, const double *theta, int32_t theta_stride, const double *cov0,
                            const int32_t *dataset_id, const phf_hier_dataset *datasets, const phf_hier_point *points,
                            const phf_hier_priors &pr, double *out, double *state, cudaStream_t s)

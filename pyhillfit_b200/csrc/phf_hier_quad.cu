@@ -25,32 +25,11 @@
 // Same algorithm, Philox stream contract and guarded pivots as the other hierarchical kernels and the oracle; the
 // log-target's summation order differs, so trajectories agree with them to rounding (tests/test_gpu_sampler.py follows
 // this kernel against the C oracle step by step like the others).
-#include "phf_common.cuh"
-#include "phf_math.cuh"
-
-// which erfcx the point loop uses: the table-driven one (32 degree-7 polynomials, 27 fp64 instructions) or the single
-// degree-22 polynomial (39) -- see phf_fastmath.cuh; a kernel uses one form throughout.  Measured: the table form
-// loses 4-13 % in this kernel (profiles/r02_quad_erfcx_ab.txt), like in the other one-point-per-lane kernels
-#ifndef PHF_QUAD_ERFCX
-#define PHF_QUAD_ERFCX fm::erfcx_nonneg
-#endif
+#include "phf_hier.cuh"
 
 namespace phf {
 
 namespace {
-
-PHF_DI double softplus_ref_q(const double *T, double arg)  // log(1 + e^arg) with the reference's overflow artefact
-{
-    double l = fm::log_pos(T, 1.0 + fm::exp_clamped(T, arg));
-    l = arg > 36.0 ? arg : l;
-    return arg > 709.782712893384 ? CUDART_INF : l;
-}
-
-PHF_DI double safe_log_q(const double *T, double x)  // log x, -inf for x <= 0; branch-free
-{
-    const double l = fm::log_pos(T, x > 0.0 ? x : 1.0);
-    return x > 0.0 ? l : -CUDART_INF;
-}
 
 template <int NE>
 struct QuadCfg {
@@ -84,35 +63,31 @@ PHF_DI double hier_quad_log_target(const double *T, const double (&th)[5 + 2 * N
 {
     constexpr int DIM = 5 + 2 * NE;
     constexpr unsigned full = 0xffffffffu;
-    // ---- support (PyHillFit.py:176-183) ----
-    bool bad = !(th[0] > pr.locs[0]) || !(th[1] > pr.locs[1]) || !(th[2] > pr.locs[2]) || !(th[3] > pr.locs[3]) ||
-               !(th[DIM - 1] > pr.locs[4]);
-#pragma unroll
-    for (int e = 0; e < NE; ++e) bad = bad || !(th[4 + 2 * e] >= pr.pic50_lower) || !(th[5 + 2 * e] >= 0.0);
-
+    const bool bad = !hier_in_support<NE>(th, pr);
     const double beta = th[1], mu = th[2], sigma = th[DIM - 1];
-    const double alpha_l = safe_log_q(T, th[0]), beta_l = safe_log_q(T, beta), s_l = safe_log_q(T, th[3]);
-    const double sigma_l = safe_log_q(T, sigma);
+    const double alpha_l = hier_safe_log(T, th[0]), beta_l = hier_safe_log(T, beta), s_l = hier_safe_log(T, th[3]);
+    const double sigma_l = hier_safe_log(T, sigma);
     const double inv_sc = fm::rcp(th[3]);
+    const auto softplus = [T](double a) { return hier_softplus(T, a); };
 
     double term;
-    // ---- Gamma hyper-priors on (alpha, beta, mu, s, sigma): dr.log_gamma_prior (doseresponse.py:308): lane q takes the
-    //      prior on theta_q, lane 0 also the one on sigma ----
+    // ---- Gamma hyper-priors on (alpha, beta, mu, s, sigma): lane q takes the prior on theta_q, lane 0 also the one on
+    //      sigma ----
     {
         const double x = q == 0 ? th[0] : (q == 1 ? th[1] : (q == 2 ? th[2] : th[3]));
         const double loc = q == 0 ? pr.locs[0] : (q == 1 ? pr.locs[1] : (q == 2 ? pr.locs[2] : pr.locs[3]));
         const double shp = q == 0 ? pr.shapes[0] : (q == 1 ? pr.shapes[1] : (q == 2 ? pr.shapes[2] : pr.shapes[3]));
         const double scl = q == 0 ? pr.scales[0] : (q == 1 ? pr.scales[1] : (q == 2 ? pr.scales[2] : pr.scales[3]));
         const double xm = x - loc, xs = sigma - pr.locs[4];
-        term = fma(shp - 1.0, fm::log_pos(T, xm > 0.0 ? xm : 1.0), -xm * (1.0 / scl));
-        const double gs = fma(pr.shapes[4] - 1.0, fm::log_pos(T, xs > 0.0 ? xs : 1.0), -xs * (1.0 / pr.scales[4]));
+        term = hier_gamma_prior(T, xm, shp - 1.0, scl);
+        const double gs = hier_gamma_prior(T, xs, pr.shapes[4] - 1.0, pr.scales[4]);
         term += q == 0 ? gs : 0.0;
     }
     // ---- ln IC50 of every experiment (cheap; every lane's points may belong to any experiment) ----
     double lic_hi[NE], lic_lo[NE];
 #pragma unroll
     for (int e = 0; e < NE; ++e) ln_ic50(th[4 + 2 * e], lic_hi[e], lic_lo[e]);
-    // ---- per-experiment logistic / log-logistic terms (PyHillFit.py:134-154): experiment q, q + 4 ----
+    // ---- per-experiment terms: experiment q, q + 4 ----
 #pragma unroll
     for (int r = 0; r < (NE + 3) / 4; ++r) {
         const int e = q + 4 * r;
@@ -124,50 +99,31 @@ PHF_DI double hier_quad_log_target(const double *T, const double (&th)[5 + 2 * N
                 hill_e = q == k ? th[5 + 2 * (4 * r + k)] : hill_e;
             }
         const double zz = (pic50_e - mu) * inv_sc;
-        double te = -zz - s_l - 2.0 * softplus_ref_q(T, -zz);
-        const double lh = safe_log_q(T, hill_e);
-        te += beta_l - beta * alpha_l + (beta - 1.0) * lh - 2.0 * softplus_ref_q(T, beta * (lh - alpha_l));
+        double te = hier_pic50_term(zz, s_l, softplus);
+        te += hier_hill_term(beta, beta_l, alpha_l, hier_safe_log(T, hill_e), softplus);
         term += e < NE ? te : 0.0;
     }
-    // ---- data likelihood, truncated-normal noise (PyHillFit.py:113-125): points q, q + 4, ... ----
+    // ---- data likelihood: points q, q + 4, ... ----
     const double inv_s = fm::rcp(sigma);
     const double inv2s2 = 0.5 * inv_s * inv_s;
     const double inv_s_rt2 = inv_s * kSqrtHalf;
-    // PHF_QUAD_PU points per trip, predicated instead of looped: independent straight-line evaluations that ptxas can
-    // interleave (a lane is otherwise a serial chain of dependent FP64 instructions)
-#ifndef PHF_QUAD_PU
-#define PHF_QUAD_PU 1  // (measured: 2 loses 9 % at 12 points per dataset -- 3 per lane, a fourth evaluated for nothing -- and ties at 16)
-#endif
-    constexpr int PU = PHF_QUAD_PU;
-    for (int base = q; base < npts_warp; base += 4 * PU) {  // (npts_warp: a multiple-of-4 bound common to the warp)
-        double contrib[PU];
+    // (one point per trip: measured, two predicated points per trip lose 9 % at 12 points per dataset and tie at 16;
+    //  the table-driven erfcx loses 4-13 % here, profiles/r02_quad_erfcx_ab.txt)
+    for (int pi = q; pi < npts_warp; pi += 4) {  // (npts_warp: a multiple-of-4 bound common to the warp)
+        const bool has = pi < npts;
+        const phf_hier_point *pp = pts + (has ? pi : 0);
+        const double2 v01 = __ldg(reinterpret_cast<const double2 *>(pp));
+        const double2 v23 = __ldg(reinterpret_cast<const double2 *>(pp) + 1);
+        const int e = (int)(__double_as_longlong(v23.y) & 0xffffffffll);
+        double lh = lic_hi[0], ll = lic_lo[0], hill_e = th[5];
 #pragma unroll
-        for (int u = 0; u < PU; ++u) {
-            const int pi = base + 4 * u;
-            const bool has = pi < npts;
-            const phf_hier_point *pp = pts + (has ? pi : 0);
-            const double2 v01 = __ldg(reinterpret_cast<const double2 *>(pp));
-            const double2 v23 = __ldg(reinterpret_cast<const double2 *>(pp) + 1);
-            const int e = (int)(__double_as_longlong(v23.y) & 0xffffffffll);
-            double lh = lic_hi[0], ll = lic_lo[0], hill_e = th[5];
-#pragma unroll
-            for (int k = 1; k < NE; ++k) {
-                lh = e == k ? lic_hi[k] : lh;
-                ll = e == k ? lic_lo[k] : ll;
-                hill_e = e == k ? th[5 + 2 * k] : hill_e;
-            }
-            const double x = hill_ratio_pow(T, v01.x, v01.y, lh, ll, hill_e);
-            const double p = hill_response(x);
-            const double r = v23.x - p;
-            const double ta = (100.0 - p) * inv_s_rt2, tb = p * inv_s_rt2;
-            const double qa = PHF_QUAD_ERFCX(T, ta) * fm::exp_clamped(T, -ta * ta);
-            const double qb = PHF_QUAD_ERFCX(T, tb) * fm::exp_clamped(T, -tb * tb);
-            const double dphi = 1.0 - 0.5 * (qa + qb);
-            const double cb = fma(r * r, inv2s2, safe_log_q(T, dphi)) + sigma_l;
-            contrib[u] = has ? cb : 0.0;
+        for (int k = 1; k < NE; ++k) {
+            lh = e == k ? lic_hi[k] : lh;
+            ll = e == k ? lic_lo[k] : ll;
+            hill_e = e == k ? th[5 + 2 * k] : hill_e;
         }
-#pragma unroll
-        for (int u = 0; u < PU; ++u) term -= contrib[u];
+        const double cb = hier_point_nll(T, v01.x, v01.y, v23.x, lh, ll, hill_e, inv2s2, inv_s_rt2, sigma_l);
+        term -= has ? cb : 0.0;
     }
     // ---- the chain's four partial sums (identical bits on the four lanes: fp addition is commutative) ----
     term += __shfl_xor_sync(full, term, 1);
@@ -238,10 +194,7 @@ __global__ void __launch_bounds__(128, MINB)
     for (uint32_t it = 0; it < cfg.n_iters; ++it) {
         ++t;
         if ((it & 31u) == 0u) {  // gamma_s is a function of t only: lane L computes it for iteration t + L
-            const uint32_t tl = t + (uint32_t)lane;
-            const double g = tl > cfg.adapt_when  // PyHillFit.py:496-497
-                                 ? fm::exp_clamped(T, -0.6 * fm::log_pos(T, (double)(tl - cfg.adapt_when) + 1.0))
-                                 : 0.0;
+            const double g = adapt_gamma(T, t + (uint32_t)lane, cfg.adapt_when);
             __syncwarp();
             gam_slots[lane] = g;
             __syncwarp();

@@ -23,107 +23,58 @@
 // Same algorithm, same operation order inside every dot product, same Philox stream contract and the same guarded
 // pivots as the lane kernel and the oracle; the reduction order of the log-target differs (gamma priors, then
 // experiments, then points), so trajectories agree with the other kernels to rounding, not bit for bit.
-#include "phf_common.cuh"
-#include "phf_math.cuh"
+#include "phf_hier.cuh"
 
 namespace phf {
 
-namespace {
-
-PHF_DI double softplus_ref_t(const double *T, double arg)  // log(1 + e^arg) with the reference's overflow artefact
-{
-    double l = fm::log_pos(T, 1.0 + fm::exp_clamped(T, arg));
-    l = arg > 36.0 ? arg : l;
-    return arg > 709.782712893384 ? CUDART_INF : l;
-}
-
-// log x, -inf for x <= 0; branch-free (a branch would end the basic block and with it the interleaving of the
-// independent evaluations around it)
-PHF_DI double safe_log_t(const double *T, double x)
-{
-    const double l = fm::log_pos(T, x > 0.0 ? x : 1.0);
-    return x > 0.0 ? l : -CUDART_INF;
-}
-
-// log_target_distribution (PyHillFit.py:173-193) for one parameter vector held in registers
+// log_target_distribution (PyHillFit.py:173-193) for one parameter vector held in registers: the Gamma hyper-priors,
+// then the experiments, then the points
 template <int NE>
 PHF_DI double hier_thread_log_target(const double *T, const double (&th)[5 + 2 * NE],
                                      const phf_hier_point *__restrict__ pts, int npts, const phf_hier_priors &pr)
 {
     constexpr int DIM = 5 + 2 * NE;
-    // ---- support (PyHillFit.py:176-183) ----
-    bool bad = !(th[0] > pr.locs[0]) || !(th[1] > pr.locs[1]) || !(th[2] > pr.locs[2]) || !(th[3] > pr.locs[3]) ||
-               !(th[DIM - 1] > pr.locs[4]);
-#pragma unroll
-    for (int e = 0; e < NE; ++e) bad = bad || !(th[4 + 2 * e] >= pr.pic50_lower) || !(th[5 + 2 * e] >= 0.0);
-
+    const bool bad = !hier_in_support<NE>(th, pr);
     const double beta = th[1], mu = th[2], sigma = th[DIM - 1];
-    const double alpha_l = safe_log_t(T, th[0]), beta_l = safe_log_t(T, beta), s_l = safe_log_t(T, th[3]);
-    const double sigma_l = safe_log_t(T, sigma);
+    const double alpha_l = hier_safe_log(T, th[0]), beta_l = hier_safe_log(T, beta), s_l = hier_safe_log(T, th[3]);
+    const double sigma_l = hier_safe_log(T, sigma);
     const double inv_sc = fm::rcp(th[3]);
+    const auto softplus = [T](double a) { return hier_softplus(T, a); };
 
-    // ---- Gamma hyper-priors on (alpha, beta, mu, s, sigma): dr.log_gamma_prior (doseresponse.py:308) ----
     double term = 0.0;
 #pragma unroll
-    for (int q = 0; q < 5; ++q) {
-        const double xm = th[q < 4 ? q : DIM - 1] - pr.locs[q];
-        term += fma(pr.shapes[q] - 1.0, fm::log_pos(T, xm > 0.0 ? xm : 1.0), -xm * (1.0 / pr.scales[q]));
-    }
-    // ---- per-experiment logistic / log-logistic terms (PyHillFit.py:134-154) ----
+    for (int q = 0; q < 5; ++q)
+        term += hier_gamma_prior(T, th[q < 4 ? q : DIM - 1] - pr.locs[q], pr.shapes[q] - 1.0, pr.scales[q]);
     double lic_hi[NE], lic_lo[NE];
 #pragma unroll
     for (int e = 0; e < NE; ++e) {
         const double pic50_e = th[4 + 2 * e], hill_e = th[5 + 2 * e];
         const double zz = (pic50_e - mu) * inv_sc;
-        term += -zz - s_l - 2.0 * softplus_ref_t(T, -zz);
-        const double lh = safe_log_t(T, hill_e);
-        term += beta_l - beta * alpha_l + (beta - 1.0) * lh - 2.0 * softplus_ref_t(T, beta * (lh - alpha_l));
+        term += hier_pic50_term(zz, s_l, softplus);
+        const double lh = hier_safe_log(T, hill_e);
+        term += hier_hill_term(beta, beta_l, alpha_l, lh, softplus);
         ln_ic50(pic50_e, lic_hi[e], lic_lo[e]);
     }
-    // ---- data likelihood, truncated-normal noise (PyHillFit.py:113-125) ----
     const double inv_s = fm::rcp(sigma);
     const double inv2s2 = 0.5 * inv_s * inv_s;
     const double inv_s_rt2 = inv_s * kSqrtHalf;
-    // PU points at a time, predicated instead of looped: the PU evaluations are independent straight-line code in
-    // one basic block, so ptxas interleaves them (a lone warp is otherwise a serial chain of 8-cycle DFMAs)
-#ifndef PHF_HIER_PU
-#define PHF_HIER_PU 1  // (measured: the rolled one-point loop beats 2-4 unrolled points: 22.7 vs 25.1 ms, smaller code)
-#endif
-    constexpr int PU = PHF_HIER_PU;
-    for (int base = 0; base < npts; base += PU) {
-        double contrib[PU];
+    // (one point per trip: measured, two to four predicated points per trip are slower -- 25.1 against 22.7 ms)
+    for (int i = 0; i < npts; ++i) {
+        // (32-byte point as two 16-byte read-only loads; warp-uniform address when the warp's chains share a dataset)
+        const double2 v01 = __ldg(reinterpret_cast<const double2 *>(pts + i));
+        const double2 v23 = __ldg(reinterpret_cast<const double2 *>(pts + i) + 1);
+        const int e = (int)(__double_as_longlong(v23.y) & 0xffffffffll);
+        double lh = lic_hi[0], ll = lic_lo[0], hill_e = th[5];
 #pragma unroll
-        for (int u = 0; u < PU; ++u) {
-            const bool has = base + u < npts;
-            const phf_hier_point *pp = pts + (has ? base + u : 0);
-            // (32-byte point as two 16-byte read-only loads; warp-uniform address when the warp's chains share a dataset)
-            const double2 v01 = __ldg(reinterpret_cast<const double2 *>(pp));
-            const double2 v23 = __ldg(reinterpret_cast<const double2 *>(pp) + 1);
-            const int e = (int)(__double_as_longlong(v23.y) & 0xffffffffll);
-            double lh = lic_hi[0], ll = lic_lo[0], hill_e = th[5];
-#pragma unroll
-            for (int k = 1; k < NE; ++k) {  // (a select chain: the experiment index is data, the arrays are registers)
-                lh = e == k ? lic_hi[k] : lh;
-                ll = e == k ? lic_lo[k] : ll;
-                hill_e = e == k ? th[5 + 2 * k] : hill_e;
-            }
-            const double x = hill_ratio_pow(T, v01.x, v01.y, lh, ll, hill_e);
-            const double p = hill_response(x);
-            const double r = v23.x - p;
-            const double ta = (100.0 - p) * inv_s_rt2, tb = p * inv_s_rt2;
-            const double qa = fm::erfcx_nonneg(T, ta) * fm::exp_clamped(T, -ta * ta);
-            const double qb = fm::erfcx_nonneg(T, tb) * fm::exp_clamped(T, -tb * tb);
-            const double dphi = 1.0 - 0.5 * (qa + qb);
-            const double cb = fma(r * r, inv2s2, safe_log_t(T, dphi)) + sigma_l;
-            contrib[u] = has ? cb : 0.0;
+        for (int k = 1; k < NE; ++k) {  // (a select chain: the experiment index is data, the arrays are registers)
+            lh = e == k ? lic_hi[k] : lh;
+            ll = e == k ? lic_lo[k] : ll;
+            hill_e = e == k ? th[5 + 2 * k] : hill_e;
         }
-#pragma unroll
-        for (int u = 0; u < PU; ++u) term -= contrib[u];
+        term -= hier_point_nll(T, v01.x, v01.y, v23.x, lh, ll, hill_e, inv2s2, inv_s_rt2, sigma_l);
     }
     return bad ? -CUDART_INF : term;
 }
-
-}  // namespace
 
 template <int NE>
 struct HierThreadCfg {
@@ -189,10 +140,7 @@ __global__ void __launch_bounds__(32 * HierThreadCfg<NE>::kMaxWarps) __maxnreg__
     for (uint32_t it = 0; it < cfg.n_iters; ++it) {
         ++t;
         if ((it & 31u) == 0u) {  // gamma_s is a function of t only: lane L computes it for iteration t + L
-            const uint32_t tl = t + (uint32_t)lane;
-            const double g = tl > cfg.adapt_when  // PyHillFit.py:496-497
-                                 ? fm::exp_clamped(T, -0.6 * fm::log_pos(T, (double)(tl - cfg.adapt_when) + 1.0))
-                                 : 0.0;
+            const double g = adapt_gamma(T, t + (uint32_t)lane, cfg.adapt_when);
             __syncwarp();
             gam_slots[lane] = g;
             __syncwarp();
@@ -342,7 +290,6 @@ static int launch_am_hier_thread(const phf_am_config &cfg, int64_t n, double *st
     return check_launch("am_hier_thread_kernel");
 }
 
-// n_expts <= PHF_HIER_THREAD_MAX_EXPTS (phf_hier.cu picks between this and the lane kernel)
 int am_hier_thread_launch(const phf_am_config &cfg, int32_t n_expts, int64_t n, double *state, const int32_t *dataset_id,
                           const phf_hier_dataset *datasets, const phf_hier_point *points, const phf_hier_priors &pr,
                           double *samples, cudaStream_t s)

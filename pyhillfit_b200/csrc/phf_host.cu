@@ -196,17 +196,6 @@ int run_segments(Workspace &w, const phf_am_config *cfg, int64_t n_chains, int d
     return PHF_OK;
 }
 
-int check_common(const phf_am_config *cfg, int32_t device, const char *who)
-{
-    if (cfg->thinning == 0) return set_error(PHF_EINVAL, "cfg.thinning must be >= 1");
-    if (cfg->sample_layout != PHF_SAMPLES_CHAIN_MAJOR && cfg->sample_layout != PHF_SAMPLES_ROW_MAJOR)
-        return set_error(PHF_EINVAL, "cfg.sample_layout must be PHF_SAMPLES_CHAIN_MAJOR or PHF_SAMPLES_ROW_MAJOR");
-    if (device < 0 || device >= 64) return set_error(PHF_EINVAL, "device index outside 0..63");
-    if ((uint64_t)cfg->t0 + cfg->n_iters > 0xFFFFFFFFull) return set_error(PHF_EINVAL, "iteration counter overflow");
-    (void)who;
-    return PHF_OK;
-}
-
 }  // namespace
 
 extern "C" int phf_release_workspaces(void)
@@ -232,14 +221,13 @@ extern "C" int phf_am_single_run_host(const phf_am_config *cfg, int64_t n_chains
 {
     if (!cfg) return set_error(PHF_EINVAL, "phf_am_single_run_host: cfg is NULL");
     if (cfg->model != 1 && cfg->model != 2) return set_error(PHF_EINVAL, "cfg.model must be 1 or 2");
-    if (int rc = check_common(cfg, device, "phf_am_single_run_host")) return rc;
+    if (int rc = check_run_config(*cfg, samples != nullptr)) return rc;
+    if (device < 0 || device >= 64) return set_error(PHF_EINVAL, "device index outside 0..63");
     if (n_chains <= 0 || n_datasets <= 0 || n_groups <= 0 || !state || !dataset_id || !temperature || !datasets ||
         !groups)
         return set_error(PHF_EINVAL, "phf_am_single_run_host: empty or null input");
     if (n_segments < 1) n_segments = 1;
     const int d = cfg->model == 1 ? 2 : 3, nf = PHF_STATE_SIZE(d);
-    if (samples && rows_written(*cfg) > cfg->rows_capacity)
-        return set_error(PHF_EINVAL, "cfg.rows_capacity is smaller than the rows this call produces");
     DeviceGuard guard;
     PHF_TRY(guard.enter(device), "cudaSetDevice");
     Workspace &w = acquire_workspace(device, 0, cfg->model);
@@ -275,7 +263,8 @@ extern "C" int phf_am_hier_run_host(const phf_am_config *cfg, int32_t n_expts, i
 {
     if (!cfg || !priors) return set_error(PHF_EINVAL, "phf_am_hier_run_host: cfg/priors is NULL");
     if (n_expts < 1 || n_expts > PHF_HIER_BIG_MAX_EXPTS) return set_error(PHF_ENOTSUP, "n_expts outside 1..128");
-    if (int rc = check_common(cfg, device, "phf_am_hier_run_host")) return rc;
+    if (int rc = check_run_config(*cfg, samples != nullptr)) return rc;
+    if (device < 0 || device >= 64) return set_error(PHF_EINVAL, "device index outside 0..63");
     if (n_chains <= 0 || n_datasets <= 0 || n_points <= 0 || !state || !dataset_id || !datasets || !points)
         return set_error(PHF_EINVAL, "phf_am_hier_run_host: empty or null input");
     // the host pack is readable here: the checks phf_am_hier_init makes on the device
@@ -294,8 +283,6 @@ extern "C" int phf_am_hier_run_host(const phf_am_config *cfg, int32_t n_expts, i
     }
     if (n_segments < 1) n_segments = 1;
     const int d = 5 + 2 * n_expts, nf = PHF_STATE_SIZE(d);
-    if (samples && rows_written(*cfg) > cfg->rows_capacity)
-        return set_error(PHF_EINVAL, "cfg.rows_capacity is smaller than the rows this call produces");
     DeviceGuard guard;
     PHF_TRY(guard.enter(device), "cudaSetDevice");
     Workspace &w = acquire_workspace(device, 1, n_expts);

@@ -50,6 +50,13 @@ __device__ __forceinline__ double guarded_pivot(double s, double diag)
     return s > fl ? s : fl;  // NaN or non-positive diagonal stays non-positive / NaN -> proposal rejected
 }
 
+// gamma_s = 1/(s+1)**0.6 with s = t - adapt_when, 0 until adaptation starts (PyHillFit.py:496-497, 841-842;
+// PyHillTemp.py:117).  A function of t only: each sampler computes it ahead of the iterations that use it.
+PHF_DI double adapt_gamma(const double *T, uint32_t t, uint32_t adapt_when)
+{
+    return t > adapt_when ? fm::exp_clamped(T, -0.6 * fm::log_pos(T, (double)(t - adapt_when) + 1.0)) : 0.0;
+}
+
 // ---- sub-warp lane groups: G consecutive lanes (G = 1, 2, 4, 8, 16 or 32) cooperate on one chain ----
 template <int G>
 PHF_DI unsigned group_mask()

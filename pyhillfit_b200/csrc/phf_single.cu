@@ -339,10 +339,7 @@ __global__ void __launch_bounds__(128, MINB)
             // gamma_s = 1/(s+1)**0.6, s = t - adapt_when (PyHillFit.py:841-842, PyHillTemp.py:117): a function of t
             // only, so lane L computes it for iteration t + L once every 32 iterations and parks it in shared
             // memory (a per-iteration broadcast LOAD instead of a shuffle: no shuffle point at the top of the loop)
-            const uint32_t tl = t + lane;
-            const double gam_lane = tl > cfg.adapt_when
-                                        ? fm::exp_clamped(T, -0.6 * fm::log_pos(T, (double)(tl - cfg.adapt_when) + 1.0))
-                                        : 0.0;
+            const double gam_lane = adapt_gamma(T, t + lane, cfg.adapt_when);
             __syncwarp();  // every lane has read the previous block's value
             gam_slots[lane] = gam_lane;
             __syncwarp();
@@ -523,14 +520,9 @@ extern "C" int phf_am_single_run(const phf_am_config *cfg, int64_t n_chains, dou
 {
     if (!cfg) return set_error(PHF_EINVAL, "phf_am_single_run: cfg is NULL");
     if (cfg->model != 1 && cfg->model != 2) return set_error(PHF_EINVAL, "cfg.model must be 1 or 2");
-    if (cfg->thinning == 0) return set_error(PHF_EINVAL, "cfg.thinning must be >= 1");
-    if (cfg->sample_layout != PHF_SAMPLES_CHAIN_MAJOR && cfg->sample_layout != PHF_SAMPLES_ROW_MAJOR)
-        return set_error(PHF_EINVAL, "cfg.sample_layout must be PHF_SAMPLES_CHAIN_MAJOR or PHF_SAMPLES_ROW_MAJOR");
+    if (int rc = check_run_config(*cfg, samples != nullptr)) return rc;
     if (n_chains < 0 || (n_chains > 0 && (!state || !dataset_id || !temperature || !datasets || !groups)))
         return set_error(PHF_EINVAL, "phf_am_single_run: null pointer");
-    if ((uint64_t)cfg->t0 + cfg->n_iters > 0xFFFFFFFFull) return set_error(PHF_EINVAL, "iteration counter overflow");
-    if (samples && rows_written(*cfg) > cfg->rows_capacity)
-        return set_error(PHF_EINVAL, "cfg.rows_capacity is smaller than the rows this call produces");
     if (n_chains == 0 || cfg->n_iters == 0) return PHF_OK;
 
     int32_t lanes = 0, depth = 0;

@@ -121,12 +121,7 @@ __global__ void __launch_bounds__(128, 3)
 
     uint32_t t = cfg.t0;  // iterations this chain has completed
     const uint32_t t_end = cfg.t0 + cfg.n_iters;
-    uint32_t until_save = cfg.thinning - (t % cfg.thinning);
-    uint32_t row = t / cfg.thinning;
-    const uint32_t row_base = first_row_written(cfg);
-    const bool row_major = cfg.sample_layout == PHF_SAMPLES_ROW_MAJOR;
-    double *const out = samples ? samples + (row_major ? (size_t)c : (size_t)c * cfg.rows_capacity) * (D + 1) : nullptr;
-    const size_t row_stride = row_major ? (size_t)n * (D + 1) : (size_t)(D + 1);
+    RowCursor rows(cfg, c, n, D, samples);
 
     // ring of prepared iterations: entry (ti % R) of this chain holds ln u, z[0..D), gamma_s of iteration ti
     double *const ring = reinterpret_cast<double *>(smem_raw + (size_t)cfg.stage_groups * sizeof(phf_dose_group)) +
@@ -156,10 +151,7 @@ __global__ void __launch_bounds__(128, 3)
             if ((filled - t) <= (uint32_t)(R - G)) {
                 const uint32_t ti = filled + 1u + (uint32_t)gl;
                 const Draws<D> mine = make_draws<D>(T, cfg.seed, chain_id, ti);
-                // gamma_s = 1/(s+1)**0.6, s = ti - adapt_when (PyHillFit.py:841-842, PyHillTemp.py:117); 0 before
-                const double gam = ti > cfg.adapt_when
-                                       ? fm::exp_clamped(T, -0.6 * fm::log_pos(T, (double)(ti - cfg.adapt_when) + 1.0))
-                                       : 0.0;
+                const double gam = adapt_gamma(T, ti, cfg.adapt_when);
                 double *e = ring + (ti % (uint32_t)R) * W;
                 e[0] = mine.log_u;
 #pragma unroll
@@ -218,14 +210,12 @@ __global__ void __launch_bounds__(128, 3)
 
         // ---- saved rows that fall on a REJECTED iteration of this round (theta, log-target unchanged): iteration
         //      t+j is saved when j = until_save, until_save + thinning, ... (PyHillFit.py:847-848) ----
-        uint32_t j_save = until_save;
+        uint32_t j_save = rows.until_save;
         while (j_save < (uint32_t)k_adv) {
-            ++row;
-            if (out && active && row >= row_base) {
-                double *o = out + (size_t)(row - row_base) * row_stride;
+            ++rows.row;
+            if (double *o = rows.dest(active))
                 for (int k = gl; k <= D; k += G) o[k] = k == 0 ? s.th[0] : (k == 1 ? s.th[1] : (k < D ? s.th[D - 1] : s.lt));
-            }
-            if (row >= cfg.burn_rows) s.l1_sum += s.l1;
+            if (rows.row >= cfg.burn_rows) s.l1_sum += s.l1;
             j_save += cfg.thinning;
         }
 
@@ -264,15 +254,13 @@ __global__ void __launch_bounds__(128, 3)
         }
         // ---- the last committed iteration's row ----
         if (k_adv > 0 && j_save == (uint32_t)k_adv) {
-            ++row;
-            if (out && active && row >= row_base) {
-                double *o = out + (size_t)(row - row_base) * row_stride;
+            ++rows.row;
+            if (double *o = rows.dest(active))
                 for (int k = gl; k <= D; k += G) o[k] = k == 0 ? s.th[0] : (k == 1 ? s.th[1] : (k < D ? s.th[D - 1] : s.lt));
-            }
-            if (row >= cfg.burn_rows) s.l1_sum += s.l1;
+            if (rows.row >= cfg.burn_rows) s.l1_sum += s.l1;
             j_save += cfg.thinning;
         }
-        until_save = j_save - (uint32_t)k_adv;
+        rows.until_save = j_save - (uint32_t)k_adv;
         t += (uint32_t)k_adv;
     }
 

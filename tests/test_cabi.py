@@ -48,6 +48,50 @@ def test_bad_arguments_return_codes_without_a_gpu():
     assert L.phf_hier_log_target_batch(0, None, 17, None, None, None, C.byref(pr), None, None) == 0
 
 
+@pytest.mark.parametrize("fault,message", [
+    (dict(thinning=0), b"cfg.thinning must be >= 1"),
+    (dict(sample_layout=2), b"cfg.sample_layout must be PHF_SAMPLES_CHAIN_MAJOR or PHF_SAMPLES_ROW_MAJOR"),
+    (dict(t0=0xFFFFFFF0, n_iters=0x20), b"iteration counter overflow"),
+    (dict(rows_capacity=9), b"cfg.rows_capacity is smaller than the rows this call produces"),
+])
+def test_run_entry_points_check_the_config_without_a_gpu(fault, message):
+    """The four sampler entry points reject a bad phf_am_config alike, before any CUDA call."""
+    from pyhillfit_b200 import _lib
+    L = _lib.load()
+    fields = dict(model=2, n_iters=100, thinning=10, rows_capacity=10, seed=1)
+    fields.update(fault)
+    cfg = _lib.AmConfig(**fields)
+    n = 4
+    p = lambda a: a.ctypes.data_as(C.c_void_p)
+    samples = np.zeros(n * 10 * 20)
+    dsid = np.zeros(n, dtype=np.int32)
+    # single-level: one dataset of one dose group
+    state = np.zeros(n * _lib.state_size(3))
+    temp = np.ones(n)
+    datasets = np.zeros(1, dtype=_lib.DATASET_DTYPE)
+    datasets["n_groups"] = 1
+    groups = np.zeros(1, dtype=_lib.DOSE_GROUP_DTYPE)
+    # hierarchical: one experiment, one point
+    hstate = np.zeros(n * _lib.state_size(7))
+    hdatasets = np.zeros(1, dtype=_lib.HIER_DATASET_DTYPE)
+    hdatasets["n_points"], hdatasets["n_expts"] = 1, 1
+    points = np.zeros(1, dtype=_lib.HIER_POINT_DTYPE)
+    pr = _lib.HierPriors()
+    calls = {
+        "phf_am_single_run": lambda: L.phf_am_single_run(C.byref(cfg), n, p(state), p(dsid), p(temp), p(datasets),
+                                                         p(groups), p(samples), None),
+        "phf_am_hier_run": lambda: L.phf_am_hier_run(C.byref(cfg), 1, n, p(hstate), p(dsid), p(hdatasets), p(points),
+                                                     C.byref(pr), p(samples), None),
+        "phf_am_single_run_host": lambda: L.phf_am_single_run_host(C.byref(cfg), n, p(state), p(dsid), p(temp), 1,
+                                                                   p(datasets), 1, p(groups), p(samples), 1, 0),
+        "phf_am_hier_run_host": lambda: L.phf_am_hier_run_host(C.byref(cfg), 1, n, p(hstate), p(dsid), 1, p(hdatasets),
+                                                               1, p(points), C.byref(pr), p(samples), 1, 0),
+    }
+    for name, call in calls.items():
+        assert call() == -1, name  # PHF_EINVAL
+        assert L.phf_last_error() == message, name
+
+
 def test_struct_layouts_match_the_header(tmp_path):
     from pyhillfit_b200 import _lib
     prog = tmp_path / "sizes.c"
