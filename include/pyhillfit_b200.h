@@ -175,6 +175,34 @@ int phf_am_single_run(const phf_am_config *cfg, int64_t n_chains, double *state,
                       double *samples, void *stream);
 
 /* ------------------------------------------------------------------------------------------------
+ * Population MCMC (state swaps between neighbouring temperatures) for the tempered single-level sampler: one swap
+ * round on the state rows, run between two phf_am_single_run launches (the sampler kernels do not change, and a launch
+ * resumes bit for bit from the state rows).  Executable statement: tests/swap_oracle.py:swap_round.
+ *   ladder_chains  [n_ladders][ladder_len] chain indices (int64).  A ladder is an ordered list of chain slots of ONE
+ *                  dataset with strictly increasing temperature[] (t_0 < t_1 < ...); no chain in two slots.  The
+ *                  caller validates the map (pyhillfit_b200/sampler.py:validate_ladders); an entry outside
+ *                  [0, n_chains) makes its pairs no-ops.
+ *   Schedule       the round that follows iteration t = sK (swap every K iterations, s = 1, 2, ...) tries the pairs
+ *                  (k, k+1) with k = parity (mod 2), parity = s mod 2.  The pairs of one round are disjoint.
+ *   Acceptance     accept iff ln u < (t_k - t_k+1) (l1(x_k+1) - l1(x_k)) with the loglik_t1 stored in the two state
+ *                  rows (the prior cancels); a non-finite l1 on either side rejects.  u = uniform53 of words 0-1 of
+ *                  philox_call(seed, ladder_id_base + ladder, t, PHF_SWAP_CALL0 + k) -- a call index the samplers
+ *                  never use; ladder ids are GLOBAL, so results do not depend on how ladders are split over ranks.
+ *   Accepted swap  theta moves between the two slots; each slot's (log_target, loglik_t1) is re-evaluated for its new
+ *                  theta at its own temperature with the function phf_log_target_batch uses (the same bits).  Mean,
+ *                  covariance, loga, loglik_t1_sum and n_accepted stay with the slot (each slot keeps its temperature,
+ *                  so chain files and thermodynamic-integration sums still belong to one temperature).
+ *   swap_counts    DEVICE, may be NULL: int64 [n_ladders][ladder_len - 1][2] (attempted, accepted) per adjacent pair,
+ *                  accumulated.
+ * Arguments are checked before any CUDA call (PHF_EINVAL).  Asynchronous on `stream`; allocates nothing.
+ * ---------------------------------------------------------------------------------------------- */
+#define PHF_SWAP_CALL0 0x80000000u
+int phf_am_single_swap(int model, int64_t n_chains, double *state, const int32_t *dataset_id,
+                       const double *temperature, const phf_dataset *datasets, const phf_dose_group *groups,
+                       int64_t n_ladders, int32_t ladder_len, const int64_t *ladder_chains, uint64_t seed,
+                       uint64_t ladder_id_base, uint32_t t, int32_t parity, int64_t *swap_counts, void *stream);
+
+/* ------------------------------------------------------------------------------------------------
  * Hierarchical model (python/PyHillFit.py:113-154, 173-193, 481-511).
  * theta = (alpha, beta, mu, s, pIC50_1, Hill_1, ..., pIC50_Ne, Hill_Ne, sigma), dim = 5 + 2 Ne.
  * ---------------------------------------------------------------------------------------------- */

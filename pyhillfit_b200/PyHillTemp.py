@@ -3,7 +3,7 @@ temperature ladder for one (drug index, channel index), all temperatures in one 
 
 Same flags as the reference (note: here -c is the CHANNEL index and -nc the core count, as in the reference).
 Writes one header-less chain file per temperature with the float temperature in the path (PyHillTemp.py:165-169).
-New optional flags: --num-chains (replicates per temperature), --seed, --segment.
+New optional flags: --num-chains (replicates per temperature), --seed, --segment, --diagnostics, --swap-every.
 """
 import argparse
 import sys
@@ -31,6 +31,10 @@ def build_parser():
     parser.add_argument("--diagnostics", action='store_true', default=False,
                         help="split R-hat and multi-chain ESS of each temperature's chains, computed on the GPU, "
                              "written beside the chain file as ..._diagnostics.txt [new]")
+    parser.add_argument("--swap-every", type=int, default=0,
+                        help="population MCMC: neighbouring temperatures of each replicate's ladder exchange states "
+                             "after every K-th iteration; per-rung swap acceptance is printed and written to "
+                             "..._swap_acceptance.txt in the model directory (0: independent chains) [new]")
     requiredNamed = parser.add_argument_group('required arguments')
     requiredNamed.add_argument("--data-file", type=str, required=True)
     requiredNamed.add_argument("-m", "--model", type=int, required=True)
@@ -41,8 +45,9 @@ def build_parser():
 
 def do_mcmc_all_temperatures(dr, args, concs, responses, temperatures):
     """python/PyHillTemp.py:57-125 for every temperature (x replicates) at once -> [T, R, rows, d+1] host array
-    of post-burn rows, the in-kernel mean temperature-1 log-likelihoods [T, R] and, with --diagnostics, the
-    [T, d+1, 5] diagnostics of each temperature's R chains (else None)."""
+    of post-burn rows, the in-kernel mean temperature-1 log-likelihoods [T, R], with --diagnostics the
+    [T, d+1, 5] diagnostics of each temperature's R chains (else None) and, with --swap-every, the [R, T-1, 2]
+    (attempted, accepted) swap counts of each replicate's ladder (else None)."""
     import torch
     from .packing import SinglePack
     from .sampler import SingleLevelSampler
@@ -65,10 +70,12 @@ def do_mcmc_all_temperatures(dr, args, concs, responses, temperatures):
     if burn == 0:
         chain[:, 0, :] = s.initial_row()
         at = 1
+    # --swap-every: ladder r is the R-strided column of replicate r, global id (model - 1) 2^40 + r (pair 0 of ti.run_ti)
+    ladders = np.arange(T * R).reshape(T, R).T
     done = 0
     while done < args.iterations:
         k = min(args.segment - args.segment % args.thinning or args.thinning, args.iterations - done)
-        seg = s.run(k, discard_burn=True)
+        seg = s.run_swapping(k, args.swap_every, ladders, (args.model - 1) * (1 << 40), discard_burn=True)
         chain[:, at:at + seg.shape[1], :] = seg
         at += seg.shape[1]
         done += k
@@ -77,7 +84,8 @@ def do_mcmc_all_temperatures(dr, args, concs, responses, temperatures):
     from .PyHillFit import run_diagnostics
     diag = run_diagnostics(args, chain, T, R, 0)
     host = chain.cpu().numpy().reshape(T, R, kept, d + 1)
-    return host, s.loglik_t1_mean().reshape(T, R), diag
+    counts = s.swap_counts.cpu().numpy() if args.swap_every > 0 else None
+    return host, s.loglik_t1_mean().reshape(T, R), diag, counts
 
 
 def main(argv=None):
@@ -98,7 +106,9 @@ def main(argv=None):
     temperatures = (np.arange(dr.n + 1.) / dr.n) ** dr.c
     print("\nDoing temperatures: {}\n".format(temperatures))
     start = time.time()
-    chains, ll1, diag = do_mcmc_all_temperatures(dr, args, concs, responses, temperatures)
+    if args.swap_every < 0:
+        parser.error("--swap-every must be >= 0")
+    chains, ll1, diag, swaps = do_mcmc_all_temperatures(dr, args, concs, responses, temperatures)
     print("\nMCMC time: {} s\n".format(int(time.time() - start)))
     for i, temperature in enumerate(temperatures):
         cdrug, cchannel, chain_file, images_dir = dr.nonhierarchical_chain_file_and_figs_dir(args.model, drug, channel, temperature)
@@ -109,6 +119,12 @@ def main(argv=None):
         if diag is not None:
             names = ["pIC50", "sigma"] if args.model == 1 else ["pIC50", "Hill", "sigma"]
             chainio.save_diagnostics(chain_file, diag[i], names + ["log-target"], args.num_chains, 0, chains.shape[2])
+    if swaps is not None:
+        f, acc = chainio.save_swap_acceptance(chain_file, temperatures, swaps, args.swap_every)
+        print("swap acceptance per rung (t_k, t_k+1), pooled over {} ladder(s):".format(args.num_chains))
+        for k in range(len(temperatures) - 1):
+            print("  {:.6g} <-> {:.6g}: {:.3f}".format(temperatures[k], temperatures[k + 1], acc[k]))
+        print("swap acceptance file:", f)
     return 0
 
 

@@ -52,7 +52,7 @@ EXPORTS = ["phf_log_target_batch", "phf_am_single_init", "phf_am_single_run", "p
            "phf_release_workspaces", "phf_best_fit_batch",
            "phf_write_rows_text_host",
            "phf_hier_predictive_cdfs", "phf_format_e18", "phf_format_e18_mismatches", "phf_version", "phf_last_error",
-           "phf_fp64_peak_probe", "phf_launch_count", "phf_chain_diagnostics"]
+           "phf_fp64_peak_probe", "phf_launch_count", "phf_chain_diagnostics", "phf_am_single_swap"]
 
 _lib = None
 _p = C.c_void_p
@@ -82,6 +82,8 @@ def load():
     L.phf_am_single_shape.argtypes = [C.c_int64, C.c_int32, C.c_int32, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]
     L.phf_am_single_resident_ctas.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int64]
     L.phf_am_single_run.argtypes = [C.POINTER(AmConfig), C.c_int64, _p, _p, _p, _p, _p, _p, _p]
+    L.phf_am_single_swap.argtypes = [C.c_int, C.c_int64, _p, _p, _p, _p, _p, C.c_int64, C.c_int32, _p, C.c_uint64,
+                                     C.c_uint64, C.c_uint32, C.c_int32, _p, _p]
     L.phf_hier_log_target_batch.argtypes = [C.c_int64, _p, C.c_int32, _p, _p, _p, C.POINTER(HierPriors), _p, _p]
     L.phf_am_hier_lanes.argtypes = [C.c_int32, C.c_int64]
     L.phf_am_hier_init.argtypes = [C.c_int32, C.c_int64, _p, _p, _p, _p, _p, C.POINTER(HierPriors), _p, _p]

@@ -87,3 +87,27 @@ def save_diagnostics(chain_file, diag, names, n_chains, row_begin, row_end):
         for name, (mean, sd, rhat, ess, lags) in zip(names, diag):
             out.write("{} {:.18e} {:.18e} {:.18e} {:.18e} {:d}\n".format(name, mean, sd, rhat, ess, int(lags)))
     return f
+
+
+def swap_acceptance_name(chain_file):
+    """File of the per-rung swap acceptance of one (drug, channel, model) ladder run (PyHillTemp --swap-every): in the
+    model directory that holds the temperature_* directories, named after the chain file without its temperature."""
+    model_dir = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(chain_file))))
+    name = os.path.basename(chain_file).split("_temp_")[0]
+    return os.path.join(model_dir, name + "_swap_acceptance.txt")
+
+
+def save_swap_acceptance(chain_file, temps, counts, swap_every):
+    """counts [R, T-1, 2] (attempted, accepted) -> one line per adjacent pair: t_k, t_k+1, attempted, accepted,
+    acceptance (pooled over the R ladders).  Returns (file, acceptance [T-1])."""
+    c = np.asarray(counts, dtype=np.int64).sum(axis=0)
+    with np.errstate(invalid="ignore", divide="ignore"):
+        acc = np.where(c[:, 0] > 0, c[:, 1] / np.maximum(c[:, 0], 1), np.nan)
+    f = swap_acceptance_name(chain_file)
+    with open(f, "w") as out:
+        out.write("# population MCMC: swaps between neighbouring temperatures every {} iterations, {} ladder(s)\n"
+                  .format(swap_every, np.asarray(counts).shape[0]))
+        out.write("# t_k t_k+1 attempted accepted acceptance\n")
+        for k in range(c.shape[0]):
+            out.write("{:.18e} {:.18e} {:d} {:d} {:.6f}\n".format(temps[k], temps[k + 1], c[k, 0], c[k, 1], acc[k]))
+    return f, acc

@@ -22,6 +22,9 @@ def build_parser():
     parser.add_argument("-i", "--iterations", type=int, default=500000, help="--all-fused: iterations per chain")
     parser.add_argument("-t", "--thinning", type=int, default=5, help="--all-fused: thinning")
     parser.add_argument("--seed", type=int, default=1, help="--all-fused: Philox seed")
+    parser.add_argument("--swap-every", type=int, default=0,
+                        help="--all-fused: population MCMC, neighbouring temperatures of each pair's ladder exchange "
+                             "states after every K-th iteration (0: independent chains)")
     requiredNamed = parser.add_argument_group('required arguments')
     requiredNamed.add_argument("-d", "--drug", type=int, help="drug index (not needed with --all-fused)")
     requiredNamed.add_argument("-c", "--channel", type=int, help="channel index (not needed with --all-fused)")
@@ -50,11 +53,17 @@ def run_all_fused(dr, args):
         jobs.append((drug, channel))
         data.append((concs, responses))
     phf_dist.init_process_group()          # (a no-op for a single process)
-    res = run_ti(data, iterations=args.iterations, thinning=args.thinning, seed=args.seed)
+    if args.swap_every < 0:
+        raise SystemExit("--swap-every must be >= 0")
+    res = run_ti(data, iterations=args.iterations, thinning=args.thinning, seed=args.seed, swap_every=args.swap_every)
     if phf_dist.world()[1] == 0:
         for (drug, channel), Bij in zip(jobs, res["B12"]):
             chainio.save_bayes_factor(drug, channel, Bij)
         print("{} Bayes factors written to BFs/".format(len(jobs)))
+        if args.swap_every > 0:
+            for m in sorted(res["swap_acceptance"]):
+                acc = np.nanmean(res["swap_acceptance"][m], axis=(0, 1))
+                print("model {} swap acceptance per rung, mean over pairs: {}".format(m, np.array2string(acc, precision=3)))
     import torch.distributed as td
     if td.is_available() and td.is_initialized():
         td.barrier()

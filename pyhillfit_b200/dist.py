@@ -29,6 +29,16 @@ def shard_bounds(weights, world_size):
     return np.maximum.accumulate(bounds)
 
 
+def shard_bounds_by_group(weights, group_size, world_size):
+    """shard_bounds for a chain list made of consecutive groups of `group_size` chains that must stay on one rank (the
+    T x R chains of one pair, whose ladders swap states): the groups are balanced by their total weight and every
+    bound is a multiple of group_size."""
+    w = np.asarray(weights, dtype=np.float64)
+    if group_size < 1 or len(w) % group_size:
+        raise ValueError("the chain list must be whole groups of group_size chains")
+    return shard_bounds(w.reshape(-1, group_size).sum(axis=1), world_size) * group_size
+
+
 def init_process_group(backend=None):
     import torch
     import torch.distributed as dist

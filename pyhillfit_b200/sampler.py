@@ -47,6 +47,32 @@ def tri_unpack(tri, d):
     return out
 
 
+def validate_ladders(ladders, dataset_id, temperature):
+    """The ladder map of population MCMC (SingleLevelSampler.run_swapping), checked on the host before it is uploaded:
+    [n_ladders, T >= 2] chain indices in [0, n), no chain in two slots, one dataset per ladder, temperatures strictly
+    increasing along each ladder.  Returns it as a C-contiguous int64 array; raises ValueError otherwise."""
+    lad = np.asarray(ladders)
+    if lad.ndim != 2 or lad.shape[1] < 2:
+        raise ValueError("ladders must be [n_ladders, T] with T >= 2")
+    if lad.size and not np.issubdtype(lad.dtype, np.integer):
+        raise ValueError("ladders must hold integer chain indices")
+    lad = np.ascontiguousarray(lad, dtype=np.int64)
+    ids = np.asarray(dataset_id).reshape(-1)
+    temps = np.asarray(temperature, dtype=np.float64).reshape(-1)
+    n = len(ids)
+    if lad.size == 0:
+        return lad
+    if lad.min() < 0 or lad.max() >= n:
+        raise ValueError("ladder entries must be chain indices in [0, %d)" % n)
+    if len(np.unique(lad)) != lad.size:
+        raise ValueError("a chain appears in more than one ladder slot")
+    if np.any(ids[lad] != ids[lad[:, :1]]):
+        raise ValueError("every chain of a ladder must have the same dataset")
+    if not np.all(temps[lad[:, 1:]] > temps[lad[:, :-1]]):
+        raise ValueError("temperatures must increase strictly along every ladder")
+    return lad
+
+
 class _Base:
     d = None
 
@@ -132,6 +158,7 @@ class SingleLevelSampler(_Base):
             raise ValueError("dataset_id must be [n] with values in [0, n_datasets)")
         self.dataset_id = torch.from_numpy(ids).to(self.device)
         self.temperature = torch.from_numpy(temps).to(self.device)
+        self._ids_host, self._temps_host = ids, temps
         self.ds_dev, self.groups_dev = pack.device(self.device)
         L = _lib.load()
         if lanes not in (0, 1, 2, 4):
@@ -200,6 +227,74 @@ class SingleLevelSampler(_Base):
         if not keep:
             return None
         return samples[:rows] if row_major else samples[:, :rows]
+
+    def run_swapping(self, n_iters, swap_every, ladders, ladder_id_base=0, samples=None, keep=True, row_major=False,
+                     discard_burn=False):
+        """run(n_iters, ...) with population MCMC: after every iteration t = s * swap_every (s = 1, 2, ...) one swap
+        round (phf_am_single_swap) exchanges states between neighbouring temperatures of each ladder.
+        ladders: [n_ladders, T] chain indices, each row one dataset in strictly increasing temperature (checked by
+        validate_ladders); ladder i has the global id ladder_id_base + i.  n_iters need not be a multiple of
+        swap_every: the schedule is on the global iteration counter, so split calls give the same chains.
+        swap_every <= 0 is run() itself.  The (attempted, accepted) counts of each adjacent pair accumulate in
+        self.swap_counts (int64 device tensor [n_ladders, T-1, 2]; reset when the ladder map changes).
+        Returns what run() returns."""
+        if swap_every <= 0:
+            return self.run(n_iters, samples, keep, row_major, discard_burn)
+        torch = self.torch
+        K = int(swap_every)
+        key = (np.asarray(ladders).tobytes(), np.shape(ladders), int(ladder_id_base))
+        if getattr(self, "_ladder_key", None) != key:
+            lad = validate_ladders(ladders, self._ids_host, self._temps_host)
+            self._ladders = torch.from_numpy(lad).to(self.device)
+            self.swap_counts = torch.zeros((lad.shape[0], lad.shape[1] - 1, 2), dtype=torch.int64, device=self.device)
+            self._ladder_key = key
+        rows = self.rows_for(n_iters, discard_burn)
+        ax_n, ax_r = (1, 0) if row_major else (0, 1)
+        if keep:
+            if samples is None:
+                shape = (max(rows, 1), self.n, self.d + 1) if row_major else (self.n, max(rows, 1), self.d + 1)
+                samples = torch.empty(shape, dtype=torch.float64, device=self.device)
+            assert samples.shape[ax_n] == self.n and samples.shape[2] == self.d + 1 and samples.shape[ax_r] >= rows
+        L = _lib.load()
+        end, at = self.t + int(n_iters), 0
+        lad = self._ladders
+        with torch.cuda.device(self.device):
+            stream = _lib.current_stream_ptr()
+            # (thermodynamic-integration runs keep no rows: one launch pair per interval with as little host work as
+            #  possible -- at K = 100 an interval is ~60 us of device time)
+            cfg = self._config(0, 0)
+            while self.t < end:
+                k = min((self.t // K + 1) * K, end) - self.t
+                if keep:
+                    r = self.rows_for(k, discard_burn)
+                    if row_major:                  # rows of all chains contiguous: the launch writes into the buffer
+                        self.run(k, samples=samples[at:at + r] if r > 0 else samples[:1], row_major=True,
+                                 discard_burn=discard_burn)
+                    else:
+                        samples[:, at:at + r] = self.run(k, discard_burn=discard_burn)
+                    at += r
+                else:
+                    cfg.t0, cfg.n_iters = self.t, k
+                    _lib.check(L.phf_am_single_run(C.byref(cfg), self.n, self.state.data_ptr(), self.dataset_id.data_ptr(),
+                                                   self.temperature.data_ptr(), self.ds_dev.data_ptr(),
+                                                   self.groups_dev.data_ptr(), None, stream), "phf_am_single_run")
+                    self.t += k
+                if self.t % K == 0:
+                    _lib.check(L.phf_am_single_swap(self.model, self.n, self.state.data_ptr(), self.dataset_id.data_ptr(),
+                                                    self.temperature.data_ptr(), self.ds_dev.data_ptr(),
+                                                    self.groups_dev.data_ptr(), lad.shape[0], lad.shape[1],
+                                                    lad.data_ptr(), int(self.seed), int(ladder_id_base), self.t,
+                                                    (self.t // K) & 1, self.swap_counts.data_ptr(), stream),
+                               "phf_am_single_swap")
+        if not keep:
+            return None
+        return samples[:rows] if row_major else samples[:, :rows]
+
+    def swap_acceptance(self):
+        """[n_ladders, T-1] accepted / attempted swaps of each adjacent pair so far (nan where none was attempted)."""
+        c = self.swap_counts.cpu().numpy().astype(np.float64)
+        with np.errstate(invalid="ignore", divide="ignore"):
+            return np.where(c[..., 0] > 0, c[..., 1] / c[..., 0], np.nan)
 
     def loglik_t1_mean(self):
         """Mean over counted rows of the temperature-1 log-likelihood (compute_bayes_factors.py:11-27)."""

@@ -37,15 +37,34 @@ def log_py_from_means(temps, means):
     return 0.5 * np.sum((temps[1:] - temps[:-1]) * (means[..., 1:] + means[..., :-1]), axis=-1)
 
 
+def pair_ladders(pair_lo, pair_hi, T, R):
+    """Ladders of population MCMC over the chain list of build_chain_list restricted to pairs [pair_lo, pair_hi):
+    [(pair_hi - pair_lo) R, T] local chain indices, one ladder per (pair, replicate) in that order, so ladder
+    (pair, r) has local index (pair - pair_lo) R + r."""
+    p = np.arange(pair_hi - pair_lo)[:, None, None]
+    r = np.arange(R)[None, :, None]
+    t = np.arange(T)[None, None, :]
+    return ((p * T + t) * R + r).reshape(-1, T)
+
+
+def ladder_id_base(model, pair_lo, R):
+    """Global id of ladder (pair_lo, 0) of `model`: ladder (pair, r) is (model - 1) 2^40 + pair R + r."""
+    return (model - 1) * (1 << 40) + pair_lo * R
+
+
 def run_ti(datasets, models=(1, 2), temps=None, replicates=1, iterations=500000, thinning=5, burn_in_fraction=4,
-           seed=1, segment=50000, device=None, progress=None, lanes=0, pack=None, speculation=0):
+           seed=1, segment=50000, device=None, progress=None, lanes=0, pack=None, speculation=0, swap_every=0):
     """datasets: list of (concs, responses).  Returns dict with log_py[model] -> [n_pairs], B12 [n_pairs],
     means[model] -> [n_pairs, T] (averaged over replicates), acceptance[model] -> [n_pairs, T, R].
     Under torch.distributed (one process per GPU) the global chain list is sharded contiguously over the ranks and
     every rank returns the full result; with a fixed `lanes` the result does not depend on the number of ranks.
     `pack`: the SinglePack of `datasets` if the caller already has it.  The whole call is ordered after the work
     already queued on the current CUDA stream and is complete (host results in hand) when it returns, so CUDA events
-    recorded on the current stream around it time the sampling, the all-gathers and the integration."""
+    recorded on the current stream around it time the sampling, the all-gathers and the integration.
+    swap_every = K > 0: population MCMC -- the T temperatures of each (pair, replicate) form a ladder whose neighbours
+    exchange states after every K-th iteration (SingleLevelSampler.run_swapping); the chains of a pair then stay on
+    one rank (dist.shard_bounds_by_group) and swap_acceptance[model] -> [n_pairs, R, T-1] is returned as well.
+    swap_every = 0 runs independent chains."""
     import torch
     temps = temperature_ladder() if temps is None else np.asarray(temps, dtype=np.float64)
     ws, rank, local = phf_dist.world()
@@ -56,7 +75,10 @@ def run_ti(datasets, models=(1, 2), temps=None, replicates=1, iterations=500000,
     out = {"temps": temps, "means": {}, "log_py": {}, "acceptance": {}}
     dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
     ids, tt = build_chain_list(n_pairs, temps, R)
-    bounds = phf_dist.shard_bounds(pack.dataset_cost()[ids], ws)   # ranks get equal work, not equal chain counts
+    if swap_every > 0:     # a pair's ladders swap states: all its chains on one rank
+        bounds = phf_dist.shard_bounds_by_group(pack.dataset_cost()[ids], T * R, ws)
+    else:
+        bounds = phf_dist.shard_bounds(pack.dataset_cost()[ids], ws)   # ranks get equal work, not equal chain counts
     lo, hi = int(bounds[rank]), int(bounds[rank + 1])
     # the models are independent: their launches go to separate streams and share the SMs
     samplers, streams = {}, {}
@@ -74,6 +96,18 @@ def run_ti(datasets, models=(1, 2), temps=None, replicates=1, iterations=500000,
         for model in models:
             streams[model].wait_stream(cur)
         done = 0
+        if swap_every > 0:
+            ladders = pair_ladders(lo // (T * R), hi // (T * R), T, R)
+            while done < iterations:
+                # one swap interval at a time, both models, so that neither stream's launches queue behind the other's
+                k = min((done // swap_every + 1) * swap_every, iterations) - done
+                for model in models:
+                    with torch.cuda.stream(streams[model]):
+                        samplers[model].run_swapping(k, swap_every, ladders, ladder_id_base(model, lo // (T * R), R),
+                                                     keep=False)
+                done += k
+                if progress and (done % segment == 0 or done == iterations):
+                    progress(done, iterations)
         while done < iterations:
             k = min(segment, iterations - done)
             for model in models:
@@ -106,6 +140,16 @@ def run_ti(datasets, models=(1, 2), temps=None, replicates=1, iterations=500000,
         out["means_per_replicate_%d" % model] = means
         out["acceptance"][model] = acc
         out["log_py"][model] = log_py_from_means(temps, out["means"][model])
+        if swap_every > 0:
+            if hi > lo:
+                local_counts = samplers[model].swap_counts.to(torch.float64).reshape(-1)
+            else:
+                local_counts = torch.zeros(0, dtype=torch.float64, device=dev)
+            counts = phf_dist.all_gather_varlen(local_counts, bounds // T * (T - 1) * 2).cpu().numpy()
+            counts = counts.reshape(n_pairs, R, T - 1, 2)
+            with np.errstate(invalid="ignore", divide="ignore"):
+                out.setdefault("swap_acceptance", {})[model] = np.where(counts[..., 0] > 0,
+                                                                         counts[..., 1] / counts[..., 0], np.nan)
     out["gather_seconds"] = time.perf_counter() - t_gather    # all-gathers + trapezium rule (first call: NCCL start-up)
     if 1 in out["log_py"] and 2 in out["log_py"]:
         out["B12"] = np.exp(out["log_py"][1] - out["log_py"][2])  # compute_bayes_factors.py:94
