@@ -33,6 +33,14 @@ class AmConfig(C.Structure):                                                    
                 ("discard_burn_rows", C.c_int32), ("speculation", C.c_int32)]
 
 
+def state_offsets(d):
+    """Columns of a chain-state row (the PHF_STATE_* offsets of include/pyhillfit_b200.h)"""
+    cov = 2 * d + 2
+    loga = cov + d * (d + 1) // 2
+    return dict(theta=slice(0, d), log_target=d, loglik_t1=d + 1, mean=slice(d + 2, cov), cov=slice(cov, loga),
+                loga=loga, loglik_t1_sum=loga + 1, n_accepted=loga + 2)
+
+
 def _check(rc):
     if rc:
         raise RuntimeError(_phf.phf_last_error().decode())
@@ -96,14 +104,14 @@ def run_single_level_loop(model, concs, responses, theta0, cov0, log_target0, lo
     pi_bit = 0.5 * len(wo) * np.log(2 * np.pi)                      # doseresponse.py:299-301 called with the mask
     g, ds = pack(y, w0, w100, wo, concs, pi_bit)
     d = len(theta0)
-    nt = d * (d + 1) // 2
     n = len(temperatures)
-    state = np.zeros((n, 2 * d + nt + 5))    # PHF_STATE_SIZE(d): theta, lt, ll1, mean, cov(tri), loga, sum, n_acc
-    state[:, :d] = theta0
-    state[:, d] = log_target0
-    state[:, d + 1] = loglik_t1_0
-    state[:, d + 2:2 * d + 2] = theta0
-    state[:, 2 * d + 2:2 * d + 2 + nt] = np.asarray(cov0)[np.tril_indices(d)]
+    off = state_offsets(d)
+    state = np.zeros((n, off["n_accepted"] + 1))    # PHF_STATE_SIZE(d)
+    state[:, off["theta"]] = theta0
+    state[:, off["log_target"]] = log_target0
+    state[:, off["loglik_t1"]] = loglik_t1_0
+    state[:, off["mean"]] = theta0
+    state[:, off["cov"]] = np.asarray(cov0)[np.tril_indices(d)]
     rows = iterations // thinning
     samples = np.empty((n, rows, d + 1))
     cfg = AmConfig(model=model, reset_mean_at_adapt=int(variant == "temp"), t0=0, n_iters=iterations,

@@ -85,7 +85,16 @@ int phf_log_target_batch(int model, int64_t n, const double *theta, const int32_
  *   loglik_t1_sum (over saved rows with index >= burn_rows), n_accepted
  * RNG: Philox4x32-10, key = seed, counter = (iteration, call, chain_id lo, chain_id hi); the stream
  * contract is written out in oracle/hill_oracle.py (the oracle reproduces GPU trajectories with it).
+ * Offsets of the fields in a row (theta at 0); every reader of the row indexes it through these.
  * ---------------------------------------------------------------------------------------------- */
+#define PHF_STATE_LOG_TARGET(d) (d)
+#define PHF_STATE_LOGLIK_T1(d) ((d) + 1)
+#define PHF_STATE_MEAN(d) ((d) + 2)
+#define PHF_STATE_COV(d) (2 * (d) + 2)
+#define PHF_STATE_LOGA(d) (PHF_STATE_COV(d) + (d) * ((d) + 1) / 2)
+#define PHF_STATE_LOGLIK_T1_SUM(d) (PHF_STATE_LOGA(d) + 1)
+#define PHF_STATE_N_ACCEPTED(d) (PHF_STATE_LOGA(d) + 2)
+/* = PHF_STATE_N_ACCEPTED(d) + 1, written out: the grouping of the run-time-d expression decides the code nvcc emits */
 #define PHF_STATE_SIZE(d) (2 * (d) + (d) * ((d) + 1) / 2 + 5)
 
 typedef struct phf_am_config {

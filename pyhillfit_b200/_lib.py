@@ -58,8 +58,17 @@ _lib = None
 _p = C.c_void_p
 
 
+def state_offsets(d):
+    """Where the fields of a chain-state row are (the PHF_STATE_* offsets of include/pyhillfit_b200.h): slices for
+    theta, mean and cov (lower triangle, row-major), column indices for the scalar fields."""
+    cov = 2 * d + 2
+    loga = cov + d * (d + 1) // 2
+    return dict(theta=slice(0, d), log_target=d, loglik_t1=d + 1, mean=slice(d + 2, cov), cov=slice(cov, loga),
+                loga=loga, loglik_t1_sum=loga + 1, n_accepted=loga + 2)
+
+
 def state_size(d):
-    return 2 * d + d * (d + 1) // 2 + 5
+    return state_offsets(d)["n_accepted"] + 1
 
 
 def load():

@@ -226,22 +226,22 @@ __global__ void __launch_bounds__(128) am_hier_init_kernel(int32_t dim, int64_t 
     double *s = state + i * nf;
     if (gl < dim) {
         s[gl] = th_j;
-        s[dim + 2 + gl] = th_j;
+        s[PHF_STATE_MEAN(dim) + gl] = th_j;
     }
-    for (int k = gl; k < nt; k += G) s[2 * dim + 2 + k] = cov0[i * nt + k];
+    for (int k = gl; k < nt; k += G) s[PHF_STATE_COV(dim) + k] = cov0[i * nt + k];
     __syncwarp();
     // a non-positive diagonal entry of cov0 becomes PHF_COV0_DIAG_FLOOR (include/pyhillfit_b200.h)
     if (gl < dim) {
         const int q = gl * (gl + 1) / 2 + gl;
         const double v = cov0[i * nt + q];
-        if (!(v > 0.0) && v == v) s[2 * dim + 2 + q] = PHF_COV0_DIAG_FLOOR;
+        if (!(v > 0.0) && v == v) s[PHF_STATE_COV(dim) + q] = PHF_COV0_DIAG_FLOOR;
     }
     if (gl == 0) {
-        s[dim] = lt;
-        s[dim + 1] = 0.0;
-        s[2 * dim + 2 + nt] = 0.0;
-        s[2 * dim + 2 + nt + 1] = 0.0;
-        s[2 * dim + 2 + nt + 2] = 0.0;
+        s[PHF_STATE_LOG_TARGET(dim)] = lt;
+        s[PHF_STATE_LOGLIK_T1(dim)] = 0.0;
+        s[PHF_STATE_LOGA(dim)] = 0.0;
+        s[PHF_STATE_LOGLIK_T1_SUM(dim)] = 0.0;
+        s[PHF_STATE_N_ACCEPTED(dim)] = 0.0;
     }
 }
 
@@ -281,13 +281,13 @@ __global__ void __launch_bounds__(128, hier_min_ctas(DIM)) am_hier_kernel(phf_am
     double *sp = state + c * NF;
     const bool row_ok = gl < DIM;
     double th_j = row_ok ? sp[gl] : 1.0;
-    double mean_j = row_ok ? sp[DIM + 2 + gl] : 1.0;
-    double lt = sp[DIM];
+    double mean_j = row_ok ? sp[PHF_STATE_MEAN(DIM) + gl] : 1.0;
+    double lt = sp[PHF_STATE_LOG_TARGET(DIM)];
     double crow[DIM];
 #pragma unroll
-    for (int k = 0; k < DIM; ++k) crow[k] = (row_ok && k <= gl) ? sp[2 * DIM + 2 + gl * (gl + 1) / 2 + k] : 0.0;
-    double loga = sp[2 * DIM + 2 + NT];
-    double n_acc = sp[2 * DIM + 2 + NT + 2];
+    for (int k = 0; k < DIM; ++k) crow[k] = (row_ok && k <= gl) ? sp[PHF_STATE_COV(DIM) + gl * (gl + 1) / 2 + k] : 0.0;
+    double loga = sp[PHF_STATE_LOGA(DIM)];
+    double n_acc = sp[PHF_STATE_N_ACCEPTED(DIM)];
 
     // ---- draws (contract: oracle/hill_oracle.py): normal pair q feeds parameters 2q, 2q+1; they depend on t only, so
     //      the G lanes prepare TWO iterations at a time: lane L < G/2 makes pair L of iteration t, lane L >= G/2 pair
@@ -378,15 +378,15 @@ __global__ void __launch_bounds__(128, hier_min_ctas(DIM)) am_hier_kernel(phf_am
     if (active) {
         if (row_ok) {
             sp[gl] = th_j;
-            sp[DIM + 2 + gl] = mean_j;
+            sp[PHF_STATE_MEAN(DIM) + gl] = mean_j;
 #pragma unroll
             for (int k = 0; k < DIM; ++k)
-                if (k <= gl) sp[2 * DIM + 2 + gl * (gl + 1) / 2 + k] = crow[k];
+                if (k <= gl) sp[PHF_STATE_COV(DIM) + gl * (gl + 1) / 2 + k] = crow[k];
         }
         if (gl == 0) {
-            sp[DIM] = lt;
-            sp[2 * DIM + 2 + NT] = loga;
-            sp[2 * DIM + 2 + NT + 2] = n_acc;
+            sp[PHF_STATE_LOG_TARGET(DIM)] = lt;
+            sp[PHF_STATE_LOGA(DIM)] = loga;
+            sp[PHF_STATE_N_ACCEPTED(DIM)] = n_acc;
         }
     }
 }

@@ -108,20 +108,20 @@ __global__ void __launch_bounds__(32) hier_big_target_kernel(int64_t n, const do
         double *s = state + i * (size_t)PHF_STATE_SIZE(dim);
         for (int j = lane; j < dim; j += 32) {
             s[j] = th[j];
-            s[dim + 2 + j] = th[j];
+            s[PHF_STATE_MEAN(dim) + j] = th[j];
         }
-        for (int k = lane; k < nt; k += 32) s[2 * dim + 2 + k] = cov0[i * (size_t)nt + k];
+        for (int k = lane; k < nt; k += 32) s[PHF_STATE_COV(dim) + k] = cov0[i * (size_t)nt + k];
         __syncwarp();
         for (int j = lane; j < dim; j += 32) {  // non-positive diagonal of cov0 -> PHF_COV0_DIAG_FLOOR (see the header)
             const double v = cov0[i * (size_t)nt + rm(j, j)];
-            if (!(v > 0.0) && v == v) s[2 * dim + 2 + rm(j, j)] = PHF_COV0_DIAG_FLOOR;
+            if (!(v > 0.0) && v == v) s[PHF_STATE_COV(dim) + rm(j, j)] = PHF_COV0_DIAG_FLOOR;
         }
         if (lane == 0) {
-            s[dim] = lt;
-            s[dim + 1] = 0.0;
-            s[2 * dim + 2 + nt] = 0.0;
-            s[2 * dim + 2 + nt + 1] = 0.0;
-            s[2 * dim + 2 + nt + 2] = 0.0;
+            s[PHF_STATE_LOG_TARGET(dim)] = lt;
+            s[PHF_STATE_LOGLIK_T1(dim)] = 0.0;
+            s[PHF_STATE_LOGA(dim)] = 0.0;
+            s[PHF_STATE_LOGLIK_T1_SUM(dim)] = 0.0;
+            s[PHF_STATE_N_ACCEPTED(dim)] = 0.0;
         }
     }
 }
@@ -148,15 +148,17 @@ __global__ void __launch_bounds__(32) am_hier_big_kernel(phf_am_config cfg, int3
     const uint64_t chain_id = cfg.chain_id_base + (uint64_t)c;
 
     double *sp = state + c * (size_t)PHF_STATE_SIZE(dim);
-    double *cov = sp + 2 * dim + 2;              // row-major packed lower triangle, updated in place
+    // row-major packed lower triangle, updated in place, at PHF_STATE_COV(dim) = 2 dim + PHF_STATE_COV(0): the constant
+    // stays a separate pointer step, which ptxas folds into the load offsets of the loops below
+    double *cov = sp + 2 * dim + PHF_STATE_COV(0);
     double *L = scratch + c * (size_t)nt;        // column-major packed lower triangle
     for (int j = lane; j < dim; j += 32) {
         th[j] = sp[j];
-        mean[j] = sp[dim + 2 + j];
+        mean[j] = sp[PHF_STATE_MEAN(dim) + j];
     }
-    double lt = sp[dim];
-    double loga = sp[2 * dim + 2 + nt];
-    double n_acc = sp[2 * dim + 2 + nt + 2];
+    double lt = sp[PHF_STATE_LOG_TARGET(dim)];
+    double loga = sp[PHF_STATE_LOGA(dim)];
+    double n_acc = sp[PHF_STATE_N_ACCEPTED(dim)];
     __syncwarp();
 
     uint32_t t = cfg.t0;
@@ -254,12 +256,12 @@ __global__ void __launch_bounds__(32) am_hier_big_kernel(phf_am_config cfg, int3
 
     for (int j = lane; j < dim; j += 32) {
         sp[j] = th[j];
-        sp[dim + 2 + j] = mean[j];
+        sp[PHF_STATE_MEAN(dim) + j] = mean[j];
     }
     if (lane == 0) {
-        sp[dim] = lt;
-        sp[2 * dim + 2 + nt] = loga;
-        sp[2 * dim + 2 + nt + 2] = n_acc;
+        sp[PHF_STATE_LOG_TARGET(dim)] = lt;
+        sp[PHF_STATE_LOGA(dim)] = loga;
+        sp[PHF_STATE_N_ACCEPTED(dim)] = n_acc;
     }
 }
 

@@ -173,14 +173,14 @@ __global__ void __launch_bounds__(128, MINB)
         const int i = q + 4 * m;
         const bool ok = i < DIM;
         th_own[m] = ok ? sp[i] : 0.0;
-        mean_own[m] = ok ? sp[DIM + 2 + i] : 0.0;
+        mean_own[m] = ok ? sp[PHF_STATE_MEAN(DIM) + i] : 0.0;
 #pragma unroll
         for (int k = 0; k < DIM; ++k)
-            if (k < 4 * m + 4) covp[(Cfg::off(m) + k) * 32] = (ok && k <= i) ? sp[2 * DIM + 2 + i * (i + 1) / 2 + k] : 0.0;
+            if (k < 4 * m + 4) covp[(Cfg::off(m) + k) * 32] = (ok && k <= i) ? sp[PHF_STATE_COV(DIM) + i * (i + 1) / 2 + k] : 0.0;
     }
-    double lt = sp[DIM];
-    double loga = sp[2 * DIM + 2 + NT];
-    double n_acc = sp[2 * DIM + 2 + NT + 2];
+    double lt = sp[PHF_STATE_LOG_TARGET(DIM)];
+    double loga = sp[PHF_STATE_LOGA(DIM)];
+    double n_acc = sp[PHF_STATE_N_ACCEPTED(DIM)];
     double fr[NOWN];  // own rows: the covariance at the top of an iteration, the factor after the factorisation
 
     uint32_t t = cfg.t0;
@@ -371,16 +371,16 @@ __global__ void __launch_bounds__(128, MINB)
             const int i = q + 4 * m;
             if (i < DIM) {
                 sp[i] = th_own[m];
-                sp[DIM + 2 + i] = mean_own[m];
+                sp[PHF_STATE_MEAN(DIM) + i] = mean_own[m];
 #pragma unroll
                 for (int k = 0; k < DIM; ++k)
-                    if (k < 4 * m + 4 && k <= i) sp[2 * DIM + 2 + i * (i + 1) / 2 + k] = covp[(Cfg::off(m) + k) * 32];
+                    if (k < 4 * m + 4 && k <= i) sp[PHF_STATE_COV(DIM) + i * (i + 1) / 2 + k] = covp[(Cfg::off(m) + k) * 32];
             }
         }
         if (q == 0) {
-            sp[DIM] = lt;
-            sp[2 * DIM + 2 + NT] = loga;
-            sp[2 * DIM + 2 + NT + 2] = n_acc;
+            sp[PHF_STATE_LOG_TARGET(DIM)] = lt;
+            sp[PHF_STATE_LOGA(DIM)] = loga;
+            sp[PHF_STATE_N_ACCEPTED(DIM)] = n_acc;
         }
     }
 }

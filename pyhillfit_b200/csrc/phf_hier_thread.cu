@@ -121,12 +121,12 @@ __global__ void __launch_bounds__(32 * HierThreadCfg<NE>::kMaxWarps) __maxnreg__
 #pragma unroll
     for (int k = 0; k < DIM; ++k) {
         th[k] = sp[k];
-        mean[k * 32] = sp[DIM + 2 + k];
+        mean[k * 32] = sp[PHF_STATE_MEAN(DIM) + k];
     }
-    for (int k = 0; k < NT; ++k) cov[k * 32] = sp[2 * DIM + 2 + k];
-    double lt = sp[DIM];
-    double loga = sp[2 * DIM + 2 + NT];
-    double n_acc = sp[2 * DIM + 2 + NT + 2];
+    for (int k = 0; k < NT; ++k) cov[k * 32] = sp[PHF_STATE_COV(DIM) + k];
+    double lt = sp[PHF_STATE_LOG_TARGET(DIM)];
+    double loga = sp[PHF_STATE_LOGA(DIM)];
+    double n_acc = sp[PHF_STATE_N_ACCEPTED(DIM)];
 
     uint32_t t = cfg.t0;
     uint32_t until_save = cfg.thinning - (t % cfg.thinning);
@@ -249,12 +249,12 @@ __global__ void __launch_bounds__(32 * HierThreadCfg<NE>::kMaxWarps) __maxnreg__
 #pragma unroll
         for (int k = 0; k < DIM; ++k) {
             sp[k] = th[k];
-            sp[DIM + 2 + k] = mean[k * 32];
+            sp[PHF_STATE_MEAN(DIM) + k] = mean[k * 32];
         }
-        for (int k = 0; k < NT; ++k) sp[2 * DIM + 2 + k] = cov[k * 32];
-        sp[DIM] = lt;
-        sp[2 * DIM + 2 + NT] = loga;
-        sp[2 * DIM + 2 + NT + 2] = n_acc;
+        for (int k = 0; k < NT; ++k) sp[PHF_STATE_COV(DIM) + k] = cov[k * 32];
+        sp[PHF_STATE_LOG_TARGET(DIM)] = lt;
+        sp[PHF_STATE_LOGA(DIM)] = loga;
+        sp[PHF_STATE_N_ACCEPTED(DIM)] = n_acc;
     }
 }
 

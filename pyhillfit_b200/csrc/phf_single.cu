@@ -58,10 +58,10 @@ __global__ void __launch_bounds__(128) am_single_init_kernel(int64_t n, const do
 #pragma unroll
     for (int k = 0; k < D; ++k) {
         s[k] = th[k];
-        s[D + 2 + k] = th[k];
+        s[PHF_STATE_MEAN(D) + k] = th[k];
     }
-    s[D] = lt;
-    s[D + 1] = l1;
+    s[PHF_STATE_LOG_TARGET(D)] = lt;
+    s[PHF_STATE_LOGLIK_T1(D)] = l1;
     {   // a non-positive diagonal entry of cov0 becomes PHF_COV0_DIAG_FLOOR (include/pyhillfit_b200.h)
         int q = 0;
 #pragma unroll
@@ -69,12 +69,12 @@ __global__ void __launch_bounds__(128) am_single_init_kernel(int64_t n, const do
 #pragma unroll
             for (int c2 = 0; c2 <= r; ++c2, ++q) {
                 const double v = cov0[i * NT + q];
-                s[2 * D + 2 + q] = (r == c2 && !(v > 0.0) && v == v) ? PHF_COV0_DIAG_FLOOR : v;
+                s[PHF_STATE_COV(D) + q] = (r == c2 && !(v > 0.0) && v == v) ? PHF_COV0_DIAG_FLOOR : v;
             }
     }
-    s[2 * D + 2 + NT] = 0.0;      // loga
-    s[2 * D + 2 + NT + 1] = 0.0;  // loglik_t1_sum
-    s[2 * D + 2 + NT + 2] = 0.0;  // n_accepted
+    s[PHF_STATE_LOGA(D)] = 0.0;
+    s[PHF_STATE_LOGLIK_T1_SUM(D)] = 0.0;
+    s[PHF_STATE_N_ACCEPTED(D)] = 0.0;
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -135,20 +135,7 @@ PHF_DI void am_step(const double *T, const ChainConst &cc, ChainRegs<MODEL> &s, 
 #pragma unroll
         for (int k = 0; k < D; ++k) s.mean[k] = s.th[k];
     }
-    {
-        const double omg = 1.0 - gam;
-        double dv[D];
-#pragma unroll
-        for (int k = 0; k < D; ++k) dv[k] = s.th[k] - s.mean[k];
-        int q = 0;
-#pragma unroll
-        for (int i = 0; i < D; ++i)
-#pragma unroll
-            for (int j = 0; j <= i; ++j, ++q) s.cov[q] = fma(gam, dv[i] * dv[j], omg * s.cov[q]);
-#pragma unroll
-        for (int k = 0; k < D; ++k) s.mean[k] = fma(gam, s.th[k], omg * s.mean[k]);
-        s.loga = fma(gam, (accepted ? 1.0 : 0.0) - 0.25, s.loga);
-    }
+    adapt_update<D>(s.mean, s.cov, s.loga, s.th, gam, (accepted ? 1.0 : 0.0) - 0.25);
 
     // ---- thinned write-out (PyHillFit.py:847-848) + Sum loglik_t1 for thermodynamic integration ----
     if (--until_save == 0u) {
@@ -233,7 +220,7 @@ __global__ void __launch_bounds__(128, MINB)
                      const double *__restrict__ temperature, const phf_dataset *__restrict__ datasets,
                      const phf_dose_group *__restrict__ groups, double *__restrict__ samples, int ordered)
 {
-    constexpr int D = SingleDims<MODEL>::D, NT = SingleDims<MODEL>::NT, NF = SingleDims<MODEL>::NF;
+    constexpr int D = SingleDims<MODEL>::D, NF = SingleDims<MODEL>::NF;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     phf_dose_group *sgroups = reinterpret_cast<phf_dose_group *>(smem_raw);
     PHF_STAGE_FASTMATH_TABLE(T);
@@ -288,18 +275,7 @@ __global__ void __launch_bounds__(128, MINB)
     // ---- load chain state into registers ----
     double *sp = state + c * NF;
     ChainRegs<MODEL> s;
-#pragma unroll
-    for (int k = 0; k < D; ++k) {
-        s.th[k] = sp[k];
-        s.mean[k] = sp[D + 2 + k];
-    }
-    s.lt = sp[D];
-    s.l1 = sp[D + 1];
-#pragma unroll
-    for (int k = 0; k < NT; ++k) s.cov[k] = sp[2 * D + 2 + k];
-    s.loga = sp[2 * D + 2 + NT];
-    s.l1_sum = sp[2 * D + 2 + NT + 1];
-    s.n_acc = sp[2 * D + 2 + NT + 2];
+    s.load(sp);
 
     uint32_t t = cfg.t0;
     uint32_t until_save = cfg.thinning - (t % cfg.thinning);
@@ -366,32 +342,22 @@ __global__ void __launch_bounds__(128, MINB)
         am_step<MODEL, G>(T, cc, s, dr, gam, t, gl, mask, until_save, row);
     }
 
-    if (active && gl == 0) {
-#pragma unroll
-        for (int k = 0; k < D; ++k) {
-            sp[k] = s.th[k];
-            sp[D + 2 + k] = s.mean[k];
-        }
-        sp[D] = s.lt;
-        sp[D + 1] = s.l1;
-#pragma unroll
-        for (int k = 0; k < NT; ++k) sp[2 * D + 2 + k] = s.cov[k];
-        sp[2 * D + 2 + NT] = s.loga;
-        sp[2 * D + 2 + NT + 1] = s.l1_sum;
-        sp[2 * D + 2 + NT + 2] = s.n_acc;
-    }
+    if (active && gl == 0) s.store(sp);
 }
 
 template <int MODEL, int G, int MINB>
-static int launch_am_single(const phf_am_config &cfg, int64_t n, int block, size_t smem, double *state,
-                            const int32_t *dataset_id, const double *temperature, const phf_dataset *datasets,
-                            const phf_dose_group *groups, double *samples, cudaStream_t s)
+static int launch_am_single(const phf_am_config &cfg, int64_t n, int block, double *state, const int32_t *dataset_id,
+                            const double *temperature, const phf_dataset *datasets, const phf_dose_group *groups,
+                            double *samples, cudaStream_t s)
 {
+    constexpr int D = SingleDims<MODEL>::D;
     auto kern = am_single_kernel<MODEL, G, MINB>;
-    cudaError_t e;
-    if (smem > 40 * 1024 &&  // (the 48 KB default limit counts the kernel's static shared memory too)
-        (e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)))
-        return set_cuda_error(e, "cudaFuncSetAttribute");
+    // staged dose groups + (G > 1) one draw slot of D+1 doubles per thread + 32 gamma_s per warp + 4 / G prepared
+    // dose-group records of 64 bytes per thread
+    const size_t smem = (size_t)cfg.stage_groups * sizeof(phf_dose_group) +
+                        (G > 1 ? (size_t)block * (D + 1) * sizeof(double) : 0) + (size_t)block * sizeof(double) +
+                        (size_t)block * (4 / G) * 64;
+    if (int rc = allow_dynamic_smem(kern, smem)) return rc;
     const int cta_chains = block / G;
     const unsigned grid = (unsigned)((n + cta_chains - 1) / cta_chains);
     // expensive chain blocks first (ordered_block_index) when there is more than one CTA per SM and one wave or so
@@ -539,18 +505,12 @@ extern "C" int phf_am_single_run(const phf_am_config *cfg, int64_t n_chains, dou
     if (depth > 1)
         return am_single_spec_launch(*cfg, lanes, depth, n_chains, block, state, dataset_id, temperature, datasets, groups,
                                      samples, (cudaStream_t)stream);
-    // staged dose groups + (lanes > 1) one draw slot of d+1 doubles per thread + 32 gamma_s per warp + 4 / lanes
-    // prepared dose-group records of 64 bytes per thread
-    const size_t smem = (size_t)cfg->stage_groups * sizeof(phf_dose_group) +
-                        (lanes > 1 ? (size_t)block * ((cfg->model == 1 ? 2 : 3) + 1) * sizeof(double) : 0) +
-                        (size_t)block * sizeof(double) + (size_t)block * (4 / lanes) * 64;
-    if (smem > 200 * 1024) return set_error(PHF_EINVAL, "cfg.stage_groups needs more than 200 KB of shared memory");
     cudaStream_t s = (cudaStream_t)stream;
     const int minb = cfg->min_ctas_hint > 0 ? cfg->min_ctas_hint : 3;  // 168 registers: no spills; measured best at every size
 #define PHF_AM_CASE(M, G, MINB)                                                                                  \
     if (cfg->model == M && lanes == G && minb == MINB)                                                                       \
-        return launch_am_single<M, G, MINB>(*cfg, n_chains, block, smem, state, dataset_id, temperature, datasets, \
-                                            groups, samples, s)
+        return launch_am_single<M, G, MINB>(*cfg, n_chains, block, state, dataset_id, temperature, datasets, groups, \
+                                            samples, s)
     PHF_AM_CASE(1, 1, 3);
     PHF_AM_CASE(1, 2, 3);
     PHF_AM_CASE(1, 4, 3);

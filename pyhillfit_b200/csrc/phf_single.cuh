@@ -2,6 +2,7 @@
 // sufficient-statistic form described in include/pyhillfit_b200.h.
 #pragma once
 #include "../../include/pyhillfit_b200.h"
+#include "phf_common.cuh"
 #include "phf_math.cuh"
 
 namespace phf {
@@ -264,13 +265,75 @@ PHF_DI Draws<D> make_draws(const double *T, uint64_t seed, uint64_t chain_id, ui
     return dr;
 }
 
-// Registers of one chain (identical on the G lanes that own it).
+// Registers of one chain (identical on the G lanes that own it), loaded from and stored to its state row.
 template <int MODEL>
 struct ChainRegs {
     static constexpr int D = SingleDims<MODEL>::D, NT = SingleDims<MODEL>::NT;
     double th[D], mean[D], cov[NT];
     double lt, l1, loga, l1_sum, n_acc;
+
+    PHF_DI void load(const double *sp)
+    {
+#pragma unroll
+        for (int k = 0; k < D; ++k) {
+            th[k] = sp[k];
+            mean[k] = sp[PHF_STATE_MEAN(D) + k];
+        }
+        lt = sp[PHF_STATE_LOG_TARGET(D)];
+        l1 = sp[PHF_STATE_LOGLIK_T1(D)];
+#pragma unroll
+        for (int k = 0; k < NT; ++k) cov[k] = sp[PHF_STATE_COV(D) + k];
+        loga = sp[PHF_STATE_LOGA(D)];
+        l1_sum = sp[PHF_STATE_LOGLIK_T1_SUM(D)];
+        n_acc = sp[PHF_STATE_N_ACCEPTED(D)];
+    }
+    PHF_DI void store(double *sp) const
+    {
+#pragma unroll
+        for (int k = 0; k < D; ++k) {
+            sp[k] = th[k];
+            sp[PHF_STATE_MEAN(D) + k] = mean[k];
+        }
+        sp[PHF_STATE_LOG_TARGET(D)] = lt;
+        sp[PHF_STATE_LOGLIK_T1(D)] = l1;
+#pragma unroll
+        for (int k = 0; k < NT; ++k) sp[PHF_STATE_COV(D) + k] = cov[k];
+        sp[PHF_STATE_LOGA(D)] = loga;
+        sp[PHF_STATE_LOGLIK_T1_SUM(D)] = l1_sum;
+        sp[PHF_STATE_N_ACCEPTED(D)] = n_acc;
+    }
 };
+
+// Adaptation after an iteration whose outcome is `acc_minus_quarter` + 0.25 (th is already the post-accept theta):
+// PyHillFit.py:840-846, PyHillTemp.py:114-122.  With gam == 0 the update is the identity bit for bit.
+template <int D>
+PHF_DI void adapt_update(double *mean, double *cov, double &loga, const double *th, double gam, double acc_minus_quarter)
+{
+    const double omg = 1.0 - gam;
+    double dv[D];
+#pragma unroll
+    for (int k = 0; k < D; ++k) dv[k] = th[k] - mean[k];
+    int q = 0;
+#pragma unroll
+    for (int i = 0; i < D; ++i)
+#pragma unroll
+        for (int j = 0; j <= i; ++j, ++q) cov[q] = fma(gam, dv[i] * dv[j], omg * cov[q]);
+#pragma unroll
+    for (int k = 0; k < D; ++k) mean[k] = fma(gam, th[k], omg * mean[k]);
+    loga = fma(gam, acc_minus_quarter, loga);
+}
+
+// Host side of a sampler launch with `smem` bytes of dynamic shared memory: at most 200 KB, and above 40 KB the kernel's
+// limit is raised (the 48 KB default counts the kernel's static shared memory too).
+template <typename Kernel>
+static int allow_dynamic_smem(Kernel kern, size_t smem)
+{
+    if (smem > 200 * 1024) return set_error(PHF_EINVAL, "cfg.stage_groups needs more than 200 KB of shared memory");
+    cudaError_t e;
+    if (smem > 40 * 1024 && (e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)))
+        return set_cuda_error(e, "cudaFuncSetAttribute");
+    return PHF_OK;
+}
 
 // proposal theta* = theta + e^{loga/2} chol(cov) z  (N(theta, e^loga cov): PyHillFit.py:831, PyHillTemp.py:88), guarded
 // pivots (phf_math.cuh); cov = lower triangle, row-major

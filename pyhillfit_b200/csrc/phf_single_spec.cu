@@ -32,25 +32,6 @@
 
 namespace phf {
 
-// adaptation after iteration `ti` whose outcome is `accepted` (th is already the post-accept theta):
-// PyHillFit.py:840-846, PyHillTemp.py:114-122 -- the same expressions as am_step (phf_single.cu)
-template <int D>
-PHF_DI void adapt_update(double *mean, double *cov, double &loga, const double *th, double gam, double acc_minus_quarter)
-{
-    const double omg = 1.0 - gam;
-    double dv[D];
-#pragma unroll
-    for (int k = 0; k < D; ++k) dv[k] = th[k] - mean[k];
-    int q = 0;
-#pragma unroll
-    for (int i = 0; i < D; ++i)
-#pragma unroll
-        for (int j = 0; j <= i; ++j, ++q) cov[q] = fma(gam, dv[i] * dv[j], omg * cov[q]);
-#pragma unroll
-    for (int k = 0; k < D; ++k) mean[k] = fma(gam, th[k], omg * mean[k]);
-    loga = fma(gam, acc_minus_quarter, loga);
-}
-
 template <int MODEL, int E, int S>
 __global__ void __launch_bounds__(128, 3)
     am_single_spec_kernel(phf_am_config cfg, int64_t n, double *__restrict__ state,
@@ -79,7 +60,8 @@ __global__ void __launch_bounds__(128, 3)
     const unsigned cbase = lane & ~(unsigned)(G - 1);  // first lane of this chain in the warp
     constexpr unsigned full = 0xffffffffu;             // every lane reaches every shuffle / vote (see phf_single.cu)
 
-    // ---- stage this CTA's dose groups (chains are sorted by dataset, so the range is contiguous) ----
+    // ---- stage this CTA's dose groups (chains are sorted by dataset, so the range is contiguous).  The same code as
+    //      am_single_kernel's, kept in step by hand: as a shared function it changes this kernel's SASS ----
     const phf_dataset ds = datasets[dataset_id[c]];
     const phf_dose_group *grp = ds.n_groups > 0 ? groups + ds.group_begin : groups;
     if (cfg.stage_groups > 0) {
@@ -106,18 +88,7 @@ __global__ void __launch_bounds__(128, 3)
     // ---- base state (identical on the G lanes of the chain) ----
     double *sp = state + c * NF;
     ChainRegs<MODEL> s;
-#pragma unroll
-    for (int k = 0; k < D; ++k) {
-        s.th[k] = sp[k];
-        s.mean[k] = sp[D + 2 + k];
-    }
-    s.lt = sp[D];
-    s.l1 = sp[D + 1];
-#pragma unroll
-    for (int k = 0; k < NT; ++k) s.cov[k] = sp[2 * D + 2 + k];
-    s.loga = sp[2 * D + 2 + NT];
-    s.l1_sum = sp[2 * D + 2 + NT + 1];
-    s.n_acc = sp[2 * D + 2 + NT + 2];
+    s.load(sp);
 
     uint32_t t = cfg.t0;  // iterations this chain has completed
     const uint32_t t_end = cfg.t0 + cfg.n_iters;
@@ -264,20 +235,7 @@ __global__ void __launch_bounds__(128, 3)
         t += (uint32_t)k_adv;
     }
 
-    if (active && gl == 0) {
-#pragma unroll
-        for (int k = 0; k < D; ++k) {
-            sp[k] = s.th[k];
-            sp[D + 2 + k] = s.mean[k];
-        }
-        sp[D] = s.lt;
-        sp[D + 1] = s.l1;
-#pragma unroll
-        for (int k = 0; k < NT; ++k) sp[2 * D + 2 + k] = s.cov[k];
-        sp[2 * D + 2 + NT] = s.loga;
-        sp[2 * D + 2 + NT + 1] = s.l1_sum;
-        sp[2 * D + 2 + NT + 2] = s.n_acc;
-    }
+    if (active && gl == 0) s.store(sp);
 }
 
 template <int MODEL, int E, int S>
@@ -290,10 +248,7 @@ static int launch_spec(const phf_am_config &cfg, int64_t n, int block, double *s
     const int cta_chains = block / G;
     const size_t smem = (size_t)cfg.stage_groups * sizeof(phf_dose_group) +
                         (size_t)cta_chains * (2 * G) * (D + 2) * sizeof(double) + (size_t)block * (4 / E) * 64;
-    cudaError_t e;
-    if (smem > 200 * 1024) return set_error(PHF_EINVAL, "cfg.stage_groups needs more than 200 KB of shared memory");
-    if (smem > 40 * 1024 && (e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)))
-        return set_cuda_error(e, "cudaFuncSetAttribute");
+    if (int rc = allow_dynamic_smem(kern, smem)) return rc;
     const unsigned grid = (unsigned)((n + cta_chains - 1) / cta_chains);
     kern<<<grid, block, smem, s>>>(cfg, n, state, dataset_id, temperature, datasets, groups, samples);
     count_launch();

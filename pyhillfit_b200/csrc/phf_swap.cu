@@ -28,7 +28,7 @@ __global__ void __launch_bounds__(128) am_single_swap_kernel(int64_t n_pairs, in
     if (ca < 0 || ca >= n_chains || cb < 0 || cb >= n_chains) return;  // (the host validates the map; never read past it)
     double *sa = state + ca * NF, *sb = state + cb * NF;
     const double ta = temperature[ca], tb = temperature[cb];
-    const double l1a = sa[D + 1], l1b = sb[D + 1];
+    const double l1a = sa[PHF_STATE_LOGLIK_T1(D)], l1b = sb[PHF_STATE_LOGLIK_T1(D)];
     const Philox4 r = philox_call(seed, ladder_id_base + (uint64_t)ladder, t, PHF_SWAP_CALL0 + (uint32_t)k);
     const double log_u = fm::log_pos(T, uniform53(r.w[0], r.w[1]));
     // the prior cancels: ln u < (t_k - t_k+1) (l1(x_k+1) - l1(x_k)); a non-finite l1 on either side rejects
@@ -56,10 +56,10 @@ __global__ void __launch_bounds__(128) am_single_swap_kernel(int64_t n_pairs, in
         sa[q] = tha[q];
         sb[q] = thb[q];
     }
-    sa[D] = lta;
-    sa[D + 1] = l1na;
-    sb[D] = ltb;
-    sb[D + 1] = l1nb;
+    sa[PHF_STATE_LOG_TARGET(D)] = lta;
+    sa[PHF_STATE_LOGLIK_T1(D)] = l1na;
+    sb[PHF_STATE_LOG_TARGET(D)] = ltb;
+    sb[PHF_STATE_LOGLIK_T1(D)] = l1nb;
 }
 
 }  // namespace phf

@@ -90,10 +90,9 @@ class _Base:
     # ---- state accessors (copies to host) ----
     def state_fields(self):
         s = self.state.cpu().numpy()
-        d, nt = self.d, self.d * (self.d + 1) // 2
-        return dict(theta=s[:, :d], log_target=s[:, d], loglik_t1=s[:, d + 1], mean=s[:, d + 2:2 * d + 2],
-                    cov=tri_unpack(s[:, 2 * d + 2:2 * d + 2 + nt], d), loga=s[:, 2 * d + 2 + nt],
-                    loglik_t1_sum=s[:, 2 * d + 3 + nt], n_accepted=s[:, 2 * d + 4 + nt])
+        fields = {name: s[:, at] for name, at in _lib.state_offsets(self.d).items()}
+        fields["cov"] = tri_unpack(fields["cov"], self.d)
+        return fields
 
     def acceptance(self):
         return self.state_fields()["n_accepted"] / max(self.t, 1)
@@ -104,6 +103,16 @@ class _Base:
         if discard_burn and self.burn_rows != NO_BURN:
             first = max(first, int(self.burn_rows))
         return max(last - first + 1, 0)
+
+    def _samples_buffer(self, samples, rows, row_major):
+        """(buffer, its capacity in rows) for a run that saves `rows` rows: `samples`, checked against n chains of d+1
+        columns, or a new [n, max(rows, 1), d+1] buffer ([max(rows, 1), n, d+1] with row_major)."""
+        ax_n, ax_r = (1, 0) if row_major else (0, 1)
+        if samples is None:
+            shape = (max(rows, 1), self.n, self.d + 1) if row_major else (self.n, max(rows, 1), self.d + 1)
+            samples = self.torch.empty(shape, dtype=self.torch.float64, device=self.device)
+        assert samples.shape[ax_n] == self.n and samples.shape[2] == self.d + 1
+        return samples, samples.shape[ax_r]
 
     def _config(self, n_iters, rows_capacity, row_major=False, discard_burn=False):
         return _lib.AmConfig(discard_burn_rows=int(bool(discard_burn)), sample_layout=_lib.SAMPLES_ROW_MAJOR if row_major else _lib.SAMPLES_CHAIN_MAJOR,
@@ -184,8 +193,8 @@ class SingleLevelSampler(_Base):
                                             self.ds_dev.data_ptr(), self.groups_dev.data_ptr(),
                                             self.state.data_ptr(), _lib.current_stream_ptr()), "phf_am_single_init")
             if burn_rows == 0:  # row 0 (the start state) is a counted row
-                nt = self.d * (self.d + 1) // 2
-                self.state[:, 2 * self.d + 3 + nt] = self.state[:, self.d + 1]
+                off = _lib.state_offsets(self.d)
+                self.state[:, off["loglik_t1_sum"]] = self.state[:, off["loglik_t1"]]
 
     def _default_block(self, n_threads):
         """mirror of default_block_threads (csrc/phf_common.cuh): needed here to size the shared-memory staging"""
@@ -206,23 +215,14 @@ class SingleLevelSampler(_Base):
         contiguous: coalesced write-out, contiguous transfers); None when keep=False (thermodynamic-integration-only
         runs).  discard_burn=True: rows with index < burn_rows are not written at all (what PyHillFit.py:861-864 and
         PyHillTemp.py:125 drop before saving); the returned rows start at max(burn_rows, first row of this call)."""
-        torch = self.torch
         rows = self.rows_for(n_iters, discard_burn)
         cap = rows
-        ax_n, ax_r = (1, 0) if row_major else (0, 1)
         if keep:
-            if samples is None:
-                shape = (max(rows, 1), self.n, self.d + 1) if row_major else (self.n, max(rows, 1), self.d + 1)
-                samples = torch.empty(shape, dtype=torch.float64, device=self.device)
-            cap = samples.shape[ax_r]
-            assert samples.shape[ax_n] == self.n and samples.shape[2] == self.d + 1 and samples.is_contiguous()
+            samples, cap = self._samples_buffer(samples, rows, row_major)
+            assert samples.is_contiguous()
         cfg = self._config(n_iters, cap, row_major, discard_burn)
-        with torch.cuda.device(self.device):
-            _lib.check(_lib.load().phf_am_single_run(C.byref(cfg), self.n, self.state.data_ptr(),
-                                                     self.dataset_id.data_ptr(), self.temperature.data_ptr(),
-                                                     self.ds_dev.data_ptr(), self.groups_dev.data_ptr(),
-                                                     samples.data_ptr() if keep else None,
-                                                     _lib.current_stream_ptr()), "phf_am_single_run")
+        with self.torch.cuda.device(self.device):
+            self._launch(cfg, samples.data_ptr() if keep else None, _lib.current_stream_ptr())
         self.t += int(n_iters)
         if not keep:
             return None
@@ -249,12 +249,9 @@ class SingleLevelSampler(_Base):
             self.swap_counts = torch.zeros((lad.shape[0], lad.shape[1] - 1, 2), dtype=torch.int64, device=self.device)
             self._ladder_key = key
         rows = self.rows_for(n_iters, discard_burn)
-        ax_n, ax_r = (1, 0) if row_major else (0, 1)
         if keep:
-            if samples is None:
-                shape = (max(rows, 1), self.n, self.d + 1) if row_major else (self.n, max(rows, 1), self.d + 1)
-                samples = torch.empty(shape, dtype=torch.float64, device=self.device)
-            assert samples.shape[ax_n] == self.n and samples.shape[2] == self.d + 1 and samples.shape[ax_r] >= rows
+            samples, cap = self._samples_buffer(samples, rows, row_major)
+            assert cap >= rows
         L = _lib.load()
         end, at = self.t + int(n_iters), 0
         lad = self._ladders
@@ -275,9 +272,7 @@ class SingleLevelSampler(_Base):
                     at += r
                 else:
                     cfg.t0, cfg.n_iters = self.t, k
-                    _lib.check(L.phf_am_single_run(C.byref(cfg), self.n, self.state.data_ptr(), self.dataset_id.data_ptr(),
-                                                   self.temperature.data_ptr(), self.ds_dev.data_ptr(),
-                                                   self.groups_dev.data_ptr(), None, stream), "phf_am_single_run")
+                    self._launch(cfg, None, stream)
                     self.t += k
                 if self.t % K == 0:
                     _lib.check(L.phf_am_single_swap(self.model, self.n, self.state.data_ptr(), self.dataset_id.data_ptr(),
@@ -289,6 +284,12 @@ class SingleLevelSampler(_Base):
         if not keep:
             return None
         return samples[:rows] if row_major else samples[:, :rows]
+
+    def _launch(self, cfg, samples_ptr, stream):
+        """phf_am_single_run of every chain with `cfg`, writing rows to `samples_ptr` (None: no rows)"""
+        _lib.check(_lib.load().phf_am_single_run(C.byref(cfg), self.n, self.state.data_ptr(), self.dataset_id.data_ptr(),
+                                                 self.temperature.data_ptr(), self.ds_dev.data_ptr(),
+                                                 self.groups_dev.data_ptr(), samples_ptr, stream), "phf_am_single_run")
 
     def swap_acceptance(self):
         """[n_ladders, T-1] accepted / attempted swaps of each adjacent pair so far (nan where none was attempted)."""
@@ -360,12 +361,9 @@ class HierarchicalSampler(_Base):
         with row_major=True (one saved iteration of all chains contiguous, as in SingleLevelSampler.run)."""
         torch = self.torch
         rows = self.rows_for(n_iters)
-        ax_n, ax_r = (1, 0) if row_major else (0, 1)
-        if samples is None:
-            shape = (max(rows, 1), self.n, self.d + 1) if row_major else (self.n, max(rows, 1), self.d + 1)
-            samples = torch.empty(shape, dtype=torch.float64, device=self.device)
-        assert samples.shape[ax_n] == self.n and samples.shape[2] == self.d + 1 and samples.is_contiguous()
-        cfg = self._config(n_iters, samples.shape[ax_r], row_major)
+        samples, cap = self._samples_buffer(samples, rows, row_major)
+        assert samples.is_contiguous()
+        cfg = self._config(n_iters, cap, row_major)
         with torch.cuda.device(self.device):
             _lib.check(_lib.load().phf_am_hier_run(C.byref(cfg), self.n_expts, self.n, self.state.data_ptr(),
                                                    self.dataset_id.data_ptr(), self.ds_dev.data_ptr(),

@@ -9,6 +9,7 @@ import time
 
 import numpy as np
 
+from . import _lib as phf_lib
 from . import dist as phf_dist
 from . import doseresponse as dr
 from .packing import SinglePack
@@ -125,12 +126,11 @@ def run_ti(datasets, models=(1, 2), temps=None, replicates=1, iterations=500000,
     out["speculation"] = {m: samplers[m].speculation for m in samplers}
     t_gather = time.perf_counter()
     for model in models:
-        d = 2 if model == 1 else 3
-        nt = d * (d + 1) // 2
+        off = phf_lib.state_offsets(2 if model == 1 else 3)
         if hi > lo:
             st = samplers[model].state
-            local_means = st[:, 2 * d + 3 + nt] / (num_saved - burn)
-            local_acc = st[:, 2 * d + 4 + nt] / iterations
+            local_means = st[:, off["loglik_t1_sum"]] / (num_saved - burn)
+            local_acc = st[:, off["n_accepted"]] / iterations
         else:
             local_means = torch.zeros(0, dtype=torch.float64, device=dev)
             local_acc = torch.zeros(0, dtype=torch.float64, device=dev)

@@ -102,7 +102,12 @@ int main(void) {
     printf("%zu %zu %zu %zu %zu %zu\n", offsetof(phf_am_config, seed), offsetof(phf_am_config, chain_id_base),
            offsetof(phf_am_config, stage_groups), offsetof(phf_am_config, lanes_per_chain),
            offsetof(phf_dataset, pi_bit), offsetof(phf_am_config, sample_layout));
-    printf("%d %d %d\n", PHF_STATE_SIZE(2), PHF_STATE_SIZE(3), PHF_STATE_SIZE(11));
+    const int ds[3] = {2, 3, 11};
+    for (int i = 0; i < 3; ++i)
+        printf("%d %d %d %d %d %d %d %d ", PHF_STATE_LOG_TARGET(ds[i]), PHF_STATE_LOGLIK_T1(ds[i]), PHF_STATE_MEAN(ds[i]),
+               PHF_STATE_COV(ds[i]), PHF_STATE_LOGA(ds[i]), PHF_STATE_LOGLIK_T1_SUM(ds[i]), PHF_STATE_N_ACCEPTED(ds[i]),
+               PHF_STATE_SIZE(ds[i]));
+    printf("\n");
     return 0;
 }
 ''')
@@ -116,7 +121,14 @@ int main(void) {
     assert offs == [_lib.AmConfig.seed.offset, _lib.AmConfig.chain_id_base.offset, _lib.AmConfig.stage_groups.offset,
                     _lib.AmConfig.lanes_per_chain.offset, _lib.DATASET_DTYPE.fields["pi_bit"][1],
                     _lib.AmConfig.sample_layout.offset]
-    assert [int(x) for x in out[2].split()] == [_lib.state_size(2), _lib.state_size(3), _lib.state_size(11)]
+    want = []
+    for d in (2, 3, 11):
+        f = _lib.state_offsets(d)
+        # the fields tile the row in the header's order: theta, log_target, loglik_t1, mean, cov, loga, sum, n_acc
+        assert (f["theta"].start, f["theta"].stop, f["mean"].stop, f["cov"].stop) == (0, d, f["cov"].start, f["loga"])
+        want += [f["log_target"], f["loglik_t1"], f["mean"].start, f["cov"].start, f["loga"], f["loglik_t1_sum"],
+                 f["n_accepted"], _lib.state_size(d)]
+    assert [int(x) for x in out[2].split()] == want
 
 
 def test_missing_library_fails_loudly(monkeypatch):
