@@ -51,19 +51,13 @@ def select_pairs(dr, args):
     return list(it.product(drugs, channels))
 
 
-def concat(experiments, num_expts):
-    concs = np.concatenate([experiments[i][:, 0] for i in range(num_expts)])     # PyHillFit.py:661-665
-    responses = np.concatenate([experiments[i][:, 1] for i in range(num_expts)])
-    return concs, responses
-
-
 def run_single_level(dr, args, pairs):
     """python/PyHillFit.py:645-867 for all pairs at once."""
     import torch
-    from . import chainio
+    from . import chainio, ess
     from .initial_fit import best_fit_batch_gpu as best_fit_batch   # phf_best_fit_batch, one thread per dataset
     from .packing import SinglePack
-    from .sampler import SingleLevelSampler
+    from .sampler import SingleLevelSampler, model_chain_id_base
     temperature = 1
     assert args.iterations % args.thinning == 0            # PyHillFit.py:805
     jobs, data = [], []
@@ -75,7 +69,7 @@ def run_single_level(dr, args, pairs):
             print("Problem loading data, guessing there are no entries for {} + {} --- skipping".format(drug, channel))
             continue
         cdrug, cchannel, chain_file, images_dir = dr.nonhierarchical_chain_file_and_figs_dir(args.model, drug, channel, temperature)
-        concs, responses = concat(experiments, num_expts)
+        concs, responses = dr.concat_experiments(experiments, num_expts)
         if np.any(np.isnan(responses)):
             print("Skipping {} because of empty responses / missing data".format((drug, channel)))
             continue
@@ -100,61 +94,27 @@ def run_single_level(dr, args, pairs):
         theta0 = theta0 * jit
     saved_iterations = args.iterations // args.thinning + 1
     burn = saved_iterations // args.burn_in_fraction
-    # (-m 1 and -m 2 are separate invocations with the same --seed: the model goes into the Philox chain id, as in
-    # pyhillfit_b200/ti.py, so that the two models' chains do not share their draws)
     s = SingleLevelSampler(args.model, pack, ids, 1.0, theta0, variant="fit", seed=args.seed,
-                           chain_id_base=(args.model - 1) * (1 << 40), thinning=args.thinning, burn_rows=burn)
-    d = s.d
-    # only the rows the reference saves (chain[burn:], PyHillFit.py:861-864) are written by the kernel and copied back
-    kept = saved_iterations - burn
-    chain = torch.empty((s.n, kept, d + 1), dtype=torch.float64, device=s.device)
-    at = 0
-    if burn == 0:
-        chain[:, 0, :] = s.initial_row()
-        at = 1
+                           chain_id_base=model_chain_id_base(args.model), thinning=args.thinning, burn_rows=burn)
     torch.cuda.synchronize()
     print("packing, CUDA start-up, sampler state: {:.2f} s".format(time.time() - t_phase))
     start = time.time()
-    done = 0
-    while done < args.iterations:
-        k = min(args.segment - args.segment % args.thinning or args.thinning, args.iterations - done)
-        seg = s.run(k, discard_burn=True)
-        chain[:, at:at + seg.shape[1], :] = seg
-        at += seg.shape[1]
-        done += k
+    # only the rows the reference saves (chain[burn:], PyHillFit.py:861-864) are written by the kernel and copied back
+    chain = s.collect(args.iterations, args.segment, discard_burn=True)
     torch.cuda.synchronize()
-    assert at == kept
     print("\n{} chains x {} iterations in {:.2f} s on the GPU\n".format(s.n, args.iterations, time.time() - start))
-    diag = run_diagnostics(args, chain, len(jobs), R, 0)
+    diag = ess.targets_diagnostics(chain, len(jobs), R, 0) if args.diagnostics else None
     t_phase = time.time()
-    host = chain.cpu().numpy()                              # burn-in already removed (PyHillFit.py:861-864)
+    host = chain.cpu().numpy().reshape(len(jobs), R, chain.shape[1], s.d + 1)
     print("chains to the host: {:.2f} s".format(time.time() - t_phase))
     t_phase = time.time()
     for j, job in enumerate(jobs):
-        for r in range(R):
-            f = job["chain_file"] if r == 0 else chainio.extra_chain_name(job["chain_file"], r)
-            chainio.save_single_level_chain(f, host[j * R + r], job["drug"], job["channel"])
-        if diag is not None:
-            names = ["pIC50", "sigma"] if args.model == 1 else ["pIC50", "Hill", "sigma"]
-            chainio.save_diagnostics(job["chain_file"], diag[j], names + ["log-target"], R, 0, kept)
+        chainio.save_target_chains(job["chain_file"], host[j],
+                                   lambda f, c: chainio.save_single_level_chain(f, c, job["drug"], job["channel"]),
+                                   None if diag is None else diag[j], chainio.single_level_columns(args.model))
         print("\n\n{} + {} complete!\n\n".format(job["drug"], job["channel"]))
     print("chain files: {:.2f} s".format(time.time() - t_phase))
     return jobs
-
-
-def run_diagnostics(args, chain, n_targets, R, row_begin):
-    """--diagnostics: split R-hat / multi-chain ESS of each target's R chains from rows [row_begin, ...) of the device
-    tensor `chain` [n_targets * R, rows, d+1] (before it is copied to the host); None without the flag."""
-    if not args.diagnostics:
-        return None
-    from . import ess
-    if chain.shape[1] - row_begin < 8:
-        print("--diagnostics: fewer than 8 rows per chain, no diagnostics written")
-        return None
-    t_phase = time.time()
-    diag = ess.chain_diagnostics_gpu(chain, np.arange(n_targets + 1) * R, row_begin=row_begin)
-    print("{} ({:.2f} s)".format(ess.diagnostics_summary(diag), time.time() - t_phase))
-    return diag
 
 
 def hierarchical_start(experiments, locs, best_fits=None):
@@ -197,7 +157,7 @@ def hierarchical_start(experiments, locs, best_fits=None):
 def run_hierarchical(dr, args, pairs):
     """python/PyHillFit.py:213-525 for all pairs at once (one sampler per number of experiments)."""
     import torch
-    from . import chainio
+    from . import chainio, ess
     from .packing import HierPack
     from .sampler import HierarchicalSampler, hier_priors
     pr, shapes, scales, locs = hier_priors()
@@ -232,32 +192,20 @@ def run_hierarchical(dr, args, pairs):
         ids = np.repeat(np.arange(len(grp), dtype=np.int32), R)
         theta0 = np.repeat(np.stack([j["theta0"] for j in grp]), R, axis=0)
         s = HierarchicalSampler(pack, ids, theta0, pr, seed=args.seed + ne, thinning=args.thinning)
-        chain = torch.empty((s.n, saved_iterations, s.d + 1), dtype=torch.float64, device=s.device)
-        chain[:, 0, :] = s.initial_row()
-        done = 0
         start = time.time()
-        while done < args.iterations:
-            k = min(args.segment - args.segment % args.thinning or args.thinning, args.iterations - done)
-            r0 = done // args.thinning + 1
-            seg = s.run(k)
-            chain[:, r0:r0 + seg.shape[1], :] = seg
-            done += k
+        chain = s.collect(args.iterations, args.segment)
         torch.cuda.synchronize()
         print("{} hierarchical chains (Ne={}) x {} iterations in {:.2f} s".format(s.n, ne, args.iterations, time.time() - start))
-        diag = run_diagnostics(args, chain, len(grp), R, burn)
-        host = chain.cpu().numpy()
+        diag = ess.targets_diagnostics(chain, len(grp), R, burn) if args.diagnostics else None
+        host = chain.cpu().numpy().reshape(len(grp), R, saved_iterations, s.d + 1)
         rng = np.random.RandomState(args.seed)
         for j, job in enumerate(grp):
-            for r in range(R):
-                f = job["chain_file"] if r == 0 else chainio.extra_chain_name(job["chain_file"], r)
-                chainio.save_hierarchical_chain(f, host[j * R + r])     # whole chain, burn-in kept (PyHillFit.py:514-515)
-            if diag is not None:
-                names = ["alpha", "beta", "mu", "s"] + [p + "_{}".format(e + 1) for e in range(ne) for p in ("pIC50", "Hill")]
-                chainio.save_diagnostics(job["chain_file"], diag[j], names + ["sigma", "log-target"], R, burn,
-                                         saved_iterations)
+            # whole chains, burn-in kept (PyHillFit.py:514-515)
+            chainio.save_target_chains(job["chain_file"], host[j], chainio.save_hierarchical_chain,
+                                       None if diag is None else diag[j], chainio.hierarchical_columns(ne), burn)
             samples_file = dr.alpha_mu_downsampling(job["drug"], job["channel"])
             print("saving (alpha,mu) samples to", samples_file)
-            chainio.save_alpha_mu_samples(samples_file, host[j * R], burn, args.num_APs, job["drug"], job["channel"], rng)
+            chainio.save_alpha_mu_samples(samples_file, host[j, 0], burn, args.num_APs, job["drug"], job["channel"], rng)
             print("\n\n{} + {} complete!\n\n".format(job["drug"], job["channel"]))
     return jobs
 

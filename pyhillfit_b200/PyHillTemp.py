@@ -47,43 +47,26 @@ def do_mcmc_all_temperatures(dr, args, concs, responses, temperatures):
     """python/PyHillTemp.py:57-125 for every temperature (x replicates) at once -> [T, R, rows, d+1] host array
     of post-burn rows, the in-kernel mean temperature-1 log-likelihoods [T, R], with --diagnostics the
     [T, d+1, 5] diagnostics of each temperature's R chains (else None) and, with --swap-every, the [R, T-1, 2]
-    (attempted, accepted) swap counts of each replicate's ladder (else None)."""
+    (attempted, accepted) swap counts of each replicate's ladder (else None).  The chains are those of pair 0 of
+    ti.run_ti: its chain list, its ladders and its Philox ids."""
     import torch
+    from . import ess, ti
     from .packing import SinglePack
-    from .sampler import SingleLevelSampler
+    from .sampler import SingleLevelSampler, model_chain_id_base
     R = args.num_chains
     T = len(temperatures)
-    d = dr.num_params
     num_saved = args.iterations // args.thinning + 1
     burn = num_saved // args.burn_in_fraction
-    pack = SinglePack([(concs, responses)])
-    tt = np.repeat(np.asarray(temperatures, dtype=np.float64), R)
-    # models 1 and 2 are run by separate invocations with the same --seed: the model goes into the Philox chain id
-    # (as pyhillfit_b200/ti.py does) so that chain k of model 1 and chain k of model 2 do not share their draws
-    s = SingleLevelSampler(args.model, pack, np.zeros(T * R, dtype=np.int32), tt, np.ones((T * R, d)), variant="temp",
-                           seed=args.seed, chain_id_base=(args.model - 1) * (1 << 40), thinning=args.thinning,
-                           burn_rows=burn)
+    ids, tt = ti.build_chain_list(1, temperatures, R)
+    s = SingleLevelSampler(args.model, SinglePack([(concs, responses)]), ids, tt, np.ones((T * R, dr.num_params)),
+                           variant="temp", seed=args.seed, chain_id_base=model_chain_id_base(args.model),
+                           thinning=args.thinning, burn_rows=burn)
     # only the rows the reference keeps (chain[burn:], PyHillTemp.py:125) are written by the kernel and copied back
-    kept = num_saved - max(burn, 0)
-    chain = torch.empty((s.n, kept, d + 1), dtype=torch.float64, device=s.device)
-    at = 0
-    if burn == 0:
-        chain[:, 0, :] = s.initial_row()
-        at = 1
-    # --swap-every: ladder r is the R-strided column of replicate r, global id (model - 1) 2^40 + r (pair 0 of ti.run_ti)
-    ladders = np.arange(T * R).reshape(T, R).T
-    done = 0
-    while done < args.iterations:
-        k = min(args.segment - args.segment % args.thinning or args.thinning, args.iterations - done)
-        seg = s.run_swapping(k, args.swap_every, ladders, (args.model - 1) * (1 << 40), discard_burn=True)
-        chain[:, at:at + seg.shape[1], :] = seg
-        at += seg.shape[1]
-        done += k
+    chain = s.collect(args.iterations, args.segment, discard_burn=True, swap_every=args.swap_every,
+                      ladders=ti.pair_ladders(0, 1, T, R), ladder_id_base=ti.ladder_id_base(args.model, 0, R))
     torch.cuda.synchronize()
-    assert at == kept
-    from .PyHillFit import run_diagnostics
-    diag = run_diagnostics(args, chain, T, R, 0)
-    host = chain.cpu().numpy().reshape(T, R, kept, d + 1)
+    diag = ess.targets_diagnostics(chain, T, R, 0) if args.diagnostics else None
+    host = chain.cpu().numpy().reshape(T, R, chain.shape[1], s.d + 1)
     counts = s.swap_counts.cpu().numpy() if args.swap_every > 0 else None
     return host, s.loglik_t1_mean().reshape(T, R), diag, counts
 
@@ -95,15 +78,14 @@ def main(argv=None):
         parser.print_help()
         return 1
     args = parser.parse_args(argv)
-    from . import chainio
+    from . import chainio, ti
     from . import doseresponse as dr
     dr.define_model(args.model)
     dr.setup(args.data_file)
     drug, channel = dr.drugs[args.drug], dr.channels[args.channel]
     num_expts, experiment_numbers, experiments = dr.load_crumb_data(drug, channel)
-    concs = np.concatenate([experiments[i][:, 0] for i in range(num_expts)])
-    responses = np.concatenate([experiments[i][:, 1] for i in range(num_expts)])
-    temperatures = (np.arange(dr.n + 1.) / dr.n) ** dr.c
+    concs, responses = dr.concat_experiments(experiments, num_expts)
+    temperatures = ti.temperature_ladder()
     print("\nDoing temperatures: {}\n".format(temperatures))
     start = time.time()
     if args.swap_every < 0:
@@ -113,12 +95,8 @@ def main(argv=None):
     for i, temperature in enumerate(temperatures):
         cdrug, cchannel, chain_file, images_dir = dr.nonhierarchical_chain_file_and_figs_dir(args.model, drug, channel, temperature)
         print("chain_file:", chain_file)
-        for r in range(args.num_chains):
-            f = chain_file if r == 0 else chainio.extra_chain_name(chain_file, r)
-            chainio.save_tempered_chain(f, chains[i, r])
-        if diag is not None:
-            names = ["pIC50", "sigma"] if args.model == 1 else ["pIC50", "Hill", "sigma"]
-            chainio.save_diagnostics(chain_file, diag[i], names + ["log-target"], args.num_chains, 0, chains.shape[2])
+        chainio.save_target_chains(chain_file, chains[i], chainio.save_tempered_chain,
+                                   None if diag is None else diag[i], chainio.single_level_columns(args.model))
     if swaps is not None:
         f, acc = chainio.save_swap_acceptance(chain_file, temperatures, swaps, args.swap_every)
         print("swap acceptance per rung (t_k, t_k+1), pooled over {} ladder(s):".format(args.num_chains))

@@ -33,6 +33,29 @@ def save_hierarchical_chain(chain_file, chain):
                                 "# alpha, beta, mu, s, hill_1, pic50_1, hill_2, pic50_2, ..., hill_Ne, pic50_Ne, sigma\n")
 
 
+def single_level_columns(model):
+    """Names of the columns of a single-level chain file of `model`."""
+    return (["pIC50", "sigma"] if model == 1 else ["pIC50", "Hill", "sigma"]) + ["log-target"]
+
+
+def hierarchical_columns(n_expts):
+    """Names of the columns of a hierarchical chain file with n_expts experiments."""
+    return (["alpha", "beta", "mu", "s"] + [p + "_{}".format(e + 1) for e in range(n_expts) for p in ("pIC50", "Hill")]
+            + ["sigma", "log-target"])
+
+
+def save_target_chains(chain_file, chains, save, diag=None, names=None, row_begin=0):
+    """The R chains [R, rows, d+1] of one target: chain 0 to chain_file, chain r > 0 to extra_chain_name(chain_file, r),
+    each written by save(file, chain); with `diag` ([d+1, 5] of ess.chain_diagnostics over rows row_begin .. rows-1),
+    also the diagnostics file beside chain_file, its columns named `names` (one name per row of `diag`)."""
+    if diag is not None and (names is None or len(names) != len(diag)):
+        raise ValueError("diagnostics need one column name per row of diag")
+    for r, chain in enumerate(chains):
+        save(chain_file if r == 0 else extra_chain_name(chain_file, r), chain)
+    if diag is not None:
+        save_diagnostics(chain_file, diag, names, len(chains), row_begin, chains.shape[1])
+
+
 def save_alpha_mu_samples(samples_file, chain, burn, num_APs, drug, channel, rng=None):
     rng = np.random if rng is None else rng
     saved_iterations = chain.shape[0]

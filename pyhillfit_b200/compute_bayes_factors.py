@@ -45,8 +45,7 @@ def run_all_fused(dr, args):
             num_expts, experiment_numbers, experiments = dr.load_crumb_data(top_drug, top_channel)
         except Exception:
             continue
-        concs = np.concatenate([experiments[i][:, 0] for i in range(num_expts)])
-        responses = np.concatenate([experiments[i][:, 1] for i in range(num_expts)])
+        concs, responses = dr.concat_experiments(experiments, num_expts)
         if np.any(np.isnan(responses)):
             continue
         drug, channel, chain_file, images_dir = dr.nonhierarchical_chain_file_and_figs_dir(1, top_drug, top_channel, 1)
@@ -92,6 +91,7 @@ def main(argv=None):
     from . import chainio
     from . import doseresponse as dr
     from .packing import SinglePack
+    from .ti import temperature_ladder
     dr.setup(args.data_file)
     if args.all_fused:
         return run_all_fused(dr, args)
@@ -99,13 +99,11 @@ def main(argv=None):
         parser.error("the following arguments are required: -d/--drug, -c/--channel")
     top_drug, top_channel = dr.drugs[args.drug], dr.channels[args.channel]
     num_expts, experiment_numbers, experiments = dr.load_crumb_data(top_drug, top_channel)
-    concs = np.concatenate([experiments[i][:, 0] for i in range(num_expts)])
-    responses = np.concatenate([experiments[i][:, 1] for i in range(num_expts)])
-    pack = SinglePack([(concs, responses)])
+    pack = SinglePack([dr.concat_experiments(experiments, num_expts)])
     expectations = {}
     for m in (1, 2):
         dr.define_model(m)
-        temps = (np.arange(dr.n + 1.) / dr.n) ** dr.c
+        temps = temperature_ladder()
         log_p_ys = np.zeros(len(temps))
         for i, temp in enumerate(temps):
             print(temp)

@@ -110,6 +110,13 @@ def load_crumb_data(drug, channel):
     return num_expts, experiment_numbers, experiments
 
 
+def concat_experiments(experiments, num_expts):
+    """(concs, responses) of experiments 0 .. num_expts-1 of a pair, one after the other (PyHillFit.py:661-665)."""
+    concs = np.concatenate([experiments[i][:, 0] for i in range(num_expts)])
+    responses = np.concatenate([experiments[i][:, 1] for i in range(num_expts)])
+    return concs, responses
+
+
 # ---------------------------------------------------------------------------------------------
 # output tree (:70-82, 93-141, 196-200, 320-348): byte-identical paths; '/' in names becomes '_'
 # ---------------------------------------------------------------------------------------------

@@ -9,6 +9,7 @@ The same function is applied to GPU chains and to CPU-reference chains.
 `phf_chain_diagnostics` (csrc/phf_diag.cu, `chain_diagnostics_gpu`) compute from chains already in HBM.
 """
 import math
+import time
 
 import numpy as np
 
@@ -134,6 +135,19 @@ def diagnostics_summary(diag, rhat_limit=1.01):
     worst = diag[:, :, 2].max(axis=1)
     return "diagnostics: {} of {} groups with max R-hat > {}; smallest ESS {:.1f}".format(
         int(np.count_nonzero(worst > rhat_limit)), diag.shape[0], rhat_limit, float(diag[:, :, 3].min()))
+
+
+def targets_diagnostics(chain, n_targets, R, row_begin):
+    """--diagnostics of the command lines: split R-hat / multi-chain ESS of each target's R chains from rows
+    [row_begin, ...) of the device tensor `chain` [n_targets * R, rows, d+1], with the summary line printed; None (and
+    a note printed) when there are fewer than 8 such rows."""
+    if chain.shape[1] - row_begin < 8:
+        print("--diagnostics: fewer than 8 rows per chain, no diagnostics written")
+        return None
+    t_phase = time.time()
+    diag = chain_diagnostics_gpu(chain, np.arange(n_targets + 1) * R, row_begin=row_begin)
+    print("{} ({:.2f} s)".format(diagnostics_summary(diag), time.time() - t_phase))
+    return diag
 
 
 def mcse_mean(x):

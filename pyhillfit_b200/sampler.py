@@ -15,6 +15,19 @@ from .packing import HierPack, SinglePack
 NO_BURN = 0xFFFFFFFF
 
 
+def model_chain_id_base(model):
+    """First Philox chain id of `model`'s chains.  Models 1 and 2 run with the same seed, so their id ranges must not
+    overlap: otherwise chain k of one model would share its draws with chain k of the other."""
+    return (model - 1) << 40
+
+
+def segment_lengths(n_iters, segment, thinning):
+    """Iterations of each launch of a run of n_iters split into segments: `segment` rounded down to a multiple of
+    thinning (at least one thinning), the last launch taking what is left."""
+    step = segment - segment % thinning or thinning
+    return [min(step, n_iters - done) for done in range(0, n_iters, step)]
+
+
 def variant_defaults(variant, theta0):
     """(cov0 [n,d,d], adapt_when, reset_mean) -- SURVEY.md section 3.5 / the reference lines cited there."""
     theta0 = np.atleast_2d(np.asarray(theta0, dtype=np.float64))
@@ -75,6 +88,10 @@ def validate_ladders(ladders, dataset_id, temperature):
 
 class _Base:
     d = None
+    model = 0            # AmConfig.model: 1 or 2 single-level, 0 hierarchical
+    speculation = 1
+    occupancy_hint = 0   # developer knobs, set on an instance (bench.py, scripts/)
+    cta_order = 0
 
     def _alloc_common(self, n, theta0, cov0, device):
         torch = _lib.require_cuda()
@@ -116,13 +133,56 @@ class _Base:
 
     def _config(self, n_iters, rows_capacity, row_major=False, discard_burn=False):
         return _lib.AmConfig(discard_burn_rows=int(bool(discard_burn)), sample_layout=_lib.SAMPLES_ROW_MAJOR if row_major else _lib.SAMPLES_CHAIN_MAJOR,
-                             model=getattr(self, "model", 0), reset_mean_at_adapt=int(self.reset_mean), t0=self.t,
+                             model=self.model, reset_mean_at_adapt=int(self.reset_mean), t0=self.t,
                              n_iters=int(n_iters), thinning=self.thinning, adapt_when=int(self.adapt_when),
                              burn_rows=int(self.burn_rows), rows_capacity=int(rows_capacity), seed=int(self.seed),
                              chain_id_base=int(self.chain_id_base), stage_groups=int(self.stage_groups),
-                             block_threads=int(self.block_threads), lanes_per_chain=int(getattr(self, "lanes", 0)),
-                             min_ctas_hint=int(getattr(self, "occupancy_hint", 0)),
-                             cta_order=int(getattr(self, "cta_order", 0)), speculation=int(getattr(self, "speculation", 1)))
+                             block_threads=int(self.block_threads), lanes_per_chain=int(self.lanes),
+                             min_ctas_hint=int(self.occupancy_hint), cta_order=int(self.cta_order),
+                             speculation=int(self.speculation))
+
+    def initial_row(self):
+        """[n, d+1] row 0 of every chain: (theta0, log_target(theta0)) -- call before run()."""
+        return self.state[:, :self.d + 1].clone()
+
+    def run(self, n_iters, samples=None, keep=True, row_major=False, discard_burn=False):
+        """Advance every chain by n_iters.  Returns the device tensor of rows saved by this call (a view of `samples`
+        if given): [n, rows, d+1], or [rows, n, d+1] with row_major=True (one saved iteration of all chains
+        contiguous: coalesced write-out, contiguous transfers); None when keep=False (thermodynamic-integration-only
+        runs).  discard_burn=True: rows with index < burn_rows are not written at all (what PyHillFit.py:861-864 and
+        PyHillTemp.py:125 drop before saving); the returned rows start at max(burn_rows, first row of this call)."""
+        rows = self.rows_for(n_iters, discard_burn)
+        cap = rows
+        if keep:
+            samples, cap = self._samples_buffer(samples, rows, row_major)
+            assert samples.is_contiguous()
+        cfg = self._config(n_iters, cap, row_major, discard_burn)
+        with self.torch.cuda.device(self.device):
+            self._launch(cfg, samples.data_ptr() if keep else None, _lib.current_stream_ptr())
+        self.t += int(n_iters)
+        if not keep:
+            return None
+        return samples[:rows] if row_major else samples[:, :rows]
+
+    def collect(self, n_iters, segment, discard_burn=False, swap_every=0, ladders=None, ladder_id_base=0):
+        """Advance every chain by n_iters, one run() per segment_lengths(n_iters, segment, thinning), and return the
+        device tensor [n, rows, d+1] of every row saved: row 0 (the start state, on a sampler that has not run yet)
+        first unless discard_burn drops it, then each segment's rows.  swap_every > 0: each segment is
+        run_swapping(k, swap_every, ladders, ladder_id_base).  Neither synchronises nor copies to the host."""
+        lead = int(self.t == 0 and not (discard_burn and self.burn_rows not in (0, NO_BURN)))
+        chain = self.torch.empty((self.n, lead + self.rows_for(n_iters, discard_burn), self.d + 1),
+                                 dtype=self.torch.float64, device=self.device)
+        if lead:
+            chain[:, 0] = self.initial_row()
+        at = lead
+        for k in segment_lengths(n_iters, segment, self.thinning):
+            if swap_every > 0:
+                seg = self.run_swapping(k, swap_every, ladders, ladder_id_base, discard_burn=discard_burn)
+            else:
+                seg = self.run(k, discard_burn=discard_burn)
+            chain[:, at:at + seg.shape[1]] = seg
+            at += seg.shape[1]
+        return chain
 
 
 class SingleLevelSampler(_Base):
@@ -204,29 +264,6 @@ class SingleLevelSampler(_Base):
         if n_threads <= sms * 16 * 64:
             return 64
         return 128
-
-    def initial_row(self):
-        """[n, d+1] row 0 of every chain: (theta0, log_target(theta0)) -- call before run()."""
-        return self.state[:, :self.d + 1].clone()
-
-    def run(self, n_iters, samples=None, keep=True, row_major=False, discard_burn=False):
-        """Advance every chain by n_iters.  Returns the device tensor of rows saved by this call (a view of `samples`
-        if given): [n, rows, d+1], or [rows, n, d+1] with row_major=True (one saved iteration of all chains
-        contiguous: coalesced write-out, contiguous transfers); None when keep=False (thermodynamic-integration-only
-        runs).  discard_burn=True: rows with index < burn_rows are not written at all (what PyHillFit.py:861-864 and
-        PyHillTemp.py:125 drop before saving); the returned rows start at max(burn_rows, first row of this call)."""
-        rows = self.rows_for(n_iters, discard_burn)
-        cap = rows
-        if keep:
-            samples, cap = self._samples_buffer(samples, rows, row_major)
-            assert samples.is_contiguous()
-        cfg = self._config(n_iters, cap, row_major, discard_burn)
-        with self.torch.cuda.device(self.device):
-            self._launch(cfg, samples.data_ptr() if keep else None, _lib.current_stream_ptr())
-        self.t += int(n_iters)
-        if not keep:
-            return None
-        return samples[:rows] if row_major else samples[:, :rows]
 
     def run_swapping(self, n_iters, swap_every, ladders, ladder_id_base=0, samples=None, keep=True, row_major=False,
                      discard_burn=False):
@@ -353,24 +390,12 @@ class HierarchicalSampler(_Base):
                                                     self.state.data_ptr(), _lib.current_stream_ptr()),
                        "phf_am_hier_init")
 
-    def initial_row(self):
-        return self.state[:, :self.d + 1].clone()
-
-    def run(self, n_iters, samples=None, row_major=False):
-        """Advance every chain by n_iters; returns the rows saved by this call: [n, rows, dim+1], or [rows, n, dim+1]
-        with row_major=True (one saved iteration of all chains contiguous, as in SingleLevelSampler.run)."""
-        torch = self.torch
-        rows = self.rows_for(n_iters)
-        samples, cap = self._samples_buffer(samples, rows, row_major)
-        assert samples.is_contiguous()
-        cfg = self._config(n_iters, cap, row_major)
-        with torch.cuda.device(self.device):
-            _lib.check(_lib.load().phf_am_hier_run(C.byref(cfg), self.n_expts, self.n, self.state.data_ptr(),
-                                                   self.dataset_id.data_ptr(), self.ds_dev.data_ptr(),
-                                                   self.pts_dev.data_ptr(), C.byref(self.priors),
-                                                   samples.data_ptr(), _lib.current_stream_ptr()), "phf_am_hier_run")
-        self.t += int(n_iters)
-        return samples[:rows] if row_major else samples[:, :rows]
+    def _launch(self, cfg, samples_ptr, stream):
+        """phf_am_hier_run of every chain with `cfg`, writing rows to `samples_ptr` (None: no rows)"""
+        _lib.check(_lib.load().phf_am_hier_run(C.byref(cfg), self.n_expts, self.n, self.state.data_ptr(),
+                                               self.dataset_id.data_ptr(), self.ds_dev.data_ptr(),
+                                               self.pts_dev.data_ptr(), C.byref(self.priors), samples_ptr, stream),
+                   "phf_am_hier_run")
 
 
 def hier_priors():

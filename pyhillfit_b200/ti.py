@@ -13,7 +13,7 @@ from . import _lib as phf_lib
 from . import dist as phf_dist
 from . import doseresponse as dr
 from .packing import SinglePack
-from .sampler import SingleLevelSampler
+from .sampler import SingleLevelSampler, model_chain_id_base
 
 
 def temperature_ladder(n=None, c=None):
@@ -49,8 +49,8 @@ def pair_ladders(pair_lo, pair_hi, T, R):
 
 
 def ladder_id_base(model, pair_lo, R):
-    """Global id of ladder (pair_lo, 0) of `model`: ladder (pair, r) is (model - 1) 2^40 + pair R + r."""
-    return (model - 1) * (1 << 40) + pair_lo * R
+    """Global id of ladder (pair_lo, 0) of `model`: ladder (pair, r) is model_chain_id_base(model) + pair R + r."""
+    return model_chain_id_base(model) + pair_lo * R
 
 
 def run_ti(datasets, models=(1, 2), temps=None, replicates=1, iterations=500000, thinning=5, burn_in_fraction=4,
@@ -88,7 +88,7 @@ def run_ti(datasets, models=(1, 2), temps=None, replicates=1, iterations=500000,
         for model in models:
             d = 2 if model == 1 else 3
             samplers[model] = SingleLevelSampler(model, pack, ids[lo:hi], tt[lo:hi], np.ones((hi - lo, d)),
-                                                 variant="temp", seed=seed, chain_id_base=(model - 1) * (1 << 40) + lo,
+                                                 variant="temp", seed=seed, chain_id_base=model_chain_id_base(model) + lo,
                                                  thinning=thinning, burn_rows=burn, device=dev, lanes=lanes, speculation=speculation,
                                                  co_resident_chains=(hi - lo) * (len(models) - 1))
             streams[model] = torch.cuda.Stream(device=dev)

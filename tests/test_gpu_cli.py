@@ -5,24 +5,9 @@ import os
 import numpy as np
 import pytest
 
-from _data import GOLD
+from _fixtures import crumb_csv  # noqa: F401  (fixture)
 
 pytestmark = pytest.mark.gpu
-
-
-@pytest.fixture()
-def crumb_csv(tmp_path, monkeypatch):
-    """data/crumb_data.csv rebuilt from the packaged fixture (the reference tree is not on the GPU box)."""
-    z = np.load(os.path.join(GOLD, "datasets.npz"))
-    os.makedirs(tmp_path / "data")
-    f = tmp_path / "data" / "crumb_data.csv"
-    with open(f, "w") as out:
-        out.write("Compound,Channel,Experiment,Dose,Response\n")
-        for row in zip(z["crumb_data__drug"], z["crumb_data__channel"], z["crumb_data__experiment"],
-                       z["crumb_data__dose"], z["crumb_data__response"]):
-            out.write("%s,%s,%d,%r,%r\n" % (row[0], row[1], row[2], float(row[3]), float(row[4])))
-    monkeypatch.chdir(tmp_path)
-    return str(f)
 
 
 def test_pyhillfit_single_level_cli(crumb_csv):

@@ -7,6 +7,7 @@ import numpy as np
 import pytest
 
 from _data import Table
+from _fixtures import crumb_csv  # noqa: F401  (fixture)
 from pyhillfit_b200 import ess
 
 pytestmark = pytest.mark.gpu
@@ -142,21 +143,6 @@ def test_rhat_flags_chains_of_two_different_pairs():
 
 
 # ---- command lines ---------------------------------------------------------------------------------------------
-
-@pytest.fixture()
-def crumb_csv(tmp_path, monkeypatch):
-    from _data import GOLD
-    z = np.load(os.path.join(GOLD, "datasets.npz"))
-    os.makedirs(tmp_path / "data")
-    f = tmp_path / "data" / "crumb_data.csv"
-    with open(f, "w") as out:
-        out.write("Compound,Channel,Experiment,Dose,Response\n")
-        for row in zip(z["crumb_data__drug"], z["crumb_data__channel"], z["crumb_data__experiment"],
-                       z["crumb_data__dose"], z["crumb_data__response"]):
-            out.write("%s,%s,%d,%r,%r\n" % (row[0], row[1], row[2], float(row[3]), float(row[4])))
-    monkeypatch.chdir(tmp_path)
-    return str(f)
-
 
 def _check_diagnostics_file(chain_file, n_chains, row_begin, n_cols):
     from pyhillfit_b200 import chainio

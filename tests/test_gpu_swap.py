@@ -1,15 +1,14 @@
 """Population MCMC on the GPU: the swap kernel against the C swap round and phf_log_target_batch, GPU ladders against
 the C ladder loop step by step, invariance under speculation, sharding and swap intervals longer than the run,
 reproducibility, and the command lines."""
-import os
-
 import numpy as np
 import pytest
 
 import c_oracle
 import hill_oracle as ho
 import swap_oracle
-from _data import GOLD, Table
+from _data import Table
+from _fixtures import crumb_csv  # noqa: F401  (fixture)
 
 pytestmark = pytest.mark.gpu
 
@@ -160,20 +159,6 @@ def test_run_ti_with_swaps_is_reproducible(table):
         assert acc.shape == (3, 2, 40) and np.all(np.isfinite(acc)) and np.all((acc >= 0) & (acc <= 1))
     c = ti.run_ti(data, **dict(kw, swap_every=0))
     assert a["means_per_replicate_2"].tobytes() != c["means_per_replicate_2"].tobytes()
-
-
-@pytest.fixture()
-def crumb_csv(tmp_path, monkeypatch):
-    z = np.load(os.path.join(GOLD, "datasets.npz"))
-    os.makedirs(tmp_path / "data")
-    f = tmp_path / "data" / "crumb_data.csv"
-    with open(f, "w") as out:
-        out.write("Compound,Channel,Experiment,Dose,Response\n")
-        for row in zip(z["crumb_data__drug"], z["crumb_data__channel"], z["crumb_data__experiment"],
-                       z["crumb_data__dose"], z["crumb_data__response"]):
-            out.write("%s,%s,%d,%r,%r\n" % (row[0], row[1], row[2], float(row[3]), float(row[4])))
-    monkeypatch.chdir(tmp_path)
-    return str(f)
 
 
 def _chain_files(model, temps):
