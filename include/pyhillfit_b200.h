@@ -363,6 +363,54 @@ int phf_chain_diagnostics(int64_t n_chains, int64_t n_rows_total, int64_t row_be
                           double *out, void *stream);
 
 /* ------------------------------------------------------------------------------------------------
+ * Leave-one-out model comparison (the reference has none): Pareto-smoothed importance-sampling LOO (PSIS-LOO) and WAIC
+ * per measurement from temperature-1 draws, as defined by pyhillfit_b200/loo.py (pointwise_loglik, psis_loo).
+ *
+ * One measurement of a single-level dataset, in the order of the concatenated responses (python/PyHillFit.py:661-665).
+ * Its log-likelihood at theta, with p the Hill curve at the point's dose and the masks of python/PyHillFit.py:675-677:
+ *   kind 0 (y == 0)        log Phi((0 - p) / sigma) - ln(2 pi) / 2
+ *   kind 1 (y == 100)      log Phi((p - 100) / sigma) - ln(2 pi) / 2
+ *   kind 2 (0 < y < 100)   -ln sigma - (y - p)^2 / (2 sigma^2) - ln(2 pi) / 2
+ *   kind 3 (in no mask)    -ln(2 pi) / 2
+ * The sum over a dataset's points is its temperature-1 log-likelihood (pi_bit counts all N points, so a censored or
+ * dropped point carries its -ln(2 pi) / 2 too: the same constant in both models).  sigma <= 1e-3 gives -inf.
+ * ---------------------------------------------------------------------------------------------- */
+typedef struct phf_point { /* 16 bytes */
+    int32_t group;   /* absolute index of the point's phf_dose_group (the dose) */
+    int32_t kind;    /* 0 zero, 1 hundred, 2 other, 3 in no mask */
+    double y;        /* response */
+} phf_point;
+
+/* Pointwise log-likelihood of every draw of every group.  Group g is chains chain_offsets[g] .. chain_offsets[g+1]-1 of
+ * a chain-major samples buffer [n_chains][n_rows_total][d+1] (what the single-level samplers write; d = 2 for model 1,
+ * 3 for model 2), rows row_begin .. n_rows_total-1 of each chain: S_g = chains x rows draws ordered (chain, row); and
+ * points point_offsets[g] .. point_offsets[g+1]-1 of `points`, whose groups the caller has checked to lie in the group's
+ * dataset (pyhillfit_b200/loo.py:validate_points).
+ *   loglik  DEVICE, out: one column per point, in point order, each column's S_g draws contiguous (sum_g n_points_g S_g
+ *           doubles)
+ * chain_offsets (strictly increasing) and point_offsets (non-decreasing) are HOST arrays of n_groups + 1 entries.
+ * Arguments are checked before any CUDA call (PHF_EINVAL).  Asynchronous on `stream`; takes a stream-ordered temporary
+ * of 48 bytes per group. */
+int phf_single_pointwise_loglik(int model, int64_t n_rows_total, int64_t row_begin, const double *samples,
+                                int32_t n_groups, const int64_t *chain_offsets /* HOST */,
+                                const int64_t *point_offsets /* HOST */, const phf_point *points,
+                                const phf_dose_group *groups, double *loglik, void *stream);
+
+/* largest draws per column phf_psis_loo accepts: M = ceil(min(0.2 S, 3 sqrt S)) <= 16384 tail draws, sorted in shared
+ * memory (256 chains x 75 001 rows is S = 19.2 M, M = 13 146) */
+#define PHF_LOO_MAX_DRAWS 29826161
+
+/* PSIS-LOO and WAIC terms of n_cols columns of a flat DEVICE buffer: column c is loglik[col_offsets[c] ..
+ * col_offsets[c+1]) (HOST offsets, non-decreasing; the columns may be any log-likelihood, not only the single-level one).
+ *   out  DEVICE, [n_cols][5]: elpd_loo_i, lppd_i, p_waic_i, khat_i, tail_len.  A column with a non-finite value gives
+ *        NaN and tail_len -1; a constant column gives elpd_loo_i = lppd_i = its value, p_waic_i = khat_i = 0, tail_len 0.
+ * A column needs 2 .. PHF_LOO_MAX_DRAWS draws (fewer: PHF_EINVAL, more: PHF_ENOTSUP), checked before any CUDA call.
+ * Asynchronous on `stream`; takes a stream-ordered temporary of about S / 256 + M doubles per column.  Deterministic:
+ * fixed-order sums over partitions that depend on the shapes alone, the same bits on every call. */
+int phf_psis_loo(int32_t n_cols, const int64_t *col_offsets /* HOST */, const double *loglik, double *out,
+                 void *stream);
+
+/* ------------------------------------------------------------------------------------------------
  * Utilities
  * ---------------------------------------------------------------------------------------------- */
 int phf_version(void);

@@ -34,6 +34,9 @@ def build_parser():
     parser.add_argument("--diagnostics", action='store_true', default=False,
                         help="split R-hat and multi-chain ESS of each pair's chains, computed on the GPU, written "
                              "beside the chain file as ..._diagnostics.txt [new]")
+    parser.add_argument("--loo", action='store_true', default=False,
+                        help="single-level only: PSIS-LOO and WAIC per measurement from each pair's chains, computed on "
+                             "the GPU, written beside the chain file as ..._loo.txt [new]")
     requiredNamed = parser.add_argument_group('required arguments')
     requiredNamed.add_argument("--data-file", type=str, help="csv file from which to read in data, in same format as provided crumb_data.csv", required=True)
     requiredNamed.add_argument("-m", "--model", type=int, help="For non-hierarchical (put anything for hierarchical):1. fix Hill=1; 2. vary Hill", required=True)
@@ -54,7 +57,7 @@ def select_pairs(dr, args):
 def run_single_level(dr, args, pairs):
     """python/PyHillFit.py:645-867 for all pairs at once."""
     import torch
-    from . import chainio, ess
+    from . import chainio, ess, loo
     from .initial_fit import best_fit_batch_gpu as best_fit_batch   # phf_best_fit_batch, one thread per dataset
     from .packing import SinglePack
     from .sampler import SingleLevelSampler, model_chain_id_base
@@ -104,6 +107,7 @@ def run_single_level(dr, args, pairs):
     torch.cuda.synchronize()
     print("\n{} chains x {} iterations in {:.2f} s on the GPU\n".format(s.n, args.iterations, time.time() - start))
     diag = ess.targets_diagnostics(chain, len(jobs), R, 0) if args.diagnostics else None
+    loo_rows, loo_draws = loo.targets_loo(chain, pack, R, args.model) if args.loo else (None, 0)
     t_phase = time.time()
     host = chain.cpu().numpy().reshape(len(jobs), R, chain.shape[1], s.d + 1)
     print("chains to the host: {:.2f} s".format(time.time() - t_phase))
@@ -112,6 +116,9 @@ def run_single_level(dr, args, pairs):
         chainio.save_target_chains(job["chain_file"], host[j],
                                    lambda f, c: chainio.save_single_level_chain(f, c, job["drug"], job["channel"]),
                                    None if diag is None else diag[j], chainio.single_level_columns(args.model))
+        if loo_rows is not None:
+            chainio.save_loo(job["chain_file"], loo_rows[j], data[j][0], data[j][1], args.model, job["drug"],
+                             job["channel"], loo_draws)
         print("\n\n{} + {} complete!\n\n".format(job["drug"], job["channel"]))
     print("chain files: {:.2f} s".format(time.time() - t_phase))
     return jobs
@@ -217,6 +224,8 @@ def main(argv=None):
         parser.print_help()
         return 1
     args = parser.parse_args(argv)
+    if args.loo and args.hierarchical:
+        parser.error("--loo is for the single-level models (the hierarchical likelihood is a different one)")
     t_import = time.time()
     from . import doseresponse as dr
     dr.define_model(args.model)

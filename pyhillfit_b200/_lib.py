@@ -43,7 +43,8 @@ DATASET_DTYPE = np.dtype([("group_begin", "<i4"), ("n_groups", "<i4"), ("pi_bit"
                           ("n_other_total", "<f8"), ("reserved", "<f8")])
 HIER_POINT_DTYPE = np.dtype([("lnc_hi", "<f8"), ("lnc_lo", "<f8"), ("y", "<f8"), ("expt", "<i4"), ("pad", "<i4")])
 HIER_DATASET_DTYPE = np.dtype([("point_begin", "<i4"), ("n_points", "<i4"), ("n_expts", "<i4"), ("pad", "<i4")])
-assert DOSE_GROUP_DTYPE.itemsize == 64 and DATASET_DTYPE.itemsize == 32
+POINT_DTYPE = np.dtype([("group", "<i4"), ("kind", "<i4"), ("y", "<f8")])
+assert DOSE_GROUP_DTYPE.itemsize == 64 and DATASET_DTYPE.itemsize == 32 and POINT_DTYPE.itemsize == 16
 assert HIER_POINT_DTYPE.itemsize == 32 and HIER_DATASET_DTYPE.itemsize == 16
 
 EXPORTS = ["phf_log_target_batch", "phf_am_single_init", "phf_am_single_run", "phf_am_single_lanes",
@@ -52,7 +53,8 @@ EXPORTS = ["phf_log_target_batch", "phf_am_single_init", "phf_am_single_run", "p
            "phf_release_workspaces", "phf_best_fit_batch",
            "phf_write_rows_text_host",
            "phf_hier_predictive_cdfs", "phf_format_e18", "phf_format_e18_mismatches", "phf_version", "phf_last_error",
-           "phf_fp64_peak_probe", "phf_launch_count", "phf_chain_diagnostics", "phf_am_single_swap"]
+           "phf_fp64_peak_probe", "phf_launch_count", "phf_chain_diagnostics", "phf_am_single_swap",
+           "phf_single_pointwise_loglik", "phf_psis_loo"]
 
 _lib = None
 _p = C.c_void_p
@@ -108,6 +110,8 @@ def load():
                                            C.c_int32]
     L.phf_best_fit_batch.argtypes = [C.c_int, C.c_int64, _p, _p, _p, C.c_double, _p, _p, _p]
     L.phf_chain_diagnostics.argtypes = [C.c_int64, C.c_int64, C.c_int64, C.c_int32, _p, C.c_int32, _p, C.c_int64, _p, _p]
+    L.phf_single_pointwise_loglik.argtypes = [C.c_int, C.c_int64, C.c_int64, _p, C.c_int32, _p, _p, _p, _p, _p, _p]
+    L.phf_psis_loo.argtypes = [C.c_int32, _p, _p, _p, _p]
     L.phf_format_e18.argtypes = [C.c_double, C.c_char_p]
     L.phf_format_e18_mismatches.argtypes = [_p, C.c_int64]
     L.phf_format_e18_mismatches.restype = C.c_int64

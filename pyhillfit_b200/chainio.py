@@ -112,6 +112,31 @@ def save_diagnostics(chain_file, diag, names, n_chains, row_begin, row_end):
     return f
 
 
+def loo_name(chain_file):
+    """File of the leave-one-out terms of one target's points (--loo), beside its chain file."""
+    root, ext = os.path.splitext(chain_file)
+    return "{}_loo{}".format(root, ext)
+
+
+def save_loo(chain_file, rows, concs, responses, model, drug, channel, n_draws):
+    """`#` header lines (model, pair, draws, khat threshold, totals of loo.summary), then one row per point:
+    index dose response elpd_loo_i lppd_i p_waic_i khat_i (np.loadtxt reads it)."""
+    from . import loo
+    s = loo.summary(rows, n_draws)
+    f = loo_name(chain_file)
+    with open(f, "w") as out:
+        out.write("# PSIS-LOO and WAIC per point, model {}, {} + {}\n".format(model, drug, channel))
+        out.write("# S = {} draws (chains x rows); khat threshold {:.6f}\n".format(n_draws, s["khat_threshold"]))
+        out.write("# elpd_loo {:.6f} +- {:.6f}, p_loo {:.6f}, elpd_waic {:.6f} +- {:.6f}, p_waic {:.6f}, "
+                  "{} of {} points with khat above the threshold\n".format(
+                      s["elpd_loo"], s["se_elpd_loo"], s["p_loo"], s["elpd_waic"], s["se_elpd_waic"], s["p_waic"],
+                      s["n_high_khat"], s["n"]))
+        out.write("# index dose response elpd_loo_i lppd_i p_waic_i khat_i\n")
+        for i, (c, y, r) in enumerate(zip(concs, responses, rows)):
+            out.write("{:d} {:.18e} {:.18e} {:.18e} {:.18e} {:.18e} {:.18e}\n".format(i, c, y, *r[:4]))
+    return f
+
+
 def swap_acceptance_name(chain_file):
     """File of the per-rung swap acceptance of one (drug, channel, model) ladder run (PyHillTemp --swap-every): in the
     model directory that holds the temperature_* directories, named after the chain file without its temperature."""

@@ -89,23 +89,58 @@ def pack_single_one(concs, responses, where_0=None, where_100=None, where_other=
     return g, float(pi_bit), float(np.count_nonzero(where_other))
 
 
+POINT_ZERO, POINT_HUNDRED, POINT_OTHER, POINT_NONE = 0, 1, 2, 3
+
+
+def point_kinds(where_0, where_100, where_other):
+    """phf_point.kind of each point from the three masks (the reference builds them disjoint; a point in none of them
+    is POINT_NONE)."""
+    k = np.full(np.shape(where_0), POINT_NONE, dtype=np.int32)
+    k[np.asarray(where_other, dtype=bool)] = POINT_OTHER
+    k[np.asarray(where_100, dtype=bool)] = POINT_HUNDRED
+    k[np.asarray(where_0, dtype=bool)] = POINT_ZERO
+    return k
+
+
+def point_list(concs, responses, where_0=None, where_100=None, where_other=None):
+    """-> phf_point records [N] of one dataset, in the order of its responses; `group` is the index of the point's dose
+    among the dataset's dose groups as pack_single_one orders them (order of first appearance)."""
+    concs = np.asarray(concs, dtype=np.float64).ravel()
+    y = np.asarray(responses, dtype=np.float64).ravel()
+    if where_0 is None:
+        where_0, where_100, where_other = masks(y)
+    index = {}
+    for cval in concs:
+        index.setdefault(cval, len(index))
+    pts = np.zeros(len(y), dtype=_lib.POINT_DTYPE)
+    pts["group"] = [index[cval] for cval in concs]
+    pts["kind"] = point_kinds(where_0, where_100, where_other)
+    pts["y"] = y
+    return pts
+
+
 class SinglePack:
     """Packed single-level datasets, host copies plus (lazily) device tensors."""
 
     def __init__(self, items):
         """items: iterable of (concs, responses) or dicts with optional masks / pi_bit."""
-        groups, ds = [], []
+        groups, ds, points = [], [], []
         begin = 0
         for it in items:
-            if isinstance(it, dict):
-                g, pb, no = pack_single_one(**it)
-            else:
-                g, pb, no = pack_single_one(*it)
+            kw = dict(it) if isinstance(it, dict) else dict(zip(("concs", "responses", "where_0", "where_100",
+                                                                 "where_other", "pi_bit"), it))
+            g, pb, no = pack_single_one(**kw)
+            kw.pop("pi_bit", None)
+            pts = point_list(**kw)
+            pts["group"] += begin
             groups.append(g)
+            points.append(pts)
             ds.append((begin, len(g), pb, no, 0.0))
             begin += len(g)
         self.groups = np.concatenate(groups) if groups else np.zeros(0, dtype=_lib.DOSE_GROUP_DTYPE)
         self.datasets = np.array(ds, dtype=_lib.DATASET_DTYPE)
+        self.points = np.concatenate(points) if points else np.zeros(0, dtype=_lib.POINT_DTYPE)
+        self.point_offsets = np.concatenate(([0], np.cumsum([len(p) for p in points], dtype=np.int64))).astype(np.int64)
         self._dev = {}
 
     @classmethod
@@ -147,6 +182,14 @@ class SinglePack:
         ds["pi_bit"] = 0.5 * len(concs) * np.log(2 * np.pi)
         ds["n_other_total"] = wo.sum(axis=1)
         self.datasets = ds
+        # point list: dataset k's points in column order, each pointing at its dose's group
+        first = np.array([uniq.index(cval) for cval in concs], dtype=np.int32)
+        pts = np.zeros((n_ds, len(concs)), dtype=_lib.POINT_DTYPE)
+        pts["group"] = np.arange(n_ds, dtype=np.int32)[:, None] * D + first[None, :]
+        pts["kind"] = point_kinds(w0, w100, wo)
+        pts["y"] = Y
+        self.points = pts.reshape(-1)
+        self.point_offsets = np.arange(n_ds + 1, dtype=np.int64) * len(concs)
         return self
 
     @property
@@ -161,6 +204,15 @@ class SinglePack:
             g = torch.from_numpy(self.groups.view(np.float64).reshape(-1, 8).copy()).to(device)
             d = torch.from_numpy(self.datasets.view(np.uint8).reshape(-1, 32).copy()).to(device)
             self._dev[key] = (d, g)
+        return self._dev[key]
+
+    def points_device(self, device=None):
+        """The point list as a device tensor (16-byte phf_point records, viewed as int64 pairs)."""
+        torch = _lib.require_cuda()
+        device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+        key = "points:" + str(device)
+        if key not in self._dev:
+            self._dev[key] = torch.from_numpy(self.points.view(np.int64).reshape(-1, 2).copy()).to(device)
         return self._dev[key]
 
     def dataset_cost(self, model=2):
