@@ -411,6 +411,30 @@ int phf_psis_loo(int32_t n_cols, const int64_t *col_offsets /* HOST */, const do
                  void *stream);
 
 /* ------------------------------------------------------------------------------------------------
+ * Error bars of thermodynamic integration (the reference has none), as defined by pyhillfit_b200/ti.py
+ * (ti_errors_host, chain_series_stats).
+ *
+ * Temperature-1 log-likelihood (pi_bit included: what loglik_t1 and phf_log_target_batch mean by it) of every row of a
+ * chain-major samples buffer [n_chains][n_rows_total][d+1] (what the single-level samplers write; d = 2 for model 1,
+ * 3 for model 2).  One thread per (chain, row): row r >= row_begin of chain c goes to out[c * out_stride + (r -
+ * row_begin)], with the bits phf_log_target_batch gives for the same theta.
+ *   dataset_id  DEVICE, [n_chains]: the dataset of each chain
+ *   out         DEVICE; out_stride >= n_rows_total - row_begin
+ * Arguments are checked before any CUDA call (PHF_EINVAL).  Asynchronous on `stream`; allocates nothing. */
+int phf_single_rows_loglik(int model, int64_t n_chains, int64_t n_rows_total, int64_t row_begin, const double *samples,
+                           const int32_t *dataset_id, const phf_dataset *datasets, const phf_dose_group *groups,
+                           double *out, int64_t out_stride, void *stream);
+
+/* Per-chain statistics of n_chains series of n_rows >= 2 values: chain c is series[c * row_stride .. + n_rows).
+ *   scale  DEVICE, [n_chains]
+ *   out    DEVICE, [n_chains][4]: mean (x0 + mean(x - x0)), sample variance (ddof 1), log mean exp(scale_c x) (shifted by
+ *          the largest scale_c x), and the count of non-finite values; any non-finite value makes the first three NaN.
+ * Arguments are checked before any CUDA call (PHF_EINVAL).  Asynchronous on `stream`; allocates nothing.  Deterministic:
+ * one CTA per chain, fixed-order sums, the same bits on every call. */
+int phf_chain_series_stats(int64_t n_chains, int64_t n_rows, const double *series, int64_t row_stride,
+                           const double *scale, double *out, void *stream);
+
+/* ------------------------------------------------------------------------------------------------
  * Utilities
  * ---------------------------------------------------------------------------------------------- */
 int phf_version(void);

@@ -54,7 +54,7 @@ EXPORTS = ["phf_log_target_batch", "phf_am_single_init", "phf_am_single_run", "p
            "phf_write_rows_text_host",
            "phf_hier_predictive_cdfs", "phf_format_e18", "phf_format_e18_mismatches", "phf_version", "phf_last_error",
            "phf_fp64_peak_probe", "phf_launch_count", "phf_chain_diagnostics", "phf_am_single_swap",
-           "phf_single_pointwise_loglik", "phf_psis_loo"]
+           "phf_single_pointwise_loglik", "phf_psis_loo", "phf_single_rows_loglik", "phf_chain_series_stats"]
 
 _lib = None
 _p = C.c_void_p
@@ -112,6 +112,8 @@ def load():
     L.phf_chain_diagnostics.argtypes = [C.c_int64, C.c_int64, C.c_int64, C.c_int32, _p, C.c_int32, _p, C.c_int64, _p, _p]
     L.phf_single_pointwise_loglik.argtypes = [C.c_int, C.c_int64, C.c_int64, _p, C.c_int32, _p, _p, _p, _p, _p, _p]
     L.phf_psis_loo.argtypes = [C.c_int32, _p, _p, _p, _p]
+    L.phf_single_rows_loglik.argtypes = [C.c_int, C.c_int64, C.c_int64, C.c_int64, _p, _p, _p, _p, _p, C.c_int64, _p]
+    L.phf_chain_series_stats.argtypes = [C.c_int64, C.c_int64, _p, C.c_int64, _p, _p, _p]
     L.phf_format_e18.argtypes = [C.c_double, C.c_char_p]
     L.phf_format_e18_mismatches.argtypes = [_p, C.c_int64]
     L.phf_format_e18_mismatches.restype = C.c_int64

@@ -85,6 +85,34 @@ def save_bayes_factor(drug, channel, Bij, bf_dir="BFs/"):
     return bf_file
 
 
+def save_bayes_factor_errors(drug, channel, temps, errors, pair, n_chains, n_rows, swap_every, bf_dir="BFs/"):
+    """BFs/<drug>_<channel>_B12_errors.txt beside the B12 file: the error bars of pair `pair` of `errors` (run_ti's
+    errors dict: errors[m] of ti.ti_errors for models 1 and 2, and errors["ln_B12_se"]).  `#` header lines (ladder and
+    chain counts; per model TI, MCSE_TI, TI_corr, SS and the three se_rep; ln B12 +- se), then one row per (model, rung)
+    that np.loadtxt reads: model t E sd ess mcse rhat lags log_r (log_r NaN on the top rung)."""
+    if not os.path.exists(bf_dir):
+        os.makedirs(bf_dir)
+    f = bf_dir + "{}_{}_B12_errors.txt".format(drug, channel)
+    e1, e2 = errors[1], errors[2]
+    with open(f, "w") as out:
+        out.write("# error bars of the thermodynamic-integration Bayes factor, {} + {}\n".format(drug, channel))
+        out.write("# T = {} temperatures, R = {} chains per temperature, n = {} post-burn rows per chain, "
+                  "swap_every = {}\n".format(len(temps), n_chains, n_rows, swap_every))
+        for m, e in ((1, e1), (2, e2)):
+            out.write("# model {}: TI {:.18e} MCSE_TI {:.18e} TI_corr {:.18e} SS {:.18e} se_rep_TI {:.18e} "
+                      "se_rep_TI_corr {:.18e} se_rep_SS {:.18e}\n".format(
+                          m, e["TI"][pair], e["mcse_TI"][pair], e["TI_corr"][pair], e["SS"][pair], e["se_rep_TI"][pair],
+                          e["se_rep_TI_corr"][pair], e["se_rep_SS"][pair]))
+        out.write("# ln B12 {:.18e} +- {:.18e}\n".format(e1["TI"][pair] - e2["TI"][pair], errors["ln_B12_se"][pair]))
+        out.write("# model t E sd ess mcse rhat lags log_r\n")
+        for m, e in ((1, e1), (2, e2)):
+            for k, t in enumerate(temps):
+                out.write("{:d} {:.18e} {:.18e} {:.18e} {:.18e} {:.18e} {:.18e} {:d} {:.18e}\n".format(
+                    m, t, e["E"][pair, k], e["sd"][pair, k], e["ess"][pair, k], e["mcse"][pair, k], e["rhat"][pair, k],
+                    int(e["lags"][pair, k]), e["log_r"][pair, k]))
+    return f
+
+
 def extra_chain_name(chain_file, k):
     """File for replicate chain k > 0 of the same target (the reference runs one chain; chain 0 keeps its name)."""
     root, ext = os.path.splitext(chain_file)
