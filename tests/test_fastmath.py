@@ -1,50 +1,28 @@
 """Accuracy of the fp64 math layer the kernels use (pyhillfit_b200/csrc/phf_fastmath.cuh), measured on its host
 build (tests/native/fastmath_host.cpp, same source; only the MUFU seed instructions are emulated) against mpmath.
-The bound that matters is the log-target parity bound (1e-12 relative); each function is held to a few ulp."""
-import ctypes as C
+The bound that matters is the log-target parity bound (1e-12 relative); each function is held to a few ulp.
+tests/test_gpu_fastmath.py holds the device build to the same bounds on the same arguments."""
 import os
-import subprocess
 
 import mpmath as mp
 import numpy as np
 import pytest
 
+import _fastmath_cases as fc
+from _fastmath_cases import call, exact, ulps
+
 HERE = os.path.dirname(os.path.abspath(__file__))
-SRC = os.path.join(HERE, "native", "fastmath_host.cpp")
-LIB = os.path.join(HERE, "native", "libfastmath_host.so")
 
 
 @pytest.fixture(scope="module")
 def L():
-    hdr = os.path.join(HERE, "..", "pyhillfit_b200", "csrc", "phf_fastmath.cuh")
-    inc = os.path.join(HERE, "..", "pyhillfit_b200", "csrc", "phf_fastmath_coeffs.inc")
-    newest = max(os.path.getmtime(p) for p in (SRC, hdr, inc))
-    if not os.path.exists(LIB) or os.path.getmtime(LIB) < newest:
-        subprocess.check_call(["g++", "-O2", "-std=c++17", "-ffp-contract=off", "-shared", "-fPIC", "-o", LIB, SRC])
-    return C.CDLL(LIB)
-
-
-def call(L, name, x):
-    x = np.ascontiguousarray(x, dtype=np.float64)
-    y = np.empty_like(x)
-    getattr(L, name)(C.c_int(len(x)), x.ctypes.data_as(C.c_void_p), y.ctypes.data_as(C.c_void_p))
-    return y
-
-
-def exact(f, x):
-    mp.mp.dps = 40
-    return np.array([float(f(mp.mpf(float(v)))) for v in x])
-
-
-def ulps(got, want):
-    return np.max(np.abs(got - want) / np.spacing(np.abs(want)))
+    return fc.host_lib()
 
 
 def test_exp(L):
-    rng = np.random.default_rng(0)
-    x = np.concatenate([rng.uniform(-700, 700, 4000), rng.uniform(-1, 1, 4000), [0.0, -0.0, 1e-300]])
+    x = fc.exp_args()
     assert ulps(call(L, "fmh_exp", x), exact(mp.exp, x)) <= 2
-    sat = call(L, "fmh_exp", np.array([-1e9, -np.inf, 1e9, np.inf]))
+    sat = call(L, "fmh_exp", fc.EXP_SATURATING)
     assert np.all(sat[:2] == sat[0]) and 0 < sat[0] < 1e-300 and np.all(sat[2:] == sat[2]) and 1e300 < sat[2] < np.inf
 
 
@@ -52,22 +30,18 @@ def test_log(L):
     """Table-driven log: <= 2 ulp wherever |log x| >= 2^-7 and inside the table's central interval (which contains 1
     and returns r + r^2 P(r) with r = x - 1 exact); in between, log c_j and log1p(r) cancel and what is bounded is the
     ABSOLUTE error (1.5e-18) -- every caller adds the result to O(1) terms or takes sqrt(-2 log u)."""
-    rng = np.random.default_rng(1)
-    x = np.concatenate([np.exp(rng.uniform(-700, 700, 4000)), rng.uniform(0.5, 2, 4000), rng.uniform(0.99, 1.01, 4000),
-                        [1.0, 2.0 ** -54, 0.5, np.nextafter(1.0, 0), np.nextafter(1.0, 2)]])
+    x = fc.log_args()
     got, want = call(L, "fmh_log", x), exact(mp.log, x)
     err = np.abs(got - want)
-    far = np.abs(want) >= 2.0 ** -7
-    central = (x > 0.9962) & (x < 1.00015)
+    far, central = fc.log_bands(x, want)
     assert np.max(err[far] / np.spacing(np.abs(want[far]))) <= 2
     assert np.max(err[central] / np.maximum(np.spacing(np.abs(want[central])), 5e-324)) <= 2
-    assert np.max(err[~far]) <= 1.5e-18
+    assert np.max(err[~far]) <= fc.LOG_ABS_BOUND
     assert call(L, "fmh_log", np.array([1.0]))[0] == 0.0
 
 
 def test_rcp_rsqrt_sqrt(L):
-    rng = np.random.default_rng(2)
-    x = np.exp(rng.uniform(-600, 600, 8000))
+    x = fc.root_args()
     assert ulps(call(L, "fmh_rcp", x), 1.0 / x) <= 1
     assert ulps(call(L, "fmh_rsqrt", x), exact(lambda v: 1 / mp.sqrt(v), x)) <= 2
     assert ulps(call(L, "fmh_sqrt", x), np.sqrt(x)) <= 2
@@ -76,36 +50,27 @@ def test_rcp_rsqrt_sqrt(L):
 
 @pytest.mark.parametrize("suffix", ["", "_pw"])   # the one-polynomial form and the table-driven (piecewise) one
 def test_erfcx_and_log_ndtr(L, suffix):
-    rng = np.random.default_rng(3)
-    t = np.concatenate([rng.uniform(0, 10, 4000), np.exp(rng.uniform(np.log(1e-8), np.log(1e6), 3000)), [0.0]])
-    got, want = call(L, "fmh_erfcx" + suffix, t), exact(lambda v: mp.exp(v * v) * mp.erfc(v), t)
+    t, z = fc.erfcx_and_log_ndtr_args()
+    got, want = call(L, "fmh_erfcx" + suffix, t), exact(fc.erfcx_mp, t)
     assert np.max(np.abs(got - want) / want) <= 2e-15
-    z = -np.concatenate([rng.uniform(0, 40, 4000), np.exp(rng.uniform(np.log(1e-8), np.log(1e5), 2000)), [0.0]])
-    got, want = call(L, "fmh_log_ndtr" + suffix, z), exact(lambda v: mp.log(mp.ncdf(v)), z)
+    got, want = call(L, "fmh_log_ndtr" + suffix, z), exact(fc.log_ndtr_mp, z)
     assert np.max(np.abs(got - want) / np.maximum(1.0, np.abs(want))) <= 3e-15
 
 
 def test_exp10(L):
-    x = np.random.default_rng(4).uniform(-300, 300, 4000)
+    x = fc.exp10_args()
     assert ulps(call(L, "fmh_exp10", x), exact(lambda v: mp.power(10, v), x)) <= 3
 
 
 def test_sincos_of_a_32_bit_turn(L):
-    rng = np.random.default_rng(5)
-    b = rng.integers(0, 2 ** 32, 6000, dtype=np.uint64).astype(np.uint32)
-    b[:8] = [0, 1, 2 ** 29, 2 ** 30, 2 ** 31, 2 ** 32 - 1, 2 ** 29 - 1, 3 * 2 ** 30]
-    s, c = np.empty(len(b)), np.empty(len(b))
-    L.fmh_sincos(C.c_int(len(b)), b.ctypes.data_as(C.c_void_p), s.ctypes.data_as(C.c_void_p),
-                 c.ctypes.data_as(C.c_void_p))
+    b = fc.sincos_args()
+    s, c = fc.sincos(L, "fmh_sincos", b)
     mp.mp.dps = 40
     ws = np.array([float(mp.sin(2 * mp.pi * int(v) / 2 ** 32)) for v in b])
     wc = np.array([float(mp.cos(2 * mp.pi * int(v) / 2 ** 32)) for v in b])
     assert np.max(np.abs(s - ws)) <= 3e-16 and np.max(np.abs(c - wc)) <= 3e-16
     # exact antisymmetry under half a turn: the proposal distribution is exactly symmetric
-    b2 = (b.astype(np.uint64) + 2 ** 31).astype(np.uint32)
-    s2, c2 = np.empty(len(b)), np.empty(len(b))
-    L.fmh_sincos(C.c_int(len(b)), b2.ctypes.data_as(C.c_void_p), s2.ctypes.data_as(C.c_void_p),
-                 c2.ctypes.data_as(C.c_void_p))
+    s2, c2 = fc.sincos(L, "fmh_sincos", fc.half_turn(b))
     assert np.array_equal(s2, -s) and np.array_equal(c2, -c)
 
 
@@ -113,26 +78,18 @@ def test_table_driven_functions_at_the_edges(L):
     """Interval boundaries of the lookup tables, the ends of the domains, and out-of-domain arguments (which the
     samplers do produce -- a proposal with a negative sigma is evaluated before it is rejected -- and which must
     come back as some finite-or-NaN number without reading outside the table)."""
-    # log: every table interval's first and last double, the smallest / largest normal numbers
-    hi = (0x3fe6a09e + np.arange(129, dtype=np.int64) * 8192) << 32
-    edges = np.concatenate([hi.view(np.float64), np.nextafter(hi.view(np.float64), 0), [2.0 ** -1022, 1.7e308]])
+    edges = fc.log_edges()
     got, want = call(L, "fmh_log", edges), exact(mp.log, edges)
     far = np.abs(want) >= 2.0 ** -7
     assert np.max(np.abs(got - want)[far] / np.spacing(np.abs(want[far]))) <= 2
-    assert np.max(np.abs(got - want)[~far]) <= 1.5e-18
-    # exp: multiples of ln2/64 (interval boundaries of the reduction) and the clamp
-    k = np.arange(-64000, 64001, 997)
-    x = np.concatenate([k * (np.log(2) / 64), (k + 0.5) * (np.log(2) / 64), [700.0, -700.0, 699.999, -699.999]])
+    assert np.max(np.abs(got - want)[~far]) <= fc.LOG_ABS_BOUND
+    x = fc.exp_edges()
     assert ulps(call(L, "fmh_exp", x), exact(mp.exp, x)) <= 2
-    # erfcx (both forms): boundaries of the 32 intervals of q = (t - 4)/(t + 4), t = 0, large t
-    q = -1 + np.arange(1, 32) / 16.0
-    t = np.concatenate([4 * (1 + q) / (1 - q), [0.0, 1e3, 7.1e4, 1e10]])
-    t = np.concatenate([t, np.nextafter(t, 0), np.nextafter(t, np.inf)])
-    t = t[t >= 0]
-    want = exact(lambda v: mp.exp(v * v) * mp.erfc(v), t)
+    t = fc.erfcx_edges()
+    want = exact(fc.erfcx_mp, t)
     for name in ("fmh_erfcx", "fmh_erfcx_pw"):
         assert np.max(np.abs(call(L, name, t) - want) / want) <= 2e-15
-    bad = call(L, "fmh_erfcx_pw", np.array([-1.0, -4.0, -1e300, np.nan, np.inf]))
+    bad = call(L, "fmh_erfcx_pw", fc.ERFCX_PW_OUT_OF_DOMAIN)
     assert bad.shape == (5,)            # no crash, whatever the values
 
 
