@@ -94,19 +94,15 @@ extern "C" int phf_hier_predictive_cdfs(int64_t n_rows, const double *rows, int3
     if (chunks > max_chunks) chunks = (int)max_chunks;
     const int64_t per = ((n_rows + chunks - 1) / chunks + kCdfTile - 1) / kCdfTile * kCdfTile;
     chunks = (int)((n_rows + per - 1) / per);
+    StreamTemp tmp(s);
     double *partial = nullptr;
-    cudaError_t e = cudaMallocAsync(&partial, (size_t)chunks * 4 * n_x * sizeof(double), s);
-    if (e != cudaSuccess) return set_cuda_error(e, "cudaMallocAsync(cdf partial sums)");
+    if (int rc = tmp.alloc("cudaMallocAsync(cdf partial sums)", slice(partial, (size_t)chunks * 4 * n_x))) return rc;
     predictive_cdf_partial_kernel<<<dim3(gx, chunks), block, 0, s>>>(
         n_rows, rows, row_stride, n_x, hill_min, (hill_max - hill_min) / (n_x - 1), pic50_min,
         (pic50_max - pic50_min) / (n_x - 1), per, partial);
     count_launch();
-    int rc = check_launch("predictive_cdf_partial_kernel");
-    if (rc == PHF_OK) {
-        predictive_cdf_reduce_kernel<<<(4 * n_x + 255) / 256, 256, 0, s>>>(chunks, n_x, n_rows, partial, out);
-        count_launch();
-        rc = check_launch("predictive_cdf_reduce_kernel");
-    }
-    cudaFreeAsync(partial, s);
-    return rc;
+    if (int rc = check_launch("predictive_cdf_partial_kernel")) return rc;
+    predictive_cdf_reduce_kernel<<<(4 * n_x + 255) / 256, 256, 0, s>>>(chunks, n_x, n_rows, partial, out);
+    count_launch();
+    return check_launch("predictive_cdf_reduce_kernel");
 }

@@ -1,7 +1,9 @@
-// Error reporting / launch bookkeeping shared by the translation units of libphf_b200.so.
+// Error reporting, launch bookkeeping and host-side launch helpers shared by the translation units of libphf_b200.so.
 #pragma once
+#include <cstddef>
 #include <cstdint>
 #include <cuda_runtime.h>
+#include <type_traits>
 
 #include "../../include/pyhillfit_b200.h"
 
@@ -12,6 +14,83 @@ int set_cuda_error(cudaError_t e, const char *what);
 int check_launch(const char *kernel_name);  // cudaGetLastError() -> PHF_OK / PHF_ECUDA
 void count_launch();
 int sm_count();
+
+// Calls f(std::integral_constant<int, 1>{}) or f(std::integral_constant<int, 2>{}), so that a launch templated on the
+// single-level model is written once.  Picks the instantiation only: each entry point checks `model` first.
+template <typename F>
+void with_model(int model, F &&f)
+{
+    if (model == 1)
+        f(std::integral_constant<int, 1>{});
+    else
+        f(std::integral_constant<int, 2>{});
+}
+
+// Raises a kernel's dynamic shared memory limit when a launch needs more than 40 KB of it: the 48 KB default also
+// counts the kernel's static shared memory.  PHF_OK or PHF_ECUDA with `what` in the error text.
+template <typename Kernel>
+int allow_dynamic_smem(Kernel kern, size_t smem, const char *what = "cudaFuncSetAttribute")
+{
+    cudaError_t e;
+    if (smem > 40 * 1024 && (e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)))
+        return set_cuda_error(e, what);
+    return PHF_OK;
+}
+
+// The device temporaries of one call in stream-ordered memory.  alloc() carves every slice out of one cudaMallocAsync
+// on the call's stream (each slice rounded up to 256 bytes); the destructor hands the block back with cudaFreeAsync
+// on the same stream, behind the work queued there, on every return path.
+class StreamTemp {
+  public:
+    template <typename T>
+    struct Slice {
+        T **p;
+        size_t n;   // elements
+    };
+
+    explicit StreamTemp(cudaStream_t s) : s_(s) {}
+    ~StreamTemp()
+    {
+        if (base_) cudaFreeAsync(base_, s_);
+    }
+    StreamTemp(const StreamTemp &) = delete;
+    StreamTemp &operator=(const StreamTemp &) = delete;
+
+    // points every slice at its part of one allocation; PHF_OK or PHF_ECUDA with `what` in the error text
+    template <typename... T>
+    int alloc(const char *what, Slice<T>... slices)
+    {
+        cudaError_t e = cudaMallocAsync(&base_, (padded(slices.n * sizeof(T)) + ...), s_);
+        if (e != cudaSuccess) {
+            base_ = nullptr;
+            return set_cuda_error(e, what);
+        }
+        size_t off = 0;
+        ((*slices.p = reinterpret_cast<T *>(base_ + off), off += padded(slices.n * sizeof(T))), ...);
+        return PHF_OK;
+    }
+
+    // copies a host table of n elements into a slice, in stream order (a pageable source has been read when this
+    // returns); PHF_OK or PHF_ECUDA with `what` in the error text
+    template <typename T>
+    int upload(T *dst, const T *src, size_t n, const char *what) const
+    {
+        const cudaError_t e = cudaMemcpyAsync(dst, src, n * sizeof(T), cudaMemcpyHostToDevice, s_);
+        return e == cudaSuccess ? PHF_OK : set_cuda_error(e, what);
+    }
+
+  private:
+    static size_t padded(size_t bytes) { return (bytes + 255) / 256 * 256; }
+    cudaStream_t s_;
+    char *base_ = nullptr;
+};
+
+// one slice of StreamTemp::alloc: n elements, whose address goes to p
+template <typename T>
+StreamTemp::Slice<T> slice(T *&p, size_t n)
+{
+    return {&p, n};
+}
 
 // CTA size for the sampler kernels (`n_threads` = chains x lanes).  Tiny launches use 32-thread CTAs so that every
 // warp gets an SM to itself; up to ~16 warps per SM 64-thread CTAs (measured 4 % faster than 32 or 128 when the

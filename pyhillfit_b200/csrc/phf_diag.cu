@@ -294,61 +294,45 @@ extern "C" int phf_chain_diagnostics(int64_t n_chains, int64_t n_rows_total, int
     std::vector<int32_t> active_chains((size_t)n_chains), group_active((size_t)n_groups, 1);
     for (int64_t j = 0; j < n_chains; ++j) active_chains[(size_t)j] = (int32_t)j;
 
-    auto up = [](size_t b) { return (b + 255) / 256 * 256; };
-    const size_t b_means = up((size_t)n_chains * 2 * n_cols * sizeof(double));
-    const size_t b_partial = up((size_t)n_chains * splits * n_cols * kDiagLags * sizeof(double));
-    const size_t b_state = up((size_t)n_groups * n_cols * sizeof(DiagCol));
-    const size_t b_off = up((size_t)(n_groups + 1) * sizeof(int64_t));
-    const size_t b_list = up((size_t)n_chains * sizeof(int32_t));
-    const size_t b_act = up((size_t)n_groups * sizeof(int32_t));
-    char *tmp = nullptr;
-    cudaError_t e = cudaMallocAsync(&tmp, b_means + b_partial + b_state + b_off + b_list + b_act, s);
-    if (e != cudaSuccess) return set_cuda_error(e, "cudaMallocAsync(diagnostics temporaries)");
-    double *means = (double *)tmp;
-    double *partial = (double *)(tmp + b_means);
-    DiagCol *state = (DiagCol *)(tmp + b_means + b_partial);
-    int64_t *d_off = (int64_t *)(tmp + b_means + b_partial + b_state);
-    int32_t *d_list = (int32_t *)(tmp + b_means + b_partial + b_state + b_off);
-    int32_t *d_act = (int32_t *)(tmp + b_means + b_partial + b_state + b_off + b_list);
-
-    int rc = PHF_OK;
-    // (pageable sources: each copy has taken its bytes when it returns)
-    if ((e = cudaMemcpyAsync(d_off, group_offsets, (n_groups + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, s)) != cudaSuccess ||
-        (e = cudaMemcpyAsync(d_act, group_active.data(), n_groups * sizeof(int32_t), cudaMemcpyHostToDevice, s)) != cudaSuccess)
-        rc = set_cuda_error(e, "cudaMemcpyAsync(diagnostics groups)");
-    if (rc == PHF_OK) {
-        diag_means_kernel<<<dim3((unsigned)n_chains, ncb), kDiagThreads, 0, s>>>(n_rows_total, row_begin, n, n_cols,
-                                                                               samples, means);
-        count_launch();
-        rc = check_launch("diag_means_kernel");
-    }
+    StreamTemp tmp(s);
+    double *means = nullptr, *partial = nullptr;
+    DiagCol *state = nullptr;
+    int64_t *d_off = nullptr;
+    int32_t *d_list = nullptr, *d_act = nullptr;
+    if (int rc = tmp.alloc("cudaMallocAsync(diagnostics temporaries)", slice(means, (size_t)n_chains * 2 * n_cols),
+                           slice(partial, (size_t)n_chains * splits * n_cols * kDiagLags),
+                           slice(state, (size_t)n_groups * n_cols), slice(d_off, (size_t)n_groups + 1),
+                           slice(d_list, (size_t)n_chains), slice(d_act, (size_t)n_groups)))
+        return rc;
+    if (int rc = tmp.upload(d_off, group_offsets, (size_t)n_groups + 1, "cudaMemcpyAsync(diagnostics groups)"))
+        return rc;
+    if (int rc = tmp.upload(d_act, group_active.data(), (size_t)n_groups, "cudaMemcpyAsync(diagnostics groups)"))
+        return rc;
+    diag_means_kernel<<<dim3((unsigned)n_chains, ncb), kDiagThreads, 0, s>>>(n_rows_total, row_begin, n, n_cols,
+                                                                           samples, means);
+    count_launch();
+    if (int rc = check_launch("diag_means_kernel")) return rc;
     int64_t n_active = n_chains;
-    for (int64_t lag0 = 0; rc == PHF_OK; lag0 += kDiagLags) {
-        if ((e = cudaMemcpyAsync(d_list, active_chains.data(), n_active * sizeof(int32_t), cudaMemcpyHostToDevice, s)) !=
-            cudaSuccess) {
-            rc = set_cuda_error(e, "cudaMemcpyAsync(diagnostics active chains)");
-            break;
-        }
+    for (int64_t lag0 = 0;; lag0 += kDiagLags) {
+        if (int rc = tmp.upload(d_list, active_chains.data(), (size_t)n_active,
+                                "cudaMemcpyAsync(diagnostics active chains)"))
+            return rc;
         diag_lag_kernel<<<dim3((unsigned)(n_active * splits), ncb), kDiagThreads, 0, s>>>(
             n_rows_total, row_begin, n, n_cols, samples, means, d_list, (int32_t)splits, chunks_per_split, lag0, partial);
         count_launch();
-        if ((rc = check_launch("diag_lag_kernel")) != PHF_OK) break;
+        if (int rc = check_launch("diag_lag_kernel")) return rc;
         diag_group_kernel<<<n_groups, kDiagThreads, 0, s>>>(n, n_cols, d_off, means, partial, (int32_t)splits, lag0,
                                                             lag_limit, state, d_act, out);
         count_launch();
-        if ((rc = check_launch("diag_group_kernel")) != PHF_OK) break;
-        if ((e = cudaMemcpyAsync(group_active.data(), d_act, n_groups * sizeof(int32_t), cudaMemcpyDeviceToHost, s)) !=
-                cudaSuccess ||
-            (e = cudaStreamSynchronize(s)) != cudaSuccess) {
-            rc = set_cuda_error(e, "diagnostics: reading the active groups");
-            break;
-        }
+        if (int rc = check_launch("diag_group_kernel")) return rc;
+        cudaError_t e;
+        if ((e = cudaMemcpyAsync(group_active.data(), d_act, n_groups * sizeof(int32_t), cudaMemcpyDeviceToHost, s)) ||
+            (e = cudaStreamSynchronize(s)))
+            return set_cuda_error(e, "diagnostics: reading the active groups");
         n_active = 0;   // the next lag block runs on the chains of the groups still active only
         for (int32_t g = 0; g < n_groups; ++g)
             if (group_active[(size_t)g])
                 for (int64_t j = group_offsets[g]; j < group_offsets[g + 1]; ++j) active_chains[(size_t)n_active++] = (int32_t)j;
-        if (n_active == 0) break;
+        if (n_active == 0) return PHF_OK;
     }
-    cudaFreeAsync(tmp, s);
-    return rc;
 }

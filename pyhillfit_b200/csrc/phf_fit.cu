@@ -191,10 +191,10 @@ extern "C" int phf_best_fit_batch(int model, int64_t n_datasets, const int64_t *
     const int block = 64;
     const unsigned grid = (unsigned)((n_datasets + block - 1) / block);
     cudaStream_t s = (cudaStream_t)stream;
-    if (model == 1)
-        best_fit_kernel<1><<<grid, block, 0, s>>>(n_datasets, offsets, concs, responses, pic50_lower, 4000, theta, ss);
-    else
-        best_fit_kernel<2><<<grid, block, 0, s>>>(n_datasets, offsets, concs, responses, pic50_lower, 8000, theta, ss);
+    with_model(model, [&](auto m) {
+        best_fit_kernel<m><<<grid, block, 0, s>>>(n_datasets, offsets, concs, responses, pic50_lower,
+                                                  m == 1 ? 4000 : 8000, theta, ss);
+    });
     count_launch();
     return check_launch("best_fit_kernel");
 }

@@ -184,15 +184,16 @@ static int validate_hier_pack(int64_t n, int32_t n_expts, int32_t theta_stride, 
                               const phf_hier_dataset *datasets, const phf_hier_point *points, cudaStream_t s,
                               const char *who)
 {
+    StreamTemp tmp(s);
     int *d_flag = nullptr, h_flag = 0;
+    if (int rc = tmp.alloc("cudaMallocAsync", slice(d_flag, 1))) return rc;
     cudaError_t e;
-    if ((e = cudaMallocAsync(&d_flag, sizeof(int), s))) return set_cuda_error(e, "cudaMallocAsync");
     if ((e = cudaMemsetAsync(d_flag, 0, sizeof(int), s))) return set_cuda_error(e, "cudaMemsetAsync");
     hier_validate_kernel<<<(unsigned)((n + 127) / 128), 128, 0, s>>>(n, n_expts, theta_stride, dataset_id, datasets, points,
                                                                      d_flag);
     count_launch();
     if (int rc = check_launch("hier_validate_kernel")) return rc;
-    if ((e = cudaMemcpyAsync(&h_flag, d_flag, sizeof(int), cudaMemcpyDeviceToHost, s)) || (e = cudaFreeAsync(d_flag, s)) ||
+    if ((e = cudaMemcpyAsync(&h_flag, d_flag, sizeof(int), cudaMemcpyDeviceToHost, s)) ||
         (e = cudaStreamSynchronize(s)))
         return set_cuda_error(e, who);
     if (h_flag & 1) return set_error(PHF_EINVAL, "hierarchical pack: a chain's dataset does not have the launch's number of experiments / does not fit theta_stride");

@@ -11,13 +11,6 @@ namespace phf {
 
 constexpr int kBigDimMax = 5 + 2 * PHF_HIER_BIG_MAX_EXPTS;
 
-PHF_DI double warp_sum(double v)
-{
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    return v;
-}
-
 // log_target_distribution (PyHillFit.py:173-193) of the theta in shared memory `th`; all 32 lanes call it, the
 // result is uniform across the warp.
 PHF_DI double hier_big_log_target(const double *T, const double *th, int dim, int n_expts,
@@ -72,7 +65,7 @@ PHF_DI double hier_big_log_target(const double *T, const double *th, int dim, in
         ln_ic50(th[4 + 2 * e], lic_hi, lic_lo);
         term -= hier_point_nll(T, v.x, v.y, v.z, lic_hi, lic_lo, th[5 + 2 * e], inv2s2, inv_s_rt2, sigma_l);
     }
-    const double total = warp_sum(term);
+    const double total = group_sum<32>(term, 0xffffffffu);
     return bad ? -CUDART_INF : total;
 }
 
@@ -194,7 +187,7 @@ __global__ void __launch_bounds__(32) am_hier_big_kernel(phf_am_config cfg, int3
             }
             // (column k of the factor starts at offset k d - k (k-1)/2, i.e. advances by d - k)
             const double diag = cov[rm(j, j)];
-            const double piv = guarded_pivot(diag - warp_sum(part), diag);
+            const double piv = guarded_pivot(diag - group_sum<32>(part, 0xffffffffu), diag);
             const double rinv = fm::rsqrt(piv);
             if (lane == 0) L[cm(j, j, dim)] = piv * rinv;
             for (int i = j + 1 + lane; i < dim; i += 32) {
@@ -281,16 +274,14 @@ int am_hier_big_launch(const phf_am_config &cfg, int32_t n_expts, int64_t n, dou
                        double *samples, cudaStream_t s)
 {
     const int dim = 5 + 2 * n_expts;
-    const size_t bytes = (size_t)n * (size_t)(dim * (dim + 1) / 2) * sizeof(double);
+    StreamTemp tmp(s);
     double *scratch = nullptr;
-    cudaError_t e = cudaMallocAsync(&scratch, bytes, s);  // stream-ordered temporary: nothing persists
-    if (e != cudaSuccess) return set_cuda_error(e, "cudaMallocAsync(Cholesky scratch)");
+    if (int rc = tmp.alloc("cudaMallocAsync(Cholesky scratch)", slice(scratch, (size_t)n * (dim * (dim + 1) / 2))))
+        return rc;
     am_hier_big_kernel<<<(unsigned)n, 32, 0, s>>>(cfg, n_expts, n, state, dataset_id, datasets, points, pr, samples,
                                                   scratch);
     count_launch();
-    const int rc = check_launch("am_hier_big_kernel");
-    cudaFreeAsync(scratch, s);
-    return rc;
+    return check_launch("am_hier_big_kernel");
 }
 
 }  // namespace phf

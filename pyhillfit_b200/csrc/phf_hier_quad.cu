@@ -395,9 +395,7 @@ static int launch_am_hier_quad(const phf_am_config &cfg, int64_t n, double *stat
     if (block % 32 != 0 || block > 128) return set_error(PHF_EINVAL, "cfg.block_threads must be a multiple of 32, at most 128");
     auto kern = am_hier_quad_kernel<NE, MINB>;
     const size_t smem = Cfg::kWarpDoubles * sizeof(double) * (size_t)(block / 32);
-    cudaError_t e;
-    if (smem > 40 * 1024 && (e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)))
-        return set_cuda_error(e, "cudaFuncSetAttribute");
+    if (int rc = allow_dynamic_smem(kern, smem)) return rc;
     const int64_t per_cta = block / 4;
     const unsigned grid = (unsigned)((n + per_cta - 1) / per_cta);
     kern<<<grid, block, smem, s>>>(cfg, n, state, dataset_id, datasets, points, pr, samples);

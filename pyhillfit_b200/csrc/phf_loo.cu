@@ -83,12 +83,7 @@ __global__ void __launch_bounds__(kLooPwThreads) loo_pointwise_kernel(int64_t n_
 {
     constexpr int D = SingleDims<MODEL>::D;
     PHF_STAGE_FASTMATH_TABLE(T);
-    int lo = 0, hi = n_groups - 1;   // the group of this CTA: the last one whose first block is <= blockIdx.x
-    while (lo < hi) {
-        const int mid = (lo + hi + 1) / 2;
-        if (grp[mid].block_begin <= (int64_t)blockIdx.x) lo = mid; else hi = mid - 1;
-    }
-    const LooGroup G = grp[lo];
+    const LooGroup G = grp[last_at_or_below(grp, n_groups, &LooGroup::block_begin, (int64_t)blockIdx.x)];
     const int64_t s = ((int64_t)blockIdx.x - G.block_begin) * blockDim.x + threadIdx.x;
     if (s >= G.n_draws) return;
     const int64_t n_rows = n_rows_total - row_begin;
@@ -127,16 +122,6 @@ __global__ void __launch_bounds__(kLooPwThreads) loo_pointwise_kernel(int64_t n_
 // ------------------------------------------------------------------------------------------------
 // PSIS-LOO and WAIC (loo.py:psis_loo)
 // ------------------------------------------------------------------------------------------------
-__device__ __forceinline__ int find_column(const LooCol *cols, int32_t n_cols, int64_t chunk)
-{
-    int lo = 0, hi = n_cols - 1;
-    while (lo < hi) {
-        const int mid = (lo + hi + 1) / 2;
-        if (cols[mid].chunk_begin <= chunk) lo = mid; else hi = mid - 1;
-    }
-    return lo;
-}
-
 // order-preserving key of a double that is not NaN (-0 is folded into +0 first)
 __device__ __forceinline__ uint64_t order_key(double v)
 {
@@ -149,37 +134,13 @@ __device__ __forceinline__ double from_order_key(uint64_t k)
     return __longlong_as_double((long long)((k >> 63) ? (k & 0x7fffffffffffffffull) : ~k));
 }
 
-// fixed-tree reduction over the CTA (blockDim.x a power of two); every thread gets the result
-template <typename Op>
-__device__ double block_reduce(double v, double *buf, Op op)
-{
-    __syncthreads();
-    buf[threadIdx.x] = v;
-    __syncthreads();
-    for (int h = blockDim.x / 2; h > 0; h >>= 1) {
-        if ((int)threadIdx.x < h) buf[threadIdx.x] = op(buf[threadIdx.x], buf[threadIdx.x + h]);
-        __syncthreads();
-    }
-    return buf[0];
-}
-
-struct AddOp {
-    __device__ double operator()(double a, double b) const { return a + b; }
-};
-struct MaxOp {   // NaN-propagating
-    __device__ double operator()(double a, double b) const { return (a > b || a != a) ? a : b; }
-};
-struct MinOp {
-    __device__ double operator()(double a, double b) const { return (a < b || a != a) ? a : b; }
-};
-
 __global__ void __launch_bounds__(kLooThreads) loo_stats_kernel(int32_t n_cols, const LooCol *__restrict__ cols,
                                                                 const double *__restrict__ loglik,
                                                                 LooStats *__restrict__ part)
 {
     __shared__ double buf[kLooThreads];
     const int64_t chunk = blockIdx.x;
-    const LooCol C = cols[find_column(cols, n_cols, chunk)];
+    const LooCol C = cols[last_at_or_below(cols, n_cols, &LooCol::chunk_begin, chunk)];
     const int64_t i0 = (chunk - C.chunk_begin) * kLooChunk, i1 = min(i0 + kLooChunk, C.n);
     const double *l = loglik + C.begin;
     double mx = -CUDART_INF, mn = CUDART_INF, sum = 0.0, bad = 0.0;
@@ -235,7 +196,7 @@ __global__ void __launch_bounds__(kLooThreads) loo_hist_kernel(int32_t n_cols, c
 {
     __shared__ uint32_t h[256];
     const int64_t chunk = blockIdx.x;
-    const int c = find_column(cols, n_cols, chunk);
+    const int c = last_at_or_below(cols, n_cols, &LooCol::chunk_begin, chunk);
     if (state[c].status != kLooActive) return;
     const LooCol C = cols[c];
     const uint64_t prefix = state[c].prefix;
@@ -288,7 +249,7 @@ __global__ void __launch_bounds__(kLooThreads) loo_sums_kernel(int32_t n_cols, c
 {
     __shared__ double buf[kLooThreads];
     const int64_t chunk = blockIdx.x;
-    const int c = find_column(cols, n_cols, chunk);
+    const int c = last_at_or_below(cols, n_cols, &LooCol::chunk_begin, chunk);
     const LooState st = state[c];
     if (st.status != kLooActive) return;
     const LooCol C = cols[c];
@@ -339,8 +300,7 @@ __device__ void gpdfit(const double *z, int L, double *buf, double *b_ary, doubl
         const double b = b_ary[j];
         double s = 0.0;
         for (int i = lane; i < L; i += 32) s += log1p(-b * z[i]);
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+        s = group_sum<32>(s, 0xffffffffu);
         if (lane == 0) {
             const double k = s / (double)L;
             len_ary[j] = (double)L * (log(-(b / k)) - k - 1.0);
@@ -513,25 +473,16 @@ extern "C" int phf_single_pointwise_loglik(int model, int64_t n_rows_total, int6
     if (blocks > 0x7fffffff) return set_error(PHF_ENOTSUP, "phf_single_pointwise_loglik: too many draws for one call");
     if (col == 0) return PHF_OK;
     cudaStream_t s = (cudaStream_t)stream;
+    StreamTemp tmp(s);
     LooGroup *d_tab = nullptr;
-    cudaError_t e = cudaMallocAsync(&d_tab, tab.size() * sizeof(LooGroup), s);
-    if (e != cudaSuccess) return set_cuda_error(e, "cudaMallocAsync(pointwise groups)");
-    int rc = PHF_OK;
-    // (pageable source: the copy has taken its bytes when it returns)
-    if ((e = cudaMemcpyAsync(d_tab, tab.data(), tab.size() * sizeof(LooGroup), cudaMemcpyHostToDevice, s)) != cudaSuccess)
-        rc = set_cuda_error(e, "cudaMemcpyAsync(pointwise groups)");
-    if (rc == PHF_OK) {
-        if (model == 1)
-            loo_pointwise_kernel<1><<<(unsigned)blocks, kLooPwThreads, 0, s>>>(n_rows_total, row_begin, samples, n_groups,
-                                                                                d_tab, points, groups, loglik);
-        else
-            loo_pointwise_kernel<2><<<(unsigned)blocks, kLooPwThreads, 0, s>>>(n_rows_total, row_begin, samples, n_groups,
-                                                                                d_tab, points, groups, loglik);
-        count_launch();
-        rc = check_launch("loo_pointwise_kernel");
-    }
-    cudaFreeAsync(d_tab, s);
-    return rc;
+    if (int rc = tmp.alloc("cudaMallocAsync(pointwise groups)", slice(d_tab, tab.size()))) return rc;
+    if (int rc = tmp.upload(d_tab, tab.data(), tab.size(), "cudaMemcpyAsync(pointwise groups)")) return rc;
+    with_model(model, [&](auto m) {
+        loo_pointwise_kernel<m><<<(unsigned)blocks, kLooPwThreads, 0, s>>>(n_rows_total, row_begin, samples, n_groups,
+                                                                            d_tab, points, groups, loglik);
+    });
+    count_launch();
+    return check_launch("loo_pointwise_kernel");
 }
 
 extern "C" int phf_psis_loo(int32_t n_cols, const int64_t *col_offsets, const double *loglik, double *out, void *stream)
@@ -560,61 +511,43 @@ extern "C" int phf_psis_loo(int32_t n_cols, const int64_t *col_offsets, const do
     int tail_pow2 = 1;
     while (tail_pow2 < m_max) tail_pow2 <<= 1;
     const size_t smem = (size_t)tail_pow2 * sizeof(double);
-    cudaError_t e = cudaFuncSetAttribute(loo_finish_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return set_cuda_error(e, "cudaFuncSetAttribute(loo_finish_kernel)");
+    if (int rc = allow_dynamic_smem(loo_finish_kernel, smem, "cudaFuncSetAttribute(loo_finish_kernel)")) return rc;
 
     cudaStream_t s = (cudaStream_t)stream;
-    auto up = [](size_t b) { return (b + 255) / 256 * 256; };
-    const size_t b_cols = up(cols.size() * sizeof(LooCol));
-    const size_t b_state = up((size_t)n_cols * sizeof(LooState));
-    const size_t b_stats = up((size_t)chunks * sizeof(LooStats));
-    const size_t b_sums = up((size_t)chunks * sizeof(LooSums));
-    const size_t b_hist = up((size_t)n_cols * 256 * sizeof(uint32_t));
-    const size_t b_tail = up((size_t)tail_total * sizeof(double));
-    char *tmp = nullptr;
-    e = cudaMallocAsync(&tmp, b_cols + b_state + b_stats + b_sums + b_hist + b_tail, s);
-    if (e != cudaSuccess) return set_cuda_error(e, "cudaMallocAsync(PSIS temporaries)");
-    LooCol *d_cols = (LooCol *)tmp;
-    LooState *d_state = (LooState *)(tmp + b_cols);
-    LooStats *d_stats = (LooStats *)(tmp + b_cols + b_state);
-    LooSums *d_sums = (LooSums *)(tmp + b_cols + b_state + b_stats);
-    uint32_t *d_hist = (uint32_t *)(tmp + b_cols + b_state + b_stats + b_sums);
-    double *d_tail = (double *)(tmp + b_cols + b_state + b_stats + b_sums + b_hist);
-
-    int rc = PHF_OK;
-    if ((e = cudaMemcpyAsync(d_cols, cols.data(), cols.size() * sizeof(LooCol), cudaMemcpyHostToDevice, s)) != cudaSuccess ||
-        (e = cudaMemsetAsync(d_hist, 0, (size_t)n_cols * 256 * sizeof(uint32_t), s)) != cudaSuccess)
-        rc = set_cuda_error(e, "cudaMemcpyAsync(PSIS columns)");
+    StreamTemp tmp(s);
+    LooCol *d_cols = nullptr;
+    LooState *d_state = nullptr;
+    LooStats *d_stats = nullptr;
+    LooSums *d_sums = nullptr;
+    uint32_t *d_hist = nullptr;
+    double *d_tail = nullptr;
+    if (int rc = tmp.alloc("cudaMallocAsync(PSIS temporaries)", slice(d_cols, cols.size()), slice(d_state, n_cols),
+                           slice(d_stats, chunks), slice(d_sums, chunks), slice(d_hist, (size_t)n_cols * 256),
+                           slice(d_tail, tail_total)))
+        return rc;
+    if (int rc = tmp.upload(d_cols, cols.data(), cols.size(), "cudaMemcpyAsync(PSIS columns)")) return rc;
+    if (cudaError_t e = cudaMemsetAsync(d_hist, 0, (size_t)n_cols * 256 * sizeof(uint32_t), s))
+        return set_cuda_error(e, "cudaMemcpyAsync(PSIS columns)");
     const unsigned col_blocks = (unsigned)((n_cols + 127) / 128);
-    if (rc == PHF_OK) {
-        loo_stats_kernel<<<(unsigned)chunks, kLooThreads, 0, s>>>(n_cols, d_cols, loglik, d_stats);
-        count_launch();
-        rc = check_launch("loo_stats_kernel");
-    }
-    if (rc == PHF_OK) {
-        loo_begin_kernel<<<col_blocks, 128, 0, s>>>(n_cols, d_cols, d_stats, d_state);
-        count_launch();
-        rc = check_launch("loo_begin_kernel");
-    }
-    for (int shift = 56; shift >= 0 && rc == PHF_OK; shift -= 8) {
+    loo_stats_kernel<<<(unsigned)chunks, kLooThreads, 0, s>>>(n_cols, d_cols, loglik, d_stats);
+    count_launch();
+    if (int rc = check_launch("loo_stats_kernel")) return rc;
+    loo_begin_kernel<<<col_blocks, 128, 0, s>>>(n_cols, d_cols, d_stats, d_state);
+    count_launch();
+    if (int rc = check_launch("loo_begin_kernel")) return rc;
+    for (int shift = 56; shift >= 0; shift -= 8) {
         loo_hist_kernel<<<(unsigned)chunks, kLooThreads, 0, s>>>(n_cols, d_cols, loglik, d_state, shift, d_hist);
         count_launch();
-        if ((rc = check_launch("loo_hist_kernel")) != PHF_OK) break;
+        if (int rc = check_launch("loo_hist_kernel")) return rc;
         loo_select_kernel<<<col_blocks, 128, 0, s>>>(n_cols, d_state, shift, d_hist);
         count_launch();
-        rc = check_launch("loo_select_kernel");
+        if (int rc = check_launch("loo_select_kernel")) return rc;
     }
-    if (rc == PHF_OK) {
-        loo_sums_kernel<<<(unsigned)chunks, kLooThreads, 0, s>>>(n_cols, d_cols, loglik, d_state, d_sums, d_tail);
-        count_launch();
-        rc = check_launch("loo_sums_kernel");
-    }
-    if (rc == PHF_OK) {
-        loo_finish_kernel<<<(unsigned)n_cols, kLooFinishThreads, smem, s>>>(n_cols, d_cols, d_state, d_sums, d_tail,
-                                                                            tail_pow2, out);
-        count_launch();
-        rc = check_launch("loo_finish_kernel");
-    }
-    cudaFreeAsync(tmp, s);
-    return rc;
+    loo_sums_kernel<<<(unsigned)chunks, kLooThreads, 0, s>>>(n_cols, d_cols, loglik, d_state, d_sums, d_tail);
+    count_launch();
+    if (int rc = check_launch("loo_sums_kernel")) return rc;
+    loo_finish_kernel<<<(unsigned)n_cols, kLooFinishThreads, smem, s>>>(n_cols, d_cols, d_state, d_sums, d_tail,
+                                                                        tail_pow2, out);
+    count_launch();
+    return check_launch("loo_finish_kernel");
 }

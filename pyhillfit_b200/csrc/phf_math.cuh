@@ -73,6 +73,45 @@ PHF_DI double group_sum(double v, unsigned mask)
     return v;
 }
 
+// ---- CTA-wide reduction ----
+// fixed-tree reduction over the CTA (blockDim.x a power of two, `buf` one double per thread): the order of the
+// operations depends on blockDim.x alone; every thread gets the result
+template <typename Op>
+__device__ double block_reduce(double v, double *buf, Op op)
+{
+    __syncthreads();
+    buf[threadIdx.x] = v;
+    __syncthreads();
+    for (int h = blockDim.x / 2; h > 0; h >>= 1) {
+        if ((int)threadIdx.x < h) buf[threadIdx.x] = op(buf[threadIdx.x], buf[threadIdx.x + h]);
+        __syncthreads();
+    }
+    return buf[0];
+}
+
+struct AddOp {
+    __device__ double operator()(double a, double b) const { return a + b; }
+};
+struct MaxOp {   // NaN-propagating
+    __device__ double operator()(double a, double b) const { return (a > b || a != a) ? a : b; }
+};
+struct MinOp {
+    __device__ double operator()(double a, double b) const { return (a < b || a != a) ? a : b; }
+};
+
+// segment lookup: of n >= 1 segments whose `first` members do not decrease, the last one with seg[i].*first <= key
+// (0 when there is none)
+template <typename Seg>
+PHF_DI int last_at_or_below(const Seg *seg, int n, int64_t Seg::*first, int64_t key)
+{
+    int lo = 0, hi = n - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) / 2;
+        if (seg[mid].*first <= key) lo = mid; else hi = mid - 1;
+    }
+    return lo;
+}
+
 // ---- Philox4x32-10 (Salmon et al. 2011); stream contract in oracle/hill_oracle.py ----
 struct Philox4 {
     uint32_t w[4];

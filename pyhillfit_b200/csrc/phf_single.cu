@@ -357,6 +357,7 @@ static int launch_am_single(const phf_am_config &cfg, int64_t n, int block, doub
     const size_t smem = (size_t)cfg.stage_groups * sizeof(phf_dose_group) +
                         (G > 1 ? (size_t)block * (D + 1) * sizeof(double) : 0) + (size_t)block * sizeof(double) +
                         (size_t)block * (4 / G) * 64;
+    if (smem > 200 * 1024) return set_error(PHF_EINVAL, "cfg.stage_groups needs more than 200 KB of shared memory");
     if (int rc = allow_dynamic_smem(kern, smem)) return rc;
     const int cta_chains = block / G;
     const unsigned grid = (unsigned)((n + cta_chains - 1) / cta_chains);
@@ -390,12 +391,10 @@ extern "C" int phf_log_target_batch(int model, int64_t n, const double *theta, c
     const int block = 128;
     const unsigned grid = (unsigned)((n + block - 1) / block);
     cudaStream_t s = (cudaStream_t)stream;
-    if (model == 1)
-        log_target_batch_kernel<1><<<grid, block, 0, s>>>(n, theta, dataset_id, temperature, datasets, groups,
+    with_model(model, [&](auto m) {
+        log_target_batch_kernel<m><<<grid, block, 0, s>>>(n, theta, dataset_id, temperature, datasets, groups,
                                                           log_target, loglik_t1);
-    else
-        log_target_batch_kernel<2><<<grid, block, 0, s>>>(n, theta, dataset_id, temperature, datasets, groups,
-                                                          log_target, loglik_t1);
+    });
     count_launch();
     return check_launch("log_target_batch_kernel");
 }
@@ -412,12 +411,10 @@ extern "C" int phf_am_single_init(int model, int64_t n_chains, const double *the
     const int block = 128;
     const unsigned grid = (unsigned)((n_chains + block - 1) / block);
     cudaStream_t s = (cudaStream_t)stream;
-    if (model == 1)
-        am_single_init_kernel<1><<<grid, block, 0, s>>>(n_chains, theta0, cov0_tri, dataset_id, temperature,
-                                                        datasets, groups, state);
-    else
-        am_single_init_kernel<2><<<grid, block, 0, s>>>(n_chains, theta0, cov0_tri, dataset_id, temperature,
-                                                        datasets, groups, state);
+    with_model(model, [&](auto m) {
+        am_single_init_kernel<m><<<grid, block, 0, s>>>(n_chains, theta0, cov0_tri, dataset_id, temperature, datasets,
+                                                        groups, state);
+    });
     count_launch();
     return check_launch("am_single_init_kernel");
 }

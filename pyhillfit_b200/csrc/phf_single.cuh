@@ -323,18 +323,6 @@ PHF_DI void adapt_update(double *mean, double *cov, double &loga, const double *
     loga = fma(gam, acc_minus_quarter, loga);
 }
 
-// Host side of a sampler launch with `smem` bytes of dynamic shared memory: at most 200 KB, and above 40 KB the kernel's
-// limit is raised (the 48 KB default counts the kernel's static shared memory too).
-template <typename Kernel>
-static int allow_dynamic_smem(Kernel kern, size_t smem)
-{
-    if (smem > 200 * 1024) return set_error(PHF_EINVAL, "cfg.stage_groups needs more than 200 KB of shared memory");
-    cudaError_t e;
-    if (smem > 40 * 1024 && (e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)))
-        return set_cuda_error(e, "cudaFuncSetAttribute");
-    return PHF_OK;
-}
-
 // proposal theta* = theta + e^{loga/2} chol(cov) z  (N(theta, e^loga cov): PyHillFit.py:831, PyHillTemp.py:88), guarded
 // pivots (phf_math.cuh); cov = lower triangle, row-major
 template <int MODEL>

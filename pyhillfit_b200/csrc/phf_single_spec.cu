@@ -248,6 +248,7 @@ static int launch_spec(const phf_am_config &cfg, int64_t n, int block, double *s
     const int cta_chains = block / G;
     const size_t smem = (size_t)cfg.stage_groups * sizeof(phf_dose_group) +
                         (size_t)cta_chains * (2 * G) * (D + 2) * sizeof(double) + (size_t)block * (4 / E) * 64;
+    if (smem > 200 * 1024) return set_error(PHF_EINVAL, "cfg.stage_groups needs more than 200 KB of shared memory");
     if (int rc = allow_dynamic_smem(kern, smem)) return rc;
     const unsigned grid = (unsigned)((n + cta_chains - 1) / cta_chains);
     kern<<<grid, block, smem, s>>>(cfg, n, state, dataset_id, temperature, datasets, groups, samples);

@@ -87,14 +87,11 @@ extern "C" int phf_am_single_swap(int model, int64_t n_chains, double *state, co
     const int block = 128;
     const unsigned grid = (unsigned)((n_pairs + block - 1) / block);
     cudaStream_t s = (cudaStream_t)stream;
-    if (model == 1)
-        am_single_swap_kernel<1><<<grid, block, 0, s>>>(n_pairs, pairs_per_ladder, n_chains, state, dataset_id,
+    with_model(model, [&](auto m) {
+        am_single_swap_kernel<m><<<grid, block, 0, s>>>(n_pairs, pairs_per_ladder, n_chains, state, dataset_id,
                                                         temperature, datasets, groups, ladder_len, ladder_chains, seed,
                                                         ladder_id_base, t, parity, swap_counts);
-    else
-        am_single_swap_kernel<2><<<grid, block, 0, s>>>(n_pairs, pairs_per_ladder, n_chains, state, dataset_id,
-                                                        temperature, datasets, groups, ladder_len, ladder_chains, seed,
-                                                        ladder_id_base, t, parity, swap_counts);
+    });
     count_launch();
     return check_launch("am_single_swap_kernel");
 }

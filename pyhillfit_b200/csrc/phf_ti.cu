@@ -45,23 +45,6 @@ __global__ void __launch_bounds__(kTiRowsThreads) ti_rows_loglik_kernel(int64_t 
     out[c * out_stride + r] = l1;
 }
 
-// fixed-tree sum / max over the CTA (blockDim.x = kTiStatsThreads); every thread gets the result
-template <bool MAX>
-__device__ double ti_block_reduce(double v, double *buf)
-{
-    __syncthreads();
-    buf[threadIdx.x] = v;
-    __syncthreads();
-    for (int h = kTiStatsThreads / 2; h > 0; h >>= 1) {
-        if ((int)threadIdx.x < h) {
-            const double a = buf[threadIdx.x], b = buf[threadIdx.x + h];
-            buf[threadIdx.x] = MAX ? fmax(a, b) : a + b;
-        }
-        __syncthreads();
-    }
-    return buf[0];
-}
-
 __global__ void __launch_bounds__(kTiStatsThreads) ti_series_stats_kernel(int64_t n_rows,
                                                                           const double *__restrict__ series,
                                                                           int64_t row_stride,
@@ -83,9 +66,9 @@ __global__ void __launch_bounds__(kTiStatsThreads) ti_series_stats_kernel(int64_
             bad += 1.0;
         }
     }
-    sum = ti_block_reduce<false>(sum, buf);
-    mx = ti_block_reduce<true>(mx, buf);
-    bad = ti_block_reduce<false>(bad, buf);
+    sum = block_reduce(sum, buf, AddOp());
+    mx = block_reduce(mx, buf, MaxOp());   // finite values and -inf only: the bits fmax would give
+    bad = block_reduce(bad, buf, AddOp());
     double* o = out + c * 4;
     if (bad > 0.0) {
         if (threadIdx.x == 0) {
@@ -101,8 +84,8 @@ __global__ void __launch_bounds__(kTiStatsThreads) ti_series_stats_kernel(int64_
         sq = fma(d, d, sq);
         se += exp(s * v - mx);
     }
-    sq = ti_block_reduce<false>(sq, buf);
-    se = ti_block_reduce<false>(se, buf);
+    sq = block_reduce(sq, buf, AddOp());
+    se = block_reduce(se, buf, AddOp());
     if (threadIdx.x == 0) {
         o[0] = mean;
         o[1] = sq / (double)(n_rows - 1);
@@ -134,14 +117,11 @@ extern "C" int phf_single_rows_loglik(int model, int64_t n_chains, int64_t n_row
     const int64_t blocks = (n_chains * n_rows + kTiRowsThreads - 1) / kTiRowsThreads;
     if (blocks > 0x7fffffff) return set_error(PHF_ENOTSUP, "phf_single_rows_loglik: too many rows for one call");
     cudaStream_t s = (cudaStream_t)stream;
-    if (model == 1)
-        ti_rows_loglik_kernel<1><<<(unsigned)blocks, kTiRowsThreads, 0, s>>>(n_chains, n_rows_total, row_begin, samples,
+    with_model(model, [&](auto m) {
+        ti_rows_loglik_kernel<m><<<(unsigned)blocks, kTiRowsThreads, 0, s>>>(n_chains, n_rows_total, row_begin, samples,
                                                                               dataset_id, datasets, groups, out,
                                                                               out_stride);
-    else
-        ti_rows_loglik_kernel<2><<<(unsigned)blocks, kTiRowsThreads, 0, s>>>(n_chains, n_rows_total, row_begin, samples,
-                                                                              dataset_id, datasets, groups, out,
-                                                                              out_stride);
+    });
     count_launch();
     return check_launch("ti_rows_loglik_kernel");
 }
