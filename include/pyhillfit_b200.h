@@ -435,6 +435,53 @@ int phf_chain_series_stats(int64_t n_chains, int64_t n_rows, const double *serie
                            const double *scale, double *out, void *stream);
 
 /* ------------------------------------------------------------------------------------------------
+ * Posterior-predictive checks (the reference has none), as defined by pyhillfit_b200/ppc.py (ppc_host, bands_host).
+ * Draws, groups and points as phf_single_pointwise_loglik takes them.  One measurement is z ~ N(p, sigma^2) with p the
+ * Hill curve at its dose, replicated as y_rep = min(max(z, 0), 100): a response of exactly 0 or 100 is the censored
+ * value.  Points of kind 3 are not modelled: NaN, and left out of every dataset statistic.
+ *
+ * Replicates: the normal of point k (0-based within its group, kind 3 points counted) of draw (chain c of the buffer,
+ * absolute row r) is box_muller of words 0 and 1 of philox_call(seed, chain_id_base + c, r, PHF_PPC_CALL0 + k/2), z0
+ * for even k and z1 for odd k.  Samplers use small call indices and swaps PHF_SWAP_CALL0 + k, so the streams are
+ * disjoint; a replicate depends on (seed, global chain, row, point) alone, not on batching or row_begin.
+ *
+ * phf_single_ppc, averaged over the S_g draws of each group:
+ *   point_out  DEVICE, [n_points][3] (n_points = point_offsets[n_groups] - point_offsets[0]):
+ *              pit_lo = mean P(y_rep < y), pit_hi = mean P(y_rep <= y), mean_rep = mean E[y_rep]
+ *   group_out  DEVICE, [n_groups][8], with D(y, theta) = -2 sum_i log p(y_i | theta) over the modelled points (the
+ *              pointwise log-likelihood without -ln(2 pi) / 2) and n_cens = #{y_i in {0, 100}}:
+ *              mean D(y), mean D(y_rep), p_D = #{D(y_rep) >= D(y)} / S, n_cens(y), #{n_cens(y_rep) >= n_cens(y)} / S,
+ *              #{n_cens(y_rep) <= n_cens(y)} / S, modelled points, draws with a non-finite D(y) (sigma <= 1e-3; when
+ *              not 0, columns 0-2, 4 and 5 are NaN)
+ * Takes a stream-ordered temporary of 24 bytes per (point, 512 draws) and 48 bytes per 512 draws (580 MB for 2 585
+ * points x 4 800 064 draws).
+ *
+ * phf_single_predictive_bands, per group and grid dose (grid: phf_dose_group records of which lnc_hi, lnc_lo and conc
+ * are read; pyhillfit_b200/packing.py:ln_hi_lo gives a grid dose equal to a data dose the sampler's bits), from
+ * K = min(S_g, max_draws) draws, draw j = floor(j S_g / K) in (chain, row) order:
+ *   out  DEVICE, [n_groups][n_x][2][n_q]: np.quantile (method 'linear') of the K curve values at each level q, then the
+ *        predictive quantile Q(q) = min{y in [0, 100] : F(y) >= q}, F(y) = (1/K) sum_j Phi((y - p_j) / sigma_j) for
+ *        y < 100, F(100) = 1 (the censored mixture, atoms at 0 and 100 included): 0 when F(0) >= q, otherwise the upper
+ *        end of 50 bisection steps on [0, 100] that keep F(lo) < q <= F(hi).
+ * Levels must lie in (0, 1), 1 <= n_q <= 8, 1 <= max_draws <= PHF_PPC_MAX_BAND_DRAWS.  Takes a stream-ordered temporary
+ * of 24 bytes per group.
+ *
+ * Both check their arguments before any CUDA call (PHF_EINVAL), are asynchronous on `stream`, and are deterministic:
+ * partitions depend on the shapes alone, floating-point sums run in a fixed order, two calls give the same bits, and a
+ * group gives the same bits alone (its chains' sub-buffer, chain_id_base + its first chain) as within a larger call.
+ * ---------------------------------------------------------------------------------------------- */
+#define PHF_PPC_CALL0 0x40000000u
+#define PHF_PPC_MAX_BAND_DRAWS 8192 /* K: (p, 1/sigma) of K draws in shared memory, 128 KB */
+int phf_single_ppc(int model, int64_t n_rows_total, int64_t row_begin, const double *samples, int32_t n_groups,
+                   const int64_t *chain_offsets /* HOST */, const int64_t *point_offsets /* HOST */,
+                   const phf_point *points, const phf_dose_group *groups, uint64_t seed, uint64_t chain_id_base,
+                   double *point_out, double *group_out, void *stream);
+int phf_single_predictive_bands(int model, int64_t n_rows_total, int64_t row_begin, const double *samples,
+                                int32_t n_groups, const int64_t *chain_offsets /* HOST */, int32_t n_x,
+                                const phf_dose_group *grid /* DEVICE [n_groups][n_x] */, int32_t max_draws,
+                                int32_t n_q, const double *q /* HOST */, double *out, void *stream);
+
+/* ------------------------------------------------------------------------------------------------
  * Utilities
  * ---------------------------------------------------------------------------------------------- */
 int phf_version(void);

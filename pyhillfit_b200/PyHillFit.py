@@ -37,6 +37,10 @@ def build_parser():
     parser.add_argument("--loo", action='store_true', default=False,
                         help="single-level only: PSIS-LOO and WAIC per measurement from each pair's chains, computed on "
                              "the GPU, written beside the chain file as ..._loo.txt [new]")
+    parser.add_argument("--ppc", action='store_true', default=False,
+                        help="single-level only: posterior-predictive checks per measurement and per pair, and "
+                             "dose-response bands, computed on the GPU, written beside the chain file as ..._ppc.txt "
+                             "and ..._predictive_bands.txt [new]")
     requiredNamed = parser.add_argument_group('required arguments')
     requiredNamed.add_argument("--data-file", type=str, help="csv file from which to read in data, in same format as provided crumb_data.csv", required=True)
     requiredNamed.add_argument("-m", "--model", type=int, help="For non-hierarchical (put anything for hierarchical):1. fix Hill=1; 2. vary Hill", required=True)
@@ -57,7 +61,7 @@ def select_pairs(dr, args):
 def run_single_level(dr, args, pairs):
     """python/PyHillFit.py:645-867 for all pairs at once."""
     import torch
-    from . import chainio, ess, loo
+    from . import chainio, ess, loo, ppc
     from .initial_fit import best_fit_batch_gpu as best_fit_batch   # phf_best_fit_batch, one thread per dataset
     from .packing import SinglePack
     from .sampler import SingleLevelSampler, model_chain_id_base
@@ -108,6 +112,8 @@ def run_single_level(dr, args, pairs):
     print("\n{} chains x {} iterations in {:.2f} s on the GPU\n".format(s.n, args.iterations, time.time() - start))
     diag = ess.targets_diagnostics(chain, len(jobs), R, 0) if args.diagnostics else None
     loo_rows, loo_draws = loo.targets_loo(chain, pack, R, args.model) if args.loo else (None, 0)
+    checks = (ppc.targets_ppc(chain, pack, R, args.model, args.seed, model_chain_id_base(args.model), data)
+              if args.ppc else None)
     t_phase = time.time()
     host = chain.cpu().numpy().reshape(len(jobs), R, chain.shape[1], s.d + 1)
     print("chains to the host: {:.2f} s".format(time.time() - t_phase))
@@ -119,6 +125,12 @@ def run_single_level(dr, args, pairs):
         if loo_rows is not None:
             chainio.save_loo(job["chain_file"], loo_rows[j], data[j][0], data[j][1], args.model, job["drug"],
                              job["channel"], loo_draws)
+        if checks is not None:
+            per, grp, grids, bands, S = checks
+            chainio.save_ppc(job["chain_file"], per[j], grp[j], data[j][0], data[j][1], args.model, job["drug"],
+                             job["channel"], S, args.seed)
+            chainio.save_predictive_bands(job["chain_file"], grids[j], bands[j], ppc.DEFAULT_LEVELS, args.model,
+                                          job["drug"], job["channel"], S, ppc.DEFAULT_MAX_DRAWS)
         print("\n\n{} + {} complete!\n\n".format(job["drug"], job["channel"]))
     print("chain files: {:.2f} s".format(time.time() - t_phase))
     return jobs
@@ -226,6 +238,9 @@ def main(argv=None):
     args = parser.parse_args(argv)
     if args.loo and args.hierarchical:
         parser.error("--loo is for the single-level models (the hierarchical likelihood is a different one)")
+    if args.ppc and args.hierarchical:
+        parser.error("--ppc is for the single-level models (construct_hierarchical_cdfs covers the hierarchical "
+                     "predictive distributions)")
     t_import = time.time()
     from . import doseresponse as dr
     dr.define_model(args.model)

@@ -165,6 +165,55 @@ def save_loo(chain_file, rows, concs, responses, model, drug, channel, n_draws):
     return f
 
 
+def ppc_name(chain_file):
+    """File of the posterior-predictive check of one target's points (--ppc), beside its chain file."""
+    root, ext = os.path.splitext(chain_file)
+    return "{}_ppc{}".format(root, ext)
+
+
+def predictive_bands_name(chain_file):
+    """File of the dose-response bands of one target (--ppc), beside its chain file."""
+    root, ext = os.path.splitext(chain_file)
+    return "{}_predictive_bands{}".format(root, ext)
+
+
+def save_ppc(chain_file, points, group_row, concs, responses, model, drug, channel, n_draws, seed):
+    """`#` header lines (model, pair, draws, seed, the dataset row of ppc.GROUP_COLUMNS), then one row per point:
+    index dose response kind pit_lo pit_hi pit_mid p_two_sided mean_rep, NaN for a point of kind 3 (np.loadtxt reads
+    it)."""
+    from . import ppc
+    from .packing import masks, point_kinds
+    mid, p2 = ppc.derived(points)
+    kinds = point_kinds(*masks(responses))
+    f = ppc_name(chain_file)
+    with open(f, "w") as out:
+        out.write("# posterior-predictive check per point, model {}, {} + {}\n".format(model, drug, channel))
+        out.write("# S = {} draws (chains x rows), seed {}\n".format(n_draws, seed))
+        out.write("# dataset: " + " ".join("{} {:.18e}".format(n, v) for n, v in zip(ppc.GROUP_COLUMNS, group_row))
+                  + "\n")
+        out.write("# index dose response kind pit_lo pit_hi pit_mid p_two_sided mean_rep\n")
+        for i, (c, y, k, r, m, p) in enumerate(zip(concs, responses, kinds, points, mid, p2)):
+            out.write("{:d} {:.18e} {:.18e} {:d} {:.18e} {:.18e} {:.18e} {:.18e} {:.18e}\n".format(
+                i, c, y, int(k), r[0], r[1], m, p, r[2]))
+    return f
+
+
+def save_predictive_bands(chain_file, grid, bands, levels, model, drug, channel, n_draws, max_draws):
+    """`#` header lines (model, pair, draws, levels), then one row per grid dose: dose, the curve quantiles at each
+    level, the predictive quantiles at each level (bands [n_x, 2, m] of ppc.bands_host / bands_gpu)."""
+    f = predictive_bands_name(chain_file)
+    m = len(levels)
+    with open(f, "w") as out:
+        out.write("# dose-response bands, model {}, {} + {}\n".format(model, drug, channel))
+        out.write("# K = {} of S = {} draws (chains x rows), levels {}\n".format(
+            min(n_draws, max_draws), n_draws, " ".join("{:g}".format(q) for q in levels)))
+        out.write("# dose " + " ".join("curve_{:g}".format(q) for q in levels) + " "
+                  + " ".join("predictive_{:g}".format(q) for q in levels) + "\n")
+        for c, b in zip(grid, bands):
+            out.write(" ".join("{:.18e}".format(v) for v in [c] + list(b[0, :m]) + list(b[1, :m])) + "\n")
+    return f
+
+
 def swap_acceptance_name(chain_file):
     """File of the per-rung swap acceptance of one (drug, channel, model) ladder run (PyHillTemp --swap-every): in the
     model directory that holds the temperature_* directories, named after the chain file without its temperature."""
