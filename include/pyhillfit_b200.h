@@ -410,6 +410,26 @@ int phf_single_pointwise_loglik(int model, int64_t n_rows_total, int64_t row_beg
 int phf_psis_loo(int32_t n_cols, const int64_t *col_offsets /* HOST */, const double *loglik, double *out,
                  void *stream);
 
+/* Held-out term of exact leave-one-out refits (pyhillfit_b200/loo.py: heldout_estimate, refit_loo).  Fold f is chains
+ * chain_offsets[f] .. chain_offsets[f+1]-1 of a chain-major samples buffer [n_chains][n_rows_total][d+1], sampled on its
+ * dataset without the point heldout[f] (a phf_point of the FULL pack, whose dose group `groups` holds: a dose the
+ * reduced dataset no longer has still gets the sampler's bits).  Buffer row r of every chain is kept row row_begin + r
+ * of n_kept (rows below burn_rows neither written nor counted); kept row a is in slot 0 for a < n = n_kept / 2, slot 1
+ * for a >= n_kept - n, and slot 2 (the middle row of an odd n_kept) otherwise.  With l the held-out point's term of
+ * phf_single_pointwise_loglik (the same bits) at each row, this call merges into
+ *   acc  DEVICE, [n_chains][PHF_HELDOUT_SLOTS][4], indexed by the buffer's chain: per slot the max m of the finite l,
+ *        sum exp(l - m) over them, the number of rows, the number of non-finite l.  Start it at (-inf, 0, 0, 0); calls
+ *        over successive segments of the rows chain (the accumulator is merged first, then the segment).
+ * chain_offsets (strictly increasing, n_folds + 1 entries) and heldout (n_folds records) are HOST arrays.  Arguments are
+ * checked before any CUDA call (PHF_EINVAL).  Asynchronous on `stream`; takes a stream-ordered temporary of 24 bytes per
+ * fold.  Deterministic: one CTA per chain, fixed-order sums over a partition of the rows that depends on the shapes
+ * alone, no floating-point atomics: the same bits on every call. */
+#define PHF_HELDOUT_SLOTS 3
+int phf_single_heldout_loglik(int model, int64_t n_rows_total, int64_t row_begin, int64_t n_kept,
+                              const double *samples, int32_t n_folds, const int64_t *chain_offsets /* HOST */,
+                              const phf_point *heldout /* HOST */, const phf_dose_group *groups, double *acc,
+                              void *stream);
+
 /* ------------------------------------------------------------------------------------------------
  * Error bars of thermodynamic integration (the reference has none), as defined by pyhillfit_b200/ti.py
  * (ti_errors_host, chain_series_stats).

@@ -37,6 +37,10 @@ def build_parser():
     parser.add_argument("--loo", action='store_true', default=False,
                         help="single-level only: PSIS-LOO and WAIC per measurement from each pair's chains, computed on "
                              "the GPU, written beside the chain file as ..._loo.txt [new]")
+    parser.add_argument("--loo-refit", nargs="?", const="khat", choices=("khat", "all"), default=None,
+                        help="single-level only, implies --loo: exact leave-one-out by refitting each pair without the "
+                             "point, on the GPU, for the points whose PSIS khat is above the threshold ('khat', the "
+                             "default) or for every modelled point ('all'); two more columns in ..._loo.txt [new]")
     parser.add_argument("--ppc", action='store_true', default=False,
                         help="single-level only: posterior-predictive checks per measurement and per pair, and "
                              "dose-response bands, computed on the GPU, written beside the chain file as ..._ppc.txt "
@@ -64,7 +68,7 @@ def run_single_level(dr, args, pairs):
     from . import chainio, ess, loo, ppc
     from .initial_fit import best_fit_batch_gpu as best_fit_batch   # phf_best_fit_batch, one thread per dataset
     from .packing import SinglePack
-    from .sampler import SingleLevelSampler, model_chain_id_base
+    from .sampler import SingleLevelSampler, model_chain_id_base, replicate_jitter
     temperature = 1
     assert args.iterations % args.thinning == 0            # PyHillFit.py:805
     jobs, data = [], []
@@ -94,11 +98,9 @@ def run_single_level(dr, args, pairs):
     pack = SinglePack(data)
     ids = np.repeat(np.arange(len(jobs), dtype=np.int32), R)
     theta0 = np.repeat(np.stack([j["theta0"] for j in jobs]), R, axis=0)
-    if R > 1:   # replicate chains start from a 2 % jitter of the fit; chain 0 starts at the fit like the reference
-        rng = np.random.default_rng(args.seed)
-        jit = 1.0 + 0.02 * rng.standard_normal(theta0.shape)
-        jit[::R] = 1.0
-        theta0 = theta0 * jit
+    jitter = replicate_jitter(len(jobs), R, theta0.shape[1], args.seed)
+    if R > 1:
+        theta0 = theta0 * jitter
     saved_iterations = args.iterations // args.thinning + 1
     burn = saved_iterations // args.burn_in_fraction
     s = SingleLevelSampler(args.model, pack, ids, 1.0, theta0, variant="fit", seed=args.seed,
@@ -112,6 +114,8 @@ def run_single_level(dr, args, pairs):
     print("\n{} chains x {} iterations in {:.2f} s on the GPU\n".format(s.n, args.iterations, time.time() - start))
     diag = ess.targets_diagnostics(chain, len(jobs), R, 0) if args.diagnostics else None
     loo_rows, loo_draws = loo.targets_loo(chain, pack, R, args.model) if args.loo else (None, 0)
+    refits = (loo.targets_refit(loo_rows, data, loo_draws, args.loo_refit, args.model, R, args.iterations,
+                                args.thinning, burn, args.seed, jitter) if args.loo_refit else None)
     checks = (ppc.targets_ppc(chain, pack, R, args.model, args.seed, model_chain_id_base(args.model), data)
               if args.ppc else None)
     t_phase = time.time()
@@ -124,7 +128,7 @@ def run_single_level(dr, args, pairs):
                                    None if diag is None else diag[j], chainio.single_level_columns(args.model))
         if loo_rows is not None:
             chainio.save_loo(job["chain_file"], loo_rows[j], data[j][0], data[j][1], args.model, job["drug"],
-                             job["channel"], loo_draws)
+                             job["channel"], loo_draws, None if refits is None else refits[j], args.loo_refit)
         if checks is not None:
             per, grp, grids, bands, S = checks
             chainio.save_ppc(job["chain_file"], per[j], grp[j], data[j][0], data[j][1], args.model, job["drug"],
@@ -236,6 +240,9 @@ def main(argv=None):
         parser.print_help()
         return 1
     args = parser.parse_args(argv)
+    if args.loo_refit and args.hierarchical:
+        parser.error("--loo-refit is for the single-level models (a fold here is one point of one pair)")
+    args.loo = args.loo or bool(args.loo_refit)
     if args.loo and args.hierarchical:
         parser.error("--loo is for the single-level models (the hierarchical likelihood is a different one)")
     if args.ppc and args.hierarchical:

@@ -146,9 +146,13 @@ def loo_name(chain_file):
     return "{}_loo{}".format(root, ext)
 
 
-def save_loo(chain_file, rows, concs, responses, model, drug, channel, n_draws):
+def save_loo(chain_file, rows, concs, responses, model, drug, channel, n_draws, refit=None, refit_mode=None):
     """`#` header lines (model, pair, draws, khat threshold, totals of loo.summary), then one row per point:
-    index dose response elpd_loo_i lppd_i p_waic_i khat_i (np.loadtxt reads it)."""
+    index dose response elpd_loo_i lppd_i p_waic_i khat_i (np.loadtxt reads it).  With `refit` ([N, 2] of
+    loo.REFIT_COLUMNS, NaN where a point was not refitted; --loo-refit `refit_mode`), one more header line (the points
+    refitted, elpd_loo with the refits in place of PSIS where there is one) and two trailing columns
+    elpd_refit_i se_refit_i.  A point of kind 3 may carry its exact constant (-ln(2 pi) / 2, se 0) there; it is not
+    counted as refitted."""
     from . import loo
     s = loo.summary(rows, n_draws)
     f = loo_name(chain_file)
@@ -159,9 +163,22 @@ def save_loo(chain_file, rows, concs, responses, model, drug, channel, n_draws):
                   "{} of {} points with khat above the threshold\n".format(
                       s["elpd_loo"], s["se_elpd_loo"], s["p_loo"], s["elpd_waic"], s["se_elpd_waic"], s["p_waic"],
                       s["n_high_khat"], s["n"]))
-        out.write("# index dose response elpd_loo_i lppd_i p_waic_i khat_i\n")
-        for i, (c, y, r) in enumerate(zip(concs, responses, rows)):
-            out.write("{:d} {:.18e} {:.18e} {:.18e} {:.18e} {:.18e} {:.18e}\n".format(i, c, y, *r[:4]))
+        if refit is None:
+            out.write("# index dose response elpd_loo_i lppd_i p_waic_i khat_i\n")
+            for i, (c, y, r) in enumerate(zip(concs, responses, rows)):
+                out.write("{:d} {:.18e} {:.18e} {:.18e} {:.18e} {:.18e} {:.18e}\n".format(i, c, y, *r[:4]))
+            return f
+        from .packing import masks, point_kinds
+        refit = np.asarray(refit, dtype=np.float64).reshape(-1, 2)
+        done = np.isfinite(refit[:, 0])
+        e = np.where(done, refit[:, 0], np.asarray(rows)[:, 0])
+        fitted = int(np.count_nonzero(done & (point_kinds(*masks(responses)) != 3)))
+        out.write("# exact refits ({}): {} of {} points refitted; elpd_loo with refits {:.6f} +- {:.6f}\n".format(
+            refit_mode, fitted, len(e), e.sum(), np.sqrt(len(e) * np.var(e))))
+        out.write("# index dose response elpd_loo_i lppd_i p_waic_i khat_i elpd_refit_i se_refit_i\n")
+        for i, (c, y, r, x) in enumerate(zip(concs, responses, rows, refit)):
+            out.write("{:d} {:.18e} {:.18e} {:.18e} {:.18e} {:.18e} {:.18e} {:.18e} {:.18e}\n".format(
+                i, c, y, *r[:4], *x))
     return f
 
 

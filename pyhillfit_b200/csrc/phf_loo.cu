@@ -43,6 +43,7 @@ constexpr double kHalfLn2Pi = 0.9189385332046727;      // 0.5 ln(2 pi) (np.float
 constexpr double kLnDblMin = -708.3964185322641;       // ln DBL_MIN (np.log(np.finfo(float).tiny))
 
 enum { kLooActive = 0, kLooConstant = 1, kLooNonFinite = 2 };
+constexpr int kHeldoutSlots = PHF_HELDOUT_SLOTS;   // first half, second half, middle row of an odd N
 
 struct LooGroup {   // one group of phf_single_pointwise_loglik
     int64_t chain_begin, n_draws, point_begin, n_points, col_base, block_begin;
@@ -73,6 +74,48 @@ struct LooState {
 // ------------------------------------------------------------------------------------------------
 // pointwise log-likelihood (loo.py:pointwise_loglik)
 // ------------------------------------------------------------------------------------------------
+// The pointwise term of one draw: the draw's curve parameters once, then point_loglik per point.  Shared by the
+// pointwise kernel and the held-out kernel of the refits, so that a refit's held-out term has the bits of the column
+// PSIS reads.
+template <int MODEL>
+struct DrawCurve {
+    bool sigma_ok;   // sigma > 1e-3; otherwise every term is -inf (doseresponse.py:212-214, 238-240)
+    double inv_s, log_s, hill, lic_hi, lic_lo, inv_ic50;
+
+    __device__ __forceinline__ DrawCurve(const double *T, const double *th)
+    {
+        constexpr int D = SingleDims<MODEL>::D;
+        const double pic50 = th[0];
+        hill = MODEL == 2 ? th[1] : 1.0;
+        const double sigma = th[D - 1];
+        sigma_ok = sigma > kSigmaLower;
+        const double sg = sigma_ok ? sigma : 1.0;
+        inv_s = fm::rcp(sg);
+        log_s = fm::log_pos(T, sg);
+        lic_hi = 0.0, lic_lo = 0.0, inv_ic50 = 0.0;
+        if (MODEL == 2)
+            ln_ic50(pic50, lic_hi, lic_lo);
+        else
+            inv_ic50 = fm::exp10_clamped(T, pic50 - 6.0);
+    }
+
+    __device__ __forceinline__ double point_loglik(const double *T, const phf_point &P, const phf_dose_group &Gd) const
+    {
+        const double x = MODEL == 2 ? hill_ratio_pow(T, Gd.lnc_hi, Gd.lnc_lo, lic_hi, lic_lo, hill) : Gd.conc * inv_ic50;
+        const double p = hill_response(x);
+        double l = 0.0;   // kind 3 (in no mask): the -0.5 ln 2 pi of pi_bit alone
+        if (P.kind == 2) {
+            const double r = P.y - p;
+            l = fma(-r * r, 0.5 * inv_s * inv_s, -log_s);
+        } else if (P.kind == 0) {
+            l = fm::log_ndtr_nonpos(T, (0.0 - p) * inv_s);
+        } else if (P.kind == 1) {
+            l = fm::log_ndtr_nonpos(T, (p - 100.0) * inv_s);
+        }
+        return sigma_ok ? l - kHalfLn2Pi : -CUDART_INF;
+    }
+};
+
 template <int MODEL>
 __global__ void __launch_bounds__(kLooPwThreads) loo_pointwise_kernel(int64_t n_rows_total, int64_t row_begin,
                                                                       const double *__restrict__ samples, int32_t n_groups,
@@ -88,34 +131,11 @@ __global__ void __launch_bounds__(kLooPwThreads) loo_pointwise_kernel(int64_t n_
     if (s >= G.n_draws) return;
     const int64_t n_rows = n_rows_total - row_begin;
     const int64_t chain = G.chain_begin + s / n_rows, row = row_begin + s % n_rows;
-    const double *th = samples + (chain * n_rows_total + row) * (D + 1);
-    const double pic50 = th[0];
-    const double hill = MODEL == 2 ? th[1] : 1.0;
-    const double sigma = th[D - 1];
-    const bool sigma_ok = sigma > kSigmaLower;   // otherwise every term is -inf (doseresponse.py:212-214, 238-240)
-    const double sg = sigma_ok ? sigma : 1.0;
-    const double inv_s = fm::rcp(sg), log_s = fm::log_pos(T, sg);
-    double lic_hi = 0.0, lic_lo = 0.0, inv_ic50 = 0.0;
-    if (MODEL == 2)
-        ln_ic50(pic50, lic_hi, lic_lo);
-    else
-        inv_ic50 = fm::exp10_clamped(T, pic50 - 6.0);
+    const DrawCurve<MODEL> cur(T, samples + (chain * n_rows_total + row) * (D + 1));
     double *out = loglik + G.col_base + s;
     for (int64_t i = 0; i < G.n_points; ++i) {
         const phf_point P = points[G.point_begin + i];
-        const phf_dose_group &Gd = groups[P.group];
-        const double x = MODEL == 2 ? hill_ratio_pow(T, Gd.lnc_hi, Gd.lnc_lo, lic_hi, lic_lo, hill) : Gd.conc * inv_ic50;
-        const double p = hill_response(x);
-        double l = 0.0;   // kind 3 (in no mask): the -0.5 ln 2 pi of pi_bit alone
-        if (P.kind == 2) {
-            const double r = P.y - p;
-            l = fma(-r * r, 0.5 * inv_s * inv_s, -log_s);
-        } else if (P.kind == 0) {
-            l = fm::log_ndtr_nonpos(T, (0.0 - p) * inv_s);
-        } else if (P.kind == 1) {
-            l = fm::log_ndtr_nonpos(T, (p - 100.0) * inv_s);
-        }
-        out[i * G.n_draws] = sigma_ok ? l - kHalfLn2Pi : -CUDART_INF;
+        out[i * G.n_draws] = cur.point_loglik(T, P, groups[P.group]);
     }
 }
 
@@ -432,6 +452,72 @@ __global__ void __launch_bounds__(kLooFinishThreads) loo_finish_kernel(int32_t n
     }
 }
 
+// ------------------------------------------------------------------------------------------------
+// held-out term of exact leave-one-out refits (loo.py:heldout_estimate)
+// ------------------------------------------------------------------------------------------------
+// One CTA per chain; slot k (0: first half, 1: second half, 2: the middle row of an odd N) is the kept rows
+// [lo_k, hi_k).  Per slot, each thread keeps a running max and the sum of exp(l - max) over its rows of the segment in
+// row order; the CTA merges its threads' partials by a fixed tree (the max first, then the sums rescaled to it), and
+// thread 0 merges that into the caller's accumulator, accumulator first.
+struct HeldFold {
+    int64_t chain_begin;
+    phf_point P;
+};
+
+__device__ __forceinline__ void heldout_merge(double &m, double &s, double m2, double s2)
+{
+    const double mx = fmax(m, m2);
+    s = (s > 0.0 ? s * exp(m - mx) : 0.0) + (s2 > 0.0 ? s2 * exp(m2 - mx) : 0.0);
+    m = mx;
+}
+
+template <int MODEL>
+__global__ void __launch_bounds__(kLooThreads) loo_heldout_kernel(int64_t n_rows_total, int64_t row_begin,
+                                                                  int64_t n_kept, const double *__restrict__ samples,
+                                                                  int32_t n_folds, const HeldFold *__restrict__ folds,
+                                                                  const phf_dose_group *__restrict__ groups,
+                                                                  double *__restrict__ acc)
+{
+    constexpr int D = SingleDims<MODEL>::D;
+    __shared__ double buf[kLooThreads];
+    PHF_STAGE_FASTMATH_TABLE(T);
+    const int64_t chain = folds[0].chain_begin + blockIdx.x;
+    const phf_point P = folds[last_at_or_below(folds, n_folds, &HeldFold::chain_begin, chain)].P;
+    const phf_dose_group Gd = groups[P.group];
+    const double *rows = samples + (size_t)chain * n_rows_total * (D + 1);
+    double *out = acc + (size_t)chain * kHeldoutSlots * 4;
+    const int64_t half = n_kept / 2;
+#pragma unroll
+    for (int k = 0; k < kHeldoutSlots; ++k) {
+        const int64_t lo = k == 0 ? 0 : (k == 1 ? n_kept - half : half);
+        const int64_t hi = k == 0 ? half : (k == 1 ? n_kept : n_kept - half);
+        const int64_t r0 = max(lo, row_begin) - row_begin, r1 = min(hi, row_begin + n_rows_total) - row_begin;
+        double m = -CUDART_INF, sum = 0.0, bad = 0.0;
+        for (int64_t r = r0 + threadIdx.x; r < r1; r += blockDim.x) {
+            const double l = DrawCurve<MODEL>(T, rows + r * (D + 1)).point_loglik(T, P, Gd);
+            if (!isfinite(l)) {
+                bad += 1.0;
+            } else if (l > m) {
+                sum = fma(sum, exp(m - l), 1.0);
+                m = l;
+            } else {
+                sum += exp(l - m);
+            }
+        }
+        const double mx = block_reduce(m, buf, MaxOp());
+        const double s = block_reduce(sum > 0.0 ? sum * exp(m - mx) : 0.0, buf, AddOp());
+        bad = block_reduce(bad, buf, AddOp());
+        if (threadIdx.x == 0) {
+            double om = out[4 * k], os = out[4 * k + 1];
+            heldout_merge(om, os, mx, s);
+            out[4 * k] = om;
+            out[4 * k + 1] = os;
+            out[4 * k + 2] += (double)max(r1 - r0, (int64_t)0);
+            out[4 * k + 3] += bad;
+        }
+    }
+}
+
 }  // namespace phf
 
 using namespace phf;
@@ -550,4 +636,40 @@ extern "C" int phf_psis_loo(int32_t n_cols, const int64_t *col_offsets, const do
                                                                         tail_pow2, out);
     count_launch();
     return check_launch("loo_finish_kernel");
+}
+
+extern "C" int phf_single_heldout_loglik(int model, int64_t n_rows_total, int64_t row_begin, int64_t n_kept,
+                                         const double *samples, int32_t n_folds, const int64_t *chain_offsets,
+                                         const phf_point *heldout, const phf_dose_group *groups, double *acc,
+                                         void *stream)
+{
+    if (model != 1 && model != 2) return set_error(PHF_EINVAL, "phf_single_heldout_loglik: model must be 1 or 2");
+    if (n_rows_total <= 0 || n_folds <= 0)
+        return set_error(PHF_EINVAL, "phf_single_heldout_loglik: counts must be positive");
+    if (row_begin < 0 || n_kept < row_begin + n_rows_total)
+        return set_error(PHF_EINVAL, "phf_single_heldout_loglik: need 0 <= row_begin and row_begin + n_rows_total <= n_kept");
+    if (!samples || !chain_offsets || !heldout || !groups || !acc)
+        return set_error(PHF_EINVAL, "phf_single_heldout_loglik: NULL pointer");
+    if (chain_offsets[0] < 0) return set_error(PHF_EINVAL, "phf_single_heldout_loglik: offsets must start at >= 0");
+    for (int32_t f = 0; f < n_folds; ++f) {
+        if (chain_offsets[f + 1] <= chain_offsets[f])
+            return set_error(PHF_EINVAL, "phf_single_heldout_loglik: chain offsets must be strictly increasing");
+        if (heldout[f].kind < 0 || heldout[f].kind > 3 || heldout[f].group < 0)
+            return set_error(PHF_EINVAL, "phf_single_heldout_loglik: a held-out point needs kind 0..3 and a group >= 0");
+    }
+    const int64_t chains = chain_offsets[n_folds] - chain_offsets[0];
+    if (chains > 0x7fffffff) return set_error(PHF_ENOTSUP, "phf_single_heldout_loglik: too many chains for one call");
+    std::vector<HeldFold> tab((size_t)n_folds);
+    for (int32_t f = 0; f < n_folds; ++f) tab[(size_t)f] = HeldFold{chain_offsets[f], heldout[f]};
+    cudaStream_t s = (cudaStream_t)stream;
+    StreamTemp tmp(s);
+    HeldFold *d_tab = nullptr;
+    if (int rc = tmp.alloc("cudaMallocAsync(held-out folds)", slice(d_tab, tab.size()))) return rc;
+    if (int rc = tmp.upload(d_tab, tab.data(), tab.size(), "cudaMemcpyAsync(held-out folds)")) return rc;
+    with_model(model, [&](auto m) {
+        loo_heldout_kernel<m><<<(unsigned)chains, kLooThreads, 0, s>>>(n_rows_total, row_begin, n_kept, samples,
+                                                                        n_folds, d_tab, groups, acc);
+    });
+    count_launch();
+    return check_launch("loo_heldout_kernel");
 }

@@ -14,6 +14,23 @@ concatenates them, masks of :675-677), p = Hill curve at the point's dose:
 so that the sum over the points is exactly the reference's log_data_likelihood(..., t=1, pi_bit): pi_bit counts all N
 points, which gives censored and dropped points their -ln(2 pi) / 2.  That constant is the same in both models, so
 comparisons do not depend on it.  sigma <= 1e-3 gives -inf, as the reference's likelihood does.
+
+Exact leave-one-out by refitting (refit_loo; PyHillFit --loo-refit).  A fold is dataset g without one modelled point i
+(kind 0, 1 or 2); a kind-3 point has l_i = -ln(2 pi) / 2 at every theta, so its exact value is that constant with se 0
+and it is not refitted.  A refit is what PyHillFit does for one pair, on the reduced dataset: variant "fit", the run's
+iterations, thinning and burn rows (rows below burn_rows are neither written nor read), R chains.  Starts: chain 0 at
+phf_best_fit_batch's fit of the reduced data (of the full data when the reduced data has no modelled point: the refit
+then samples the prior), chain r at that fit times the jitter factors of chain r of dataset g in the main run
+(sampler.replicate_jitter).  Philox ids: chain r of the j-th refitted fold, in point order among the refitted folds,
+is model_chain_id_base(m) + REFIT_ID_OFFSET + j R + r, disjoint from the main run's model_chain_id_base(m) + g R + r.
+So the draws of a fold depend on which folds were selected (through j), but not on how the folds are split into
+launches or memory batches.  The held-out estimate of a fold from the S kept draws of its R chains (heldout_estimate):
+    elpd_refit_i = ln((1/S) sum_s exp l_i(theta_s))            (l_i as pointwise_loglik, comparable with elpd_loo_i)
+    se_refit_i   = sd(E_h, ddof 1) / sqrt(2R) / E
+with E the mean of exp l_i over all draws and E_h its mean over half-chain h: each chain's N kept rows split into
+[0, n) and [N - n, N), n = N // 2, as ess.chain_diagnostics splits them (the middle row of an odd N is in E only).
+Every mean is taken shifted by the largest l_i, so that l_i < -708 at every draw still gives the right value; a
+non-finite l_i at any draw gives NaN.
 """
 import time
 
@@ -21,12 +38,15 @@ import numpy as np
 from scipy.special import log_ndtr, logsumexp
 
 from . import _lib
-from .packing import masks, point_kinds, POINT_ZERO, POINT_HUNDRED, POINT_OTHER
+from .packing import masks, point_kinds, SinglePack, POINT_ZERO, POINT_HUNDRED, POINT_OTHER, POINT_NONE
 
 HALF_LN_2PI = 0.5 * np.log(2 * np.pi)
 LN_DBL_MIN = np.log(np.finfo(float).tiny)
 SIGMA_LOWER = 1e-3
 LOO_COLUMNS = ("elpd_loo_i", "lppd_i", "p_waic_i", "khat_i", "tail_len")
+REFIT_COLUMNS = ("elpd_refit_i", "se_refit_i")
+REFIT_ID_OFFSET = 1 << 39        # refit chain ids: model_chain_id_base(m) + REFIT_ID_OFFSET + j R + r
+HELDOUT_SLOTS = 3                # PHF_HELDOUT_SLOTS: first half, second half, middle row of each chain
 
 
 def pointwise_loglik(model, concs, responses, theta, where_0=None, where_100=None, where_other=None):
@@ -289,3 +309,205 @@ def targets_loo(chain, pack, R, model):
     S = R * chain.shape[1]
     print("{} ({:.2f} s)".format(summary_line(per, [S] * len(per)), time.time() - t_phase))
     return per, S
+
+
+# ---- exact leave-one-out by refitting ---------------------------------------------------------------------------
+
+def select_refit_points(rows, S, mode):
+    """Indices of the points of one pack's rows [n_points, 5] (LOO_COLUMNS) to refit: mode "all", every modelled point
+    (khat is 0 for a kind-3 point, whose PSIS column is constant; the caller drops kind 3 by its kind); mode "khat",
+    those whose khat exceeds khat_threshold(S) or is NaN or inf."""
+    rows = np.asarray(rows, dtype=np.float64).reshape(-1, 5)
+    if mode == "all":
+        return np.arange(len(rows))
+    if mode == "khat":
+        k = rows[:, 3]
+        return np.flatnonzero(~(k <= khat_threshold(S)) | ~np.isfinite(k))
+    raise ValueError("mode must be 'khat' or 'all'")
+
+
+def refit_folds(pack, data, points):
+    """The folds of the points `points` (indices into pack.points, ascending) of SinglePack(data): (modelled
+    [len(points)] bool, dataset of each modelled point, its index within the dataset, the reduced datasets
+    [(concs, responses)], their SinglePack, the held-out records: pack.points of the modelled points)."""
+    points = np.asarray(points, dtype=np.int64)
+    if np.any(np.diff(points) <= 0) or (len(points) and (points[0] < 0 or points[-1] >= len(pack.points))):
+        raise ValueError("points must be ascending indices into the pack's points")
+    modelled = pack.points["kind"][points] != POINT_NONE
+    p = points[modelled]
+    ds = np.searchsorted(pack.point_offsets, p, side="right") - 1
+    local = p - pack.point_offsets[ds]
+    reduced = [(np.delete(data[g][0], i), np.delete(data[g][1], i)) for g, i in zip(ds, local)]
+    return modelled, ds, local, reduced, SinglePack(reduced), pack.points[p].copy()
+
+
+def refit_chain_ids(model, n_folds, R):
+    """[n_folds, R] Philox chain ids of the refit chains (see the module docstring)."""
+    from .sampler import model_chain_id_base
+    return model_chain_id_base(model) + REFIT_ID_OFFSET + np.arange(n_folds * R, dtype=np.int64).reshape(-1, R)
+
+
+def refit_starts(model, data, reduced, ds, R, jitter=None):
+    """[n_folds * R, d] starts of the refit chains: the least-squares fit of each reduced dataset (of the full dataset
+    when the reduced one has no modelled point) times the main run's jitter factors of its dataset's chains (jitter
+    [n_datasets * R, d], as sampler.replicate_jitter gives them; None: no jitter)."""
+    from .initial_fit import best_fit_batch_gpu
+    d = 2 if model == 1 else 3
+    has = np.array([np.any(point_kinds(*masks(y)) != POINT_NONE) for _, y in reduced], dtype=bool)
+    fits = np.empty((len(reduced), d))
+    if np.any(has):
+        fits[has] = best_fit_batch_gpu(model, [reduced[j] for j in np.flatnonzero(has)])[0]
+    if not np.all(has):
+        full = np.unique(ds[~has])
+        ff = best_fit_batch_gpu(model, [data[g] for g in full])[0]
+        fits[~has] = ff[np.searchsorted(full, ds[~has])]
+    theta0 = np.repeat(fits, R, axis=0)
+    if jitter is not None:
+        jitter = np.asarray(jitter, dtype=np.float64).reshape(-1, R, d)
+        theta0 = theta0 * jitter[ds].reshape(-1, d)
+    return theta0
+
+
+def heldout_estimate(ll):
+    """(elpd_refit_i, se_refit_i) of one fold from ll [R, N]: the held-out point's l_i at the N kept rows of each of
+    its R chains (the host statement of the module docstring)."""
+    ll = np.atleast_2d(np.asarray(ll, dtype=np.float64))
+    R, N = ll.shape
+    if not np.all(np.isfinite(ll)):
+        return np.nan, np.nan
+    m = ll.max()
+    w = np.exp(ll - m)
+    E = w.mean()
+    n = N // 2
+    with np.errstate(invalid="ignore", divide="ignore"):
+        Eh = np.concatenate([w[:, :n].mean(axis=1), w[:, N - n:].mean(axis=1)]) if n else np.full(2 * R, np.nan)
+        se = np.std(Eh, ddof=1) / np.sqrt(2 * R) / E
+    return m + np.log(E), se
+
+
+def heldout_finish(acc, chain_offsets):
+    """[n_folds, 2] (elpd_refit_i, se_refit_i) from the accumulators [n_chains, HELDOUT_SLOTS, 4] that
+    phf_single_heldout_loglik fills (per chain and slot: max, sum exp(l - max), rows, non-finite rows); fold f is
+    chains chain_offsets[f] .. chain_offsets[f+1]-1.  The numbers of heldout_estimate."""
+    acc = np.asarray(acc, dtype=np.float64)
+    off = np.asarray(chain_offsets, dtype=np.int64)
+    out = np.full((len(off) - 1, 2), np.nan)
+    for f in range(len(off) - 1):
+        a = acc[off[f]:off[f + 1]]
+        if np.any(a[:, :, 3] > 0):
+            continue
+        m = a[:, :, 0].max()
+        with np.errstate(invalid="ignore", divide="ignore"):
+            w = np.where(a[:, :, 1] > 0, a[:, :, 1] * np.exp(a[:, :, 0] - m), 0.0)   # [R, slots], shifted to m
+            E = w.sum() / a[:, :, 2].sum()
+            Eh = np.concatenate([w[:, 0] / a[:, 0, 2], w[:, 1] / a[:, 1, 2]])
+            out[f] = m + np.log(E), np.std(Eh, ddof=1) / np.sqrt(len(Eh)) / E
+    return out
+
+
+def heldout_gpu(seg, row_begin, n_kept, model, chain_offsets, heldout, groups, acc):
+    """phf_single_heldout_loglik of the device rows `seg` [n_chains, n_rows, d+1] (chain-major, contiguous), kept rows
+    row_begin .. of n_kept, into the device accumulator `acc` [n_chains, HELDOUT_SLOTS, 4]; fold f is chains
+    chain_offsets[f] .. chain_offsets[f+1]-1 and holds out the record heldout[f] (POINT_DTYPE) of the pack whose
+    device dose groups are `groups`."""
+    torch = _check_chain(seg, model)
+    coff = np.ascontiguousarray(chain_offsets, dtype=np.int64)
+    rec = np.ascontiguousarray(heldout, dtype=_lib.POINT_DTYPE)
+    if len(rec) != len(coff) - 1 or coff[-1] > seg.shape[0]:
+        raise ValueError("one held-out record per fold, chain offsets within the chains")
+    if not (acc.is_cuda and acc.dtype == torch.float64 and acc.is_contiguous()
+            and tuple(acc.shape) == (seg.shape[0], HELDOUT_SLOTS, 4)):
+        raise ValueError("acc must be a contiguous float64 CUDA tensor [n_chains, %d, 4]" % HELDOUT_SLOTS)
+    with torch.cuda.device(seg.device):
+        _lib.check(_lib.load().phf_single_heldout_loglik(
+            model, seg.shape[1], int(row_begin), int(n_kept), seg.data_ptr(), len(rec), coff.ctypes.data,
+            rec.ctypes.data, groups.data_ptr(), acc.data_ptr(), _lib.current_stream_ptr()), "phf_single_heldout_loglik")
+
+
+def new_accumulator(n_chains, device):
+    """A device accumulator for heldout_gpu, at (-inf, 0, 0, 0) in every slot."""
+    torch = _lib.require_cuda()
+    acc = torch.zeros((n_chains, HELDOUT_SLOTS, 4), dtype=torch.float64, device=device)
+    acc[:, :, 0] = -np.inf
+    return acc
+
+
+def refit_loo(model, data, points, R, n_iters, thinning, burn_rows, seed, jitter=None, budget_bytes=8 << 30,
+              max_chains=1 << 24, lanes=0):
+    """[len(points), 2] (elpd_refit_i, se_refit_i) of the points `points` (ascending indices into
+    SinglePack(data).points) by exact refits (module docstring); a kind-3 point gets (-ln(2 pi) / 2, 0).
+
+    The folds run in one SingleLevelSampler, or in contiguous batches of at most max_chains chains, for n_iters
+    iterations in segments of a multiple of thinning whose rows (of all folds' chains) fit budget_bytes.  Each segment's
+    rows are reduced on the device by phf_single_heldout_loglik and dropped: no row goes to the host.  The lane count
+    is chosen once from all folds' chains (lanes=0) or pinned, and the segment length depends on the folds selected,
+    not on the batches, so batching does not change the result.  Synchronises the current stream."""
+    from .sampler import SingleLevelSampler, segment_lengths
+    torch = _lib.require_cuda()
+    import ctypes as C
+    pack = SinglePack(data)
+    points = np.asarray(points, dtype=np.int64)
+    out = np.full((len(points), 2), np.nan)
+    modelled, ds, local, reduced, rpack, heldout = refit_folds(pack, data, points)
+    out[~modelled] = (-HALF_LN_2PI, 0.0)
+    n_folds = len(reduced)
+    if n_folds == 0:
+        return out
+    d = 2 if model == 1 else 3
+    theta0 = refit_starts(model, data, reduced, ds, R, jitter)
+    ids = refit_chain_ids(model, n_folds, R)
+    n_kept = n_iters // thinning + 1 - burn_rows
+    if not 0 <= burn_rows < n_iters // thinning + 1:
+        raise ValueError("burn_rows must leave at least one kept row")
+    if lanes == 0:
+        lo, so = C.c_int32(0), C.c_int32(0)
+        _lib.check(_lib.load().phf_am_single_shape(n_folds * R, 0, 0, C.byref(lo), C.byref(so)), "phf_am_single_shape")
+        lanes = int(lo.value)
+    seg_rows = max(1, int(budget_bytes) // (n_folds * R * (d + 1) * 8))
+    per_batch = max(1, int(max_chains) // R)
+    dev = torch.device("cuda", torch.cuda.current_device())
+    res = np.empty((n_folds, 2))
+    for j0 in range(0, n_folds, per_batch):
+        j1 = min(j0 + per_batch, n_folds)
+        bpack = SinglePack(reduced[j0:j1])
+        s = SingleLevelSampler(model, bpack, np.repeat(np.arange(j1 - j0, dtype=np.int32), R), 1.0,
+                               theta0[j0 * R:j1 * R], variant="fit", seed=seed, chain_id_base=int(ids[j0, 0]),
+                               thinning=thinning, burn_rows=burn_rows, lanes=lanes)
+        acc = new_accumulator(s.n, dev)
+        coff = np.arange(j1 - j0 + 1, dtype=np.int64) * R
+        _, groups = pack.device(dev)
+        rec = heldout[j0:j1]
+        at = 0
+        if burn_rows == 0:                       # row 0, the start state, is a kept row
+            heldout_gpu(s.initial_row().reshape(s.n, 1, d + 1).contiguous(), 0, n_kept, model, coff, rec, groups, acc)
+            at = 1
+        for k in segment_lengths(n_iters, seg_rows * thinning, thinning):
+            seg = s.run(k, discard_burn=True)
+            if seg.shape[1]:
+                heldout_gpu(seg, at, n_kept, model, coff, rec, groups, acc)
+                at += seg.shape[1]
+            del seg
+        assert at == n_kept
+        res[j0:j1] = heldout_finish(acc.cpu().numpy(), coff)
+        del s, acc
+    out[modelled] = res
+    return out
+
+
+def targets_refit(per_dataset, data, S, mode, model, R, n_iters, thinning, burn_rows, seed, jitter):
+    """--loo-refit of PyHillFit: refit_loo of the points `mode` selects (select_refit_points) among the datasets whose
+    PSIS rows are per_dataset, with the summary line printed.  Returns a list of [N_k, 2] arrays, NaN where not
+    refitted."""
+    t_phase = time.time()
+    rows = np.concatenate(per_dataset).reshape(-1, 5)
+    pts = select_refit_points(rows, S, mode)
+    full = np.full((len(rows), 2), np.nan)
+    full[pts] = refit_loo(model, data, pts, R, n_iters, thinning, burn_rows, seed, jitter)
+    ends = np.cumsum([len(r) for r in per_dataset])
+    elpd = np.where(np.isfinite(full[:, 0]), full[:, 0], rows[:, 0]).sum()
+    kinds = np.concatenate([point_kinds(*masks(y)) for _, y in data])
+    fitted = pts[kinds[pts] != POINT_NONE]          # kind-3 points get their constant: nothing is refitted
+    print("LOO refits ({}): {} points in {} datasets, {} chains x {} iterations each; elpd_loo with refits {:.3f} "
+          "({:.2f} s)".format(mode, len(fitted), len(np.unique(np.searchsorted(ends, fitted, side="right"))), R,
+                              n_iters, elpd, time.time() - t_phase))
+    return np.split(full, ends[:-1])

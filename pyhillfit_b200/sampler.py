@@ -21,6 +21,18 @@ def model_chain_id_base(model):
     return (model - 1) << 40
 
 
+def replicate_jitter(n_datasets, R, d, seed):
+    """[n_datasets * R, d] factors of PyHillFit's replicate-chain starts: chain r > 0 of a dataset starts at the
+    least-squares fit times 1 + 0.02 N(0, 1) (numpy default_rng(seed), chains in order), chain 0 at the fit itself
+    like the reference.  All ones when R == 1."""
+    jit = np.ones((n_datasets * R, d))
+    if R > 1:
+        rng = np.random.default_rng(seed)
+        jit = 1.0 + 0.02 * rng.standard_normal(jit.shape)
+        jit[::R] = 1.0
+    return jit
+
+
 def segment_lengths(n_iters, segment, thinning):
     """Iterations of each launch of a run of n_iters split into segments: `segment` rounded down to a multiple of
     thinning (at least one thinning), the last launch taking what is left."""
